@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the hot path on synthetic MARS-shaped data, one JSON line (see DESIGN.md, "Measurement").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Job (BASELINE.json metric "MARS-shape tracklets/s (graph head) + query x gallery eval ms"):
 one STEP is a whole MARS-shaped test pass minus the stock backbone -- the graph head over
@@ -314,6 +314,8 @@ def run_b200(args):
         total_ms, head_ms, eval_ms = cx.max_over_ranks(total_ms, head_ms, eval_ms)
         ms_per_step = total_ms / args.steps
         value = world * J / (ms_per_step * 1e-3)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, feats, result)
 
         # ---- kernel timeline of one more step (CUDA events after every kernel, same stream) ------
         # (every rank runs the pass -- eval_pass holds collectives at N > 1 -- rank 0's timeline is reported)
@@ -451,6 +453,22 @@ def run_b200(args):
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_FEATURE_ROWS = 2048        # 2048 x 4096 fp32 = 32 MB of the 11310-row feature matrix (185 MB in full)
+
+
+def dump_outputs(out_dir, feats, result):
+    """What the last timed step handed its caller, as .npy files that two builds can be compared on: `features`, a fixed
+    seeded sample of the head's feature rows in ascending row order (float32), and the evaluation's `cmc` and `mAP`
+    (float64)."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = min(DUMP_FEATURE_ROWS, feats.shape[0])
+    rows = np.sort(np.random.RandomState(0).choice(feats.shape[0], n, replace=False))
+    sample = feats[torch.as_tensor(rows, device=feats.device)].cpu().numpy().astype(np.float32)
+    np.save(os.path.join(out_dir, 'features.npy'), sample)
+    np.save(os.path.join(out_dir, 'cmc.npy'), np.asarray(result[0], dtype=np.float64))
+    np.save(os.path.join(out_dir, 'mAP.npy'), np.asarray(result[1], dtype=np.float64))
 
 
 def guarded(fn):
@@ -1069,7 +1087,13 @@ def main():
     ap.add_argument('--eager-sample', type=int, default=256, help='tracklets of the pool the comparator head is timed on')
     ap.add_argument('--no-fast-mode', action='store_true', help='skip the extra head pass with the fp16 single-plane GEMM')
     ap.add_argument('--quick', action='store_true', help='only the timed region + kernel table (profiling runs)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write what the last timed step computed to DIR/<name>.npy '
+                                                          '(features sample, cmc, mAP)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl != 'b200' or args.workload != 'mars'):
+        ap.error('--dump-outputs applies to the B200 arm of the MARS workload')
     if args.quick:
         args.no_e2e = args.no_cpu_baseline = args.no_parity = args.no_energy = args.no_curve = True
         args.no_configs = args.no_eager = args.no_fast_mode = True

@@ -280,3 +280,24 @@ def make_rerank():
 
 if __name__ == '__main__' and ('rerank' in sys.argv[1:] or not sys.argv[1:]):
     make_rerank()
+
+
+# ------------------------------------------------------------------------------- rank_cy on dataset shapes
+def make_rank_cy_fresh():
+    """The reference's compiled rank_cy (numpy.argsort forced stable) on the dataset-shaped inputs of
+    tests/test_oracle_rank.py::test_port_vs_compiled_reference_rank_cy: cmc and mAP per case, and a checksum of the
+    inputs (they are regenerated from their seeds, not stored)."""
+    sys.path.insert(0, os.path.dirname(HERE))
+    from test_oracle_rank import FRESH_CY, FRESH_CY_CASES, fresh_cy_inputs
+    out = {}
+    for case in FRESH_CY_CASES:
+        key, d, qp, qc, gp, gc, checksum = fresh_cy_inputs(*case)
+        cmc, mAP = orank.reference_evaluate_cy(d, qp, gp, qc, gc, 50)
+        out[key + '_cmc'], out[key + '_mAP'], out[key + '_checksum'] = np.asarray(cmc), np.float64(mAP), checksum
+        assert out[key + '_cmc'].dtype == np.float32
+    np.savez_compressed(os.path.join(HERE, FRESH_CY), **out)
+    print(FRESH_CY, sorted(out))
+
+
+if __name__ == '__main__' and ('rank_cy' in sys.argv[1:] or not sys.argv[1:]):
+    make_rank_cy_fresh()

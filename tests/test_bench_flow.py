@@ -132,6 +132,49 @@ def test_a_failing_extra_figure_does_not_cost_the_line(fake_device, monkeypatch,
     assert model.head_split == _lib.SPLIT_BF16X2
 
 
+class CallCountingModel(FakeModel):
+    """Feature row i of the c-th head call (from 0) holds 1000 * c + i: a dumped row names the call that wrote it."""
+
+    def head(self, x1, x2, adj, S, out=None):
+        super().head(x1, x2, adj, S, out=out)
+        c = len(self.calls) - 1
+        out.copy_((1000 * c + torch.arange(out.shape[0], dtype=out.dtype))[:, None].expand_as(out))
+        return out
+
+
+def test_dump_outputs_writes_the_last_timed_step(fake_device, monkeypatch, capsys, tmp_path):
+    evals = []
+
+    def evaluate_rank(*a, **k):                                     # the n-th evaluation (from 1) returns cmc = mAP = n
+        evals.append(None)
+        return np.full(50, float(len(evals))), np.float64(len(evals))
+    monkeypatch.setattr(metrics, 'evaluate_rank', evaluate_rank)
+    line = run(monkeypatch, capsys, CallCountingModel(), ['--dump-outputs', str(tmp_path)])
+    warmup, steps, pool, J = line['warmup'], line['steps'], line['config']['pool_tracklets'], bench.NQ + bench.NG
+    assert (warmup, steps) == (3, 2) and len(evals) > warmup + steps            # evaluations also ran after the timed steps
+    assert sorted(p.name for p in tmp_path.iterdir()) == ['cmc.npy', 'features.npy', 'mAP.npy']
+    d = {k: np.load(str(tmp_path / (k + '.npy'))) for k in ('features', 'cmc', 'mAP')}
+    assert d['features'].dtype == np.float32 and d['cmc'].dtype == np.float64 and d['mAP'].dtype == np.float64
+    assert d['cmc'].shape == (50,) and d['mAP'].shape == ()
+    assert np.all(d['cmc'] == warmup + steps) and float(d['mAP']) == warmup + steps     # the last timed evaluation
+    # the fixed seeded row sample, each row as the last timed head pass wrote it
+    rows = np.sort(np.random.RandomState(0).choice(J, bench.DUMP_FEATURE_ROWS, replace=False))
+    calls_per_pass = -(-J // pool)
+    want = 1000 * ((warmup + steps - 1) * calls_per_pass + rows // pool) + rows % pool
+    f = d['features']
+    assert f.shape == (bench.DUMP_FEATURE_ROWS, 2 * bench.C) and np.all(f == f[:, :1])
+    assert np.array_equal(f[:, 0], want.astype(np.float32))
+    assert sum(a.nbytes for a in d.values()) <= 64 << 20
+
+
+@pytest.mark.parametrize('argv', [['--steps', '0'], ['--impl', 'reference', '--dump-outputs', 'x'],
+                                  ['--workload', 'sweep', '--dump-outputs', 'x']])
+def test_rejected_arguments(monkeypatch, argv):
+    monkeypatch.setattr(bench.sys, 'argv', ['bench.py'] + argv)
+    with pytest.raises(SystemExit):
+        bench.main()
+
+
 def test_reference_arm_line_reports_what_it_executed(monkeypatch, capsys):
     """--impl reference: same metric / unit / workload string as the B200 arm, the executed step time as ms_per_step, the
     extrapolation flagged (tiny sample here so that the CPU suite stays fast)."""

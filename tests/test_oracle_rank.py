@@ -1,6 +1,6 @@
 """Pin the ranking oracle (oracle/rank_oracle.c) to the reference: golden vectors produced by the
-reference's evaluate_rank (tests/golden/make_golden.py) and, when present, the reference's own
-compiled rank_cy (oracle/_ref) on fresh random inputs."""
+reference's evaluate_rank (tests/golden/make_golden.py) and the reference's own compiled rank_cy on larger
+dataset-shaped inputs: its recorded outputs (tests/golden/fresh_rank_cy.npz) or, when built, oracle/_ref itself."""
 import os
 
 import numpy as np
@@ -54,17 +54,35 @@ def test_pairwise_sum_is_numpys(n):
     assert orank.pairwise_sum_f64(x) == (np.add.reduce(x) if n else 0.0)
 
 
-@pytest.mark.skipif(orank.reference_rank_cy() is None, reason='oracle/_ref not built')
-@pytest.mark.parametrize('shape,seed,ties', [('dukev', 0, False), ('dukev', 1, True), ('ilidsvid', 2, False),
-                                             ((200, 3000, 40, 5), 3, True)])
-def test_port_vs_compiled_reference_rank_cy(shape, seed, ties):
+FRESH_CY = 'fresh_rank_cy.npz'          # rank_cy's outputs on the inputs below (tests/golden/make_golden.py rank_cy)
+FRESH_CY_CASES = [('dukev', 0, False), ('dukev', 1, True), ('ilidsvid', 2, False), ((200, 3000, 40, 5), 3, True)]
+
+
+def fresh_cy_inputs(shape, seed, ties):
+    """(key, distmat, q_pids, q_camids, g_pids, g_camids, checksum) of one case, regenerated from its seed."""
     qp, qc, gp, gc = synth.eval_labels(shape, seed=seed)
     nq, ng = len(qp), len(gp)
     if ties:
         d = synth.quantised_distmat(nq, ng, seed=seed)
     else:
         d = np.random.RandomState(seed).randn(nq, ng).astype(np.float32)
+    key = '%s_%d_%d' % (shape if isinstance(shape, str) else 'x'.join(map(str, shape)), seed, ties)
+    checksum = np.float64(d.astype(np.float64).sum() + sum((i + 2) * x.astype(np.float64).sum()
+                                                           for i, x in enumerate((qp, qc, gp, gc))))
+    return key, d, qp, qc, gp, gc, checksum
+
+
+@pytest.mark.skipif(not os.path.exists(os.path.join(GOLDEN, FRESH_CY)) and orank.reference_rank_cy() is None,
+                    reason='no stored outputs of the reference rank_cy (tests/golden/%s) and oracle/_ref not built' % FRESH_CY)
+@pytest.mark.parametrize('shape,seed,ties', FRESH_CY_CASES)
+def test_port_vs_compiled_reference_rank_cy(shape, seed, ties):
+    key, d, qp, qc, gp, gc, checksum = fresh_cy_inputs(shape, seed, ties)
     cmc, mAP = orank.market1501_port(d, qp, gp, qc, gc, 50)
-    rcmc, rmAP = orank.reference_evaluate_cy(d, qp, gp, qc, gc, 50)
+    if os.path.exists(os.path.join(GOLDEN, FRESH_CY)):
+        g = _load(FRESH_CY)
+        assert g[key + '_checksum'] == checksum, 'regenerated inputs drifted from the recorded ones'
+        rcmc, rmAP = g[key + '_cmc'], float(g[key + '_mAP'])
+    else:
+        rcmc, rmAP = orank.reference_evaluate_cy(d, qp, gp, qc, gc, 50)
     assert np.array_equal(cmc.view(np.uint32), np.asarray(rcmc).view(np.uint32))
     assert mAP == rmAP
