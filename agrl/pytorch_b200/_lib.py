@@ -17,6 +17,7 @@ ST_NO_VALID_QUERY, ST_ZERO_DIVISION, ST_LABEL_RANGE, ST_TOPK_OVERFLOW = 1, 2, 4,
 METRIC_EUCLIDEAN, METRIC_COSINE = 0, 1
 SPLIT_BF16X3, SPLIT_BF16X2, SPLIT_FP16X1, SPLIT_FP16_E4M3, SPLIT_FP16X2 = 3, 2, 1, 4, 5
 CLIP_POOL_AVG, CLIP_POOL_MAX = 0, 1
+MAPS_FP32, MAPS_BF16, MAPS_FP16 = 0, 1, 2
 HEAD_MAX_LAYERS = 4
 
 c_i64, c_i32, c_sz, c_vp, c_int = ctypes.c_int64, ctypes.c_int32, ctypes.c_size_t, ctypes.c_void_p, ctypes.c_int
@@ -34,7 +35,7 @@ class HeadParams(ctypes.Structure):
         ('global_bn', c_vp * 4), ('att_bn', c_vp * 4),
         ('maps_nhwc', c_i32),
         ('lowrank_off', c_i32), ('pool_register_loads', c_i32), ('pool_stages', c_i32), ('pool_no_l2_hint', c_i32),
-        ('gemm_no_pair', c_i32),
+        ('gemm_no_pair', c_i32), ('maps_dtype', c_i32),
     ]
 
 

@@ -2,7 +2,8 @@
 //
 // Per batch of B tracklets (S frames, P = 7 pyramid strips, V = S*P region nodes, C channels):
 //
-//   pool_tma_kernel    one pass over both layer4 maps (the only HBM-heavy step, 2 x S*C*h*w*4 B per tracklet): strip
+//   pool_tma_kernel    one pass over both layer4 maps (the only HBM-heavy step, 2 x S*C*h*w*4 B per tracklet, half that
+//                      for the bf16 / fp16 maps of an autocast backbone, read as they are and summed in fp32): strip
 //                      means -> node tensor X0 (B,V,C) written directly in node order (vmgn.py:304-308, no cat / transpose
 //                      copies, x4_2 read once instead of three times) and the global mean -> BN neck -> out[:, :C]
 //                      (vmgn.py:299-301).  Persistent CTAs, loads kept in flight in a shared-memory ring by cp.async.bulk;
@@ -95,10 +96,42 @@ static Prepared carve_prepared(const agrl_head_params *p, void *buf) {
 }
 
 // ------------------------------------------------------------------------------------------------
+// element types of the layer4 maps (agrl_head_params.maps_dtype): fp32, or the bf16 / fp16 maps an autocast backbone
+// returns.  Every pooling kernel converts on load (exact: both 16-bit formats, inf and NaN included, are subsets of fp32)
+// and then sums exactly as it does for fp32, so 16-bit maps give the bits that their .float() copy gives.
+// Vec4 is four consecutive elements: one 16-byte load at fp32, one 8-byte load at 16 bits.
+// ------------------------------------------------------------------------------------------------
+template <class T> struct MapElem;
+template <> struct MapElem<float> {
+    using Vec4 = float4;
+    static __device__ __forceinline__ float cvt(float v) { return v; }
+    static __device__ __forceinline__ float4 cvt4(const float4 &v) { return v; }
+};
+template <> struct MapElem<__nv_bfloat16> {
+    using Vec4 = uint2;
+    static __device__ __forceinline__ float cvt(__nv_bfloat16 v) { return __bfloat162float(v); }
+    static __device__ __forceinline__ float4 cvt4(const uint2 &v) {
+        const float2 lo = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162 *>(&v.x));
+        const float2 hi = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162 *>(&v.y));
+        return make_float4(lo.x, lo.y, hi.x, hi.y);
+    }
+};
+template <> struct MapElem<__half> {
+    using Vec4 = uint2;
+    static __device__ __forceinline__ float cvt(__half v) { return __half2float(v); }
+    static __device__ __forceinline__ float4 cvt4(const uint2 &v) {
+        const float2 lo = __half22float2(*reinterpret_cast<const __half2 *>(&v.x));
+        const float2 hi = __half22float2(*reinterpret_cast<const __half2 *>(&v.y));
+        return make_float4(lo.x, lo.y, hi.x, hi.y);
+    }
+};
+
+// ------------------------------------------------------------------------------------------------
 // pooling: grid (C/64, B), 8 warps x 8 channels, loop over the S frames
 // ------------------------------------------------------------------------------------------------
+template <class T>
 struct PoolArgs {
-    const float *x41, *x42;            // (B*S, C, hw)
+    const T *x41, *x42;                // (B*S, C, hw)
     float *nodes;                      // (B, V, C)
     float *out; int64_t ld_out;        // (B, 2C): global branch -> [:, :C]
     const float *g_scale, *g_shift;    // folded global_bottleneck
@@ -107,9 +140,11 @@ struct PoolArgs {
 
 constexpr int kPoolCh = 64;            // channels per CTA
 
-template <bool kVec>
+template <bool kVec, class T>
 __global__ void __launch_bounds__(kHeadThreads)
-pool_kernel(PoolArgs a) {
+pool_kernel(PoolArgs<T> a) {
+    using E = MapElem<T>;
+    using Vec4 = typename E::Vec4;
     extern __shared__ float s_nodes[];                 // [S][7][kPoolCh]
     const int b = blockIdx.y, c0 = blockIdx.x * kPoolCh;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -126,12 +161,12 @@ pool_kernel(PoolArgs a) {
         const size_t frame = (static_cast<size_t>(b) * a.S + s) * a.C;
         float q1[8], q2[8];
         if (kVec) {
-            // hw == 128: one float4 per lane covers a (frame, channel) plane; 16 loads in flight per lane
+            // hw == 128: four elements per lane cover a (frame, channel) plane; 16 loads in flight per lane
 #pragma unroll
             for (int i = 0; i < 8; ++i) {
                 const size_t off = (frame + c0 + warp * 8 + i) * hw + lane * 4;
-                const float4 v1 = __ldcs(reinterpret_cast<const float4 *>(a.x41 + off));
-                const float4 v2 = __ldcs(reinterpret_cast<const float4 *>(a.x42 + off));
+                const float4 v1 = E::cvt4(__ldcs(reinterpret_cast<const Vec4 *>(a.x41 + off)));
+                const float4 v2 = E::cvt4(__ldcs(reinterpret_cast<const Vec4 *>(a.x42 + off)));
                 q1[i] = (v1.x + v1.y) + (v1.z + v1.w);
                 q2[i] = (v2.x + v2.y) + (v2.z + v2.w);
             }
@@ -140,7 +175,7 @@ pool_kernel(PoolArgs a) {
             for (int i = 0; i < 8; ++i) {
                 const size_t off = (frame + c0 + warp * 8 + i) * hw + grp * qlen;
                 float s1 = 0.f, s2 = 0.f;
-                for (int e = sub; e < qlen; e += 8) { s1 += a.x41[off + e]; s2 += a.x42[off + e]; }
+                for (int e = sub; e < qlen; e += 8) { s1 += E::cvt(a.x41[off + e]); s2 += E::cvt(a.x42[off + e]); }
                 q1[i] = s1; q2[i] = s2;
             }
         }
@@ -185,14 +220,17 @@ pool_kernel(PoolArgs a) {
 // pooling, channels-last maps (SURVEY.md section 8f row 4, the part that stays on our side of the cuDNN boundary):
 // a backbone run in torch.channels_last hands over (B*S, h, w, C)-ordered memory; converting it back to NCHW would
 // cost a second pass over the 16 MiB per tracklet.  Here a thread owns 4 consecutive channels (one 16-byte load per
-// pixel, fully coalesced across the CTA), keeps the four quarter-strip sums in registers and writes node rows
-// straight from them.  grid (C / 1024, B), 256 threads.
+// pixel at fp32, 8 bytes at 16 bits, fully coalesced across the CTA), keeps the four quarter-strip sums in registers and
+// writes node rows straight from them.  grid (C / 1024, B), 256 threads.  Needs maps aligned to 4 elements.
 // ------------------------------------------------------------------------------------------------
 __device__ __forceinline__ void add4(float4 &a, const float4 &b) { a.x += b.x; a.y += b.y; a.z += b.z; a.w += b.w; }
 __device__ __forceinline__ float4 scale4(const float4 &a, float s) { return make_float4(a.x * s, a.y * s, a.z * s, a.w * s); }
 
+template <class T>
 __global__ void __launch_bounds__(kHeadThreads)
-pool_nhwc_kernel(PoolArgs a) {
+pool_nhwc_kernel(PoolArgs<T> a) {
+    using E = MapElem<T>;
+    using Vec4 = typename E::Vec4;
     const int b = blockIdx.y;
     const int c = (blockIdx.x * kHeadThreads + threadIdx.x) * 4;
     if (c >= a.C) return;
@@ -210,8 +248,8 @@ pool_nhwc_kernel(PoolArgs a) {
             const size_t base = frame + static_cast<size_t>(k) * qlen * a.C;
 #pragma unroll 8
             for (int p = 0; p < qlen; ++p) {
-                add4(s1, __ldcs(reinterpret_cast<const float4 *>(a.x41 + base + static_cast<size_t>(p) * a.C)));
-                add4(s2, __ldcs(reinterpret_cast<const float4 *>(a.x42 + base + static_cast<size_t>(p) * a.C)));
+                add4(s1, E::cvt4(__ldcs(reinterpret_cast<const Vec4 *>(a.x41 + base + static_cast<size_t>(p) * a.C))));
+                add4(s2, E::cvt4(__ldcs(reinterpret_cast<const Vec4 *>(a.x42 + base + static_cast<size_t>(p) * a.C))));
             }
             add4(g, s1);
             q[k] = s2;
@@ -240,21 +278,26 @@ pool_nhwc_kernel(PoolArgs a) {
 // pooling, bulk-copy (TMA) flavour: a persistent, deliberately small CTA (1 producer + 4 consumer
 // warps, < 64 registers, two per SM) that keeps its loads in flight in a shared-memory ring instead of in
 // registers.
-//   work unit   (tracklet b, 32-channel chunk): 2*S ring stages of 16 KiB, each one frame of one map
-//               (32 channels x 128 floats are contiguous in NCHW), fetched with one cp.async.bulk
-//               (L2 evict-first) that completes on the stage's mbarrier
-//   consumers   warp w owns channels 8w..8w+7 of the chunk: one conflict-free LDS.128 per lane covers a
-//               16x8 plane, strip sums by shuffles exactly as in pool_kernel
+//   work unit   (tracklet b, 32-channel chunk): 2*S ring stages, each one frame of one map (32 channels x
+//               128 elements are contiguous in NCHW: 16 KiB at fp32, 8 KiB at 16 bits), fetched with one
+//               cp.async.bulk (L2 evict-first) that completes on the stage's mbarrier
+//   consumers   warp w owns channels 8w..8w+7 of the chunk: one conflict-free LDS.128 (fp32) or LDS.64 (16 bits)
+//               per lane covers a 16x8 plane, strip sums by shuffles exactly as in pool_kernel
 //   output      node rows staged in (double-buffered) smem -> full 128-byte row segments
 // Requires h*w == 128 (the canonical 16x8 maps) and 16-byte aligned maps; otherwise pool_kernel runs.
 // ------------------------------------------------------------------------------------------------
 constexpr int kTpCh = 32;
-constexpr int kTpStageBytes = kTpCh * 128 * 4;
 constexpr int kTpConsumerWarps = 4;
 constexpr int kTpThreads = 32 * (1 + kTpConsumerWarps);
+template <class T> constexpr int tp_stage_bytes() { return kTpCh * 128 * static_cast<int>(sizeof(T)); }
+// default ring depth: 4 stages (64 KiB in flight per CTA) at fp32; 12 of 8 KiB at 16 bits, where 4 stages are 5 % slower
+// and 8 to 12 within 1-3 % of each other (profiles/half_maps/half_maps_bench.json, DESIGN.md section 3); at S <= 8 two
+// CTAs still fit on an SM
+template <class T> constexpr int tp_default_stages() { return sizeof(T) == 4 ? 4 : 12; }
 
+template <class T>
 struct PoolTmaArgs {
-    const float *x41, *x42;            // (batch*S, C, 128), already offset to this sub-batch
+    const T *x41, *x42;                // (batch*S, C, 128), already offset to this sub-batch
     float *nodes;                      // (batch, V, C)
     float *out; int64_t ld_out;        // (batch, 2C)
     const float *g_scale, *g_shift;
@@ -264,8 +307,8 @@ struct PoolTmaArgs {
 };
 
 // dynamic shared memory: ring | two node tiles | barriers (+ alignment slack)
-static size_t pool_tma_smem(int S, int stages) {
-    const size_t b = static_cast<size_t>(stages) * kTpStageBytes + 2 * static_cast<size_t>(S) * kParts * kTpCh * sizeof(float) +
+static size_t pool_tma_smem(int S, int stages, int stage_bytes) {
+    const size_t b = static_cast<size_t>(stages) * stage_bytes + 2 * static_cast<size_t>(S) * kParts * kTpCh * sizeof(float) +
                      2 * static_cast<size_t>(stages) * 8;
     return ((b + 127) & ~static_cast<size_t>(127)) + 128;
 }
@@ -301,14 +344,19 @@ __device__ __forceinline__ void bulk_load(uint32_t dst, const void *src, uint32_
                  ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
 }
 
+template <class T>
 __global__ void __maxnreg__(48)
-pool_tma_kernel(PoolTmaArgs a) {
+pool_tma_kernel(PoolTmaArgs<T> a) {
+    using E = MapElem<T>;
+    using Vec4 = typename E::Vec4;
+    constexpr int kStageBytes = tp_stage_bytes<T>();
+    constexpr int kStageVec4 = kTpCh * 128 / 4;                   // 4-element loads per stage
     extern __shared__ __align__(16) unsigned char tp_smem_dyn[];
     const int stages = a.stages, S = a.S, C = a.C, V = S * kParts;
     // align to 128 B by OFFSET (not by casting through an integer) so that the compiler keeps emitting LDS / STS
     unsigned char *smem = tp_smem_dyn + ((128u - (gemm::smem_u32(tp_smem_dyn) & 127u)) & 127u);
-    const float4 *ring_f4 = reinterpret_cast<const float4 *>(smem);
-    float *s_nodes = reinterpret_cast<float *>(smem + stages * kTpStageBytes);   // [2][V][32]
+    const Vec4 *ring_v = reinterpret_cast<const Vec4 *>(smem);
+    float *s_nodes = reinterpret_cast<float *>(smem + stages * kStageBytes);     // [2][V][32]
     uint64_t *bars = reinterpret_cast<uint64_t *>(s_nodes + 2 * V * kTpCh);
     const uint32_t ring = gemm::smem_u32(smem);
     const uint32_t bar_full = gemm::smem_u32(bars), bar_empty = bar_full + 8 * stages;
@@ -339,9 +387,9 @@ pool_tma_kernel(PoolTmaArgs a) {
                     for (int m = 0; m < 2; ++m) {
                         gemm::mbar_wait(bar_empty + 8 * stage, phase ^ 1);
                         const uint32_t full = bar_full + 8 * stage;
-                        gemm::mbar_arrive_expect_tx(full, kTpStageBytes);
-                        if (a.l2_hint) bulk_load_evict_first(ring + stage * kTpStageBytes, (m ? a.x42 : a.x41) + off, kTpStageBytes, full, policy);
-                        else bulk_load(ring + stage * kTpStageBytes, (m ? a.x42 : a.x41) + off, kTpStageBytes, full);
+                        gemm::mbar_arrive_expect_tx(full, kStageBytes);
+                        if (a.l2_hint) bulk_load_evict_first(ring + stage * kStageBytes, (m ? a.x42 : a.x41) + off, kStageBytes, full, policy);
+                        else bulk_load(ring + stage * kStageBytes, (m ? a.x42 : a.x41) + off, kStageBytes, full);
                         if (++stage == stages) { stage = 0; phase ^= 1; }
                     }
                 }
@@ -363,10 +411,10 @@ pool_tma_kernel(PoolTmaArgs a) {
                 // ---- layer4_1 frame: only the global mean needs it -> per-lane partial sums ----
                 gemm::mbar_wait(bar_full + 8 * stage, phase);
                 {
-                    const float4 *p = ring_f4 + stage * (kTpStageBytes / 16) + (cw * 8) * 32 + lane;
+                    const Vec4 *p = ring_v + stage * kStageVec4 + (cw * 8) * 32 + lane;
 #pragma unroll
                     for (int i = 0; i < 8; ++i) {
-                        const float4 v = p[i * 32];
+                        const float4 v = E::cvt4(p[i * 32]);
                         gsum[i] += (v.x + v.y) + (v.z + v.w);
                     }
                 }
@@ -380,11 +428,11 @@ pool_tma_kernel(PoolTmaArgs a) {
                 // ---- layer4_2 frame: quarter / half / whole strip means -> node rows ----
                 gemm::mbar_wait(bar_full + 8 * stage, phase);
                 {
-                    const float4 *p = ring_f4 + stage * (kTpStageBytes / 16) + (cw * 8) * 32 + lane;
+                    const Vec4 *p = ring_v + stage * kStageVec4 + (cw * 8) * 32 + lane;
                     float q[8];
 #pragma unroll
                     for (int i = 0; i < 8; ++i) {
-                        const float4 v = p[i * 32];
+                        const float4 v = E::cvt4(p[i * 32]);
                         q[i] = (v.x + v.y) + (v.z + v.w);
                     }
                     asm volatile("" ::"f"(q[0]), "f"(q[1]), "f"(q[2]), "f"(q[3]), "f"(q[4]), "f"(q[5]), "f"(q[6]), "f"(q[7]) : "memory");
@@ -1222,6 +1270,7 @@ static int check_params(const agrl_head_params *p) {
     if (p->channels < kChunk || p->channels % kChunk != 0) return AGRL_E_UNSUPPORTED;
     if (!p->use_pose && !p->learn_graph) return AGRL_E_INVALID;            // vmgn.py:92 assert
     if (p->pool_stages != 0 && (p->pool_stages < 2 || p->pool_stages > 12)) return AGRL_E_INVALID;
+    if (p->maps_dtype != AGRL_MAPS_FP32 && p->maps_dtype != AGRL_MAPS_BF16 && p->maps_dtype != AGRL_MAPS_FP16) return AGRL_E_INVALID;
     return AGRL_OK;
 }
 
@@ -1298,9 +1347,10 @@ extern "C" size_t agrl_head_workspace_bytes(const agrl_head_params *p, int64_t b
 
 namespace agrl {
 
-// pooling of `n` tracklets starting at tracklet `b0`, on stream `st`
-static int launch_pool(const agrl_head_params *p, const Prepared &pr, const HeadWorkspace &hwk, const float *x4_1,
-                       const float *x4_2, float *out, int64_t ld_out, int64_t b0, int64_t n, int S, int hw, bool tma,
+// pooling of `n` tracklets starting at tracklet `b0`, on stream `st`; maps of element type T
+template <class T>
+static int launch_pool(const agrl_head_params *p, const Prepared &pr, const HeadWorkspace &hwk, const T *x4_1,
+                       const T *x4_2, float *out, int64_t ld_out, int64_t b0, int64_t n, int S, int hw, bool tma,
                        cudaStream_t st) {
     const int C = p->channels, V = S * kParts, L = p->num_layers;
     const size_t in_off = static_cast<size_t>(b0) * S * C * hw;
@@ -1308,32 +1358,52 @@ static int launch_pool(const agrl_head_params *p, const Prepared &pr, const Head
     float *o = out + static_cast<size_t>(b0) * ld_out;
     AGRL_LAUNCH_BEGIN(st);
     if (p->maps_nhwc) {
-        PoolArgs pa{x4_1 + in_off, x4_2 + in_off, nodes, o, ld_out, pr.scale[L], pr.shift[L], S, C, hw};
+        PoolArgs<T> pa{x4_1 + in_off, x4_2 + in_off, nodes, o, ld_out, pr.scale[L], pr.shift[L], S, C, hw};
         const dim3 grid((C / 4 + kHeadThreads - 1) / kHeadThreads, static_cast<unsigned>(n));
-        pool_nhwc_kernel<<<grid, kHeadThreads, 0, st>>>(pa);
+        pool_nhwc_kernel<T><<<grid, kHeadThreads, 0, st>>>(pa);
         AGRL_LAUNCH_CHECK(st, "pool");
         return AGRL_OK;
     }
     if (tma) {
         const int64_t units = n * (C / kTpCh);
-        PoolTmaArgs ta{x4_1 + in_off, x4_2 + in_off, nodes, o, ld_out, pr.scale[L], pr.shift[L], S, C,
-                       p->pool_stages ? p->pool_stages : 4, 0, static_cast<int>(units), p->pool_no_l2_hint ? 0 : 1};
-        const size_t smem = pool_tma_smem(S, ta.stages);
-        AGRL_CUDA_TRY(cudaFuncSetAttribute(pool_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+        PoolTmaArgs<T> ta{x4_1 + in_off, x4_2 + in_off, nodes, o, ld_out, pr.scale[L], pr.shift[L], S, C,
+                          p->pool_stages ? p->pool_stages : tp_default_stages<T>(), 0, static_cast<int>(units),
+                          p->pool_no_l2_hint ? 0 : 1};
+        const size_t smem = pool_tma_smem(S, ta.stages, tp_stage_bytes<T>());
+        AGRL_CUDA_TRY(cudaFuncSetAttribute(pool_tma_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
         int64_t grid = static_cast<int64_t>(kNumSMs) * 2;                 // persistent, two small CTAs per SM
         if (grid > units) grid = units;
-        pool_tma_kernel<<<static_cast<unsigned>(grid), kTpThreads, smem, st>>>(ta);
+        pool_tma_kernel<T><<<static_cast<unsigned>(grid), kTpThreads, smem, st>>>(ta);
         AGRL_LAUNCH_CHECK(st, "pool");
         return AGRL_OK;
     }
-    PoolArgs pa{x4_1 + in_off, x4_2 + in_off, nodes, o, ld_out, pr.scale[L], pr.shift[L], S, C, hw};
+    PoolArgs<T> pa{x4_1 + in_off, x4_2 + in_off, nodes, o, ld_out, pr.scale[L], pr.shift[L], S, C, hw};
     const size_t pool_smem = static_cast<size_t>(S) * kParts * kPoolCh * sizeof(float);
     const dim3 pgrid(C / kPoolCh, static_cast<unsigned>(n));
-    const bool vec = (hw == 128) && ((reinterpret_cast<uintptr_t>(x4_1) & 15u) == 0) && ((reinterpret_cast<uintptr_t>(x4_2) & 15u) == 0);
-    if (vec) pool_kernel<true><<<pgrid, kHeadThreads, pool_smem, st>>>(pa);
-    else pool_kernel<false><<<pgrid, kHeadThreads, pool_smem, st>>>(pa);
+    // vector loads of four elements need the maps aligned to four elements
+    const uintptr_t vec_align = 4 * sizeof(T) - 1;
+    const bool vec = (hw == 128) && ((reinterpret_cast<uintptr_t>(x4_1) | reinterpret_cast<uintptr_t>(x4_2)) & vec_align) == 0;
+    if (vec) pool_kernel<true, T><<<pgrid, kHeadThreads, pool_smem, st>>>(pa);
+    else pool_kernel<false, T><<<pgrid, kHeadThreads, pool_smem, st>>>(pa);
     AGRL_LAUNCH_CHECK(st, "pool");
     return AGRL_OK;
+}
+
+// the maps' element type chosen at run time (agrl_head_params.maps_dtype; check_params has vetted it)
+static int launch_pool_any(const agrl_head_params *p, const Prepared &pr, const HeadWorkspace &hwk, const void *x4_1,
+                           const void *x4_2, float *out, int64_t ld_out, int64_t b0, int64_t n, int S, int hw, bool tma,
+                           cudaStream_t st) {
+    switch (p->maps_dtype) {
+        case AGRL_MAPS_BF16:
+            return launch_pool(p, pr, hwk, static_cast<const __nv_bfloat16 *>(x4_1), static_cast<const __nv_bfloat16 *>(x4_2),
+                               out, ld_out, b0, n, S, hw, tma, st);
+        case AGRL_MAPS_FP16:
+            return launch_pool(p, pr, hwk, static_cast<const __half *>(x4_1), static_cast<const __half *>(x4_2),
+                               out, ld_out, b0, n, S, hw, tma, st);
+        default:
+            return launch_pool(p, pr, hwk, static_cast<const float *>(x4_1), static_cast<const float *>(x4_2),
+                               out, ld_out, b0, n, S, hw, tma, st);
+    }
 }
 
 // one GEMM of a graph layer in the caller's operand mode; Epi is built by `make(fp8)` for the scaled modes
@@ -1457,13 +1527,16 @@ static int head_forward_impl(const agrl_head_params *p, const void *prepared,
     if (!p->use_pose) { adj = nullptr; masks = nullptr; }
     if (adj) masks = nullptr;
 
-    if (p->maps_nhwc && (((reinterpret_cast<uintptr_t>(x4_1) | reinterpret_cast<uintptr_t>(x4_2)) & 15u) != 0)) return AGRL_E_UNSUPPORTED;
-    const bool tma = !p->maps_nhwc && !p->pool_register_loads && hw == 128 && C % kTpCh == 0 &&
-                     ((reinterpret_cast<uintptr_t>(x4_1) | reinterpret_cast<uintptr_t>(x4_2)) & 15u) == 0;
+    // channels-last pooling loads four channels at once: maps aligned to four elements (16 B at fp32, 8 B at 16 bits);
+    // the bulk copies need 16-byte aligned sources whatever the element size
+    const uintptr_t maps_bits = reinterpret_cast<uintptr_t>(x4_1) | reinterpret_cast<uintptr_t>(x4_2);
+    const uintptr_t vec_align = (p->maps_dtype == AGRL_MAPS_FP32 ? 16u : 8u) - 1u;
+    if (p->maps_nhwc && (maps_bits & vec_align) != 0) return AGRL_E_UNSUPPORTED;
+    const bool tma = !p->maps_nhwc && !p->pool_register_loads && hw == 128 && C % kTpCh == 0 && (maps_bits & 15u) == 0;
     constexpr int64_t kMaxPerLaunch = 32768;           // grid.y / int index limits of the per-tracklet kernels
     for (int64_t b0 = 0; b0 < batch; b0 += kMaxPerLaunch) {
         const int64_t n = batch - b0 < kMaxPerLaunch ? batch - b0 : kMaxPerLaunch;
-        if ((rc = launch_pool(p, pr, hwk, x4_1, x4_2, out, ld_out, b0, n, S, hw, tma, st))) return rc;
+        if ((rc = launch_pool_any(p, pr, hwk, x4_1, x4_2, out, ld_out, b0, n, S, hw, tma, st))) return rc;
         if ((rc = launch_layers(p, pr, hwk, adj, masks, out, ld_out, nodes_out, b0, n, batch, S, st))) return rc;
     }
     return AGRL_OK;

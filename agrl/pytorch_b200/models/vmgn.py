@@ -22,6 +22,7 @@ from .. import _lib
 __all__ = ['vmgn', 'VMGN', 'pool_clips']
 
 RESNET50_URL = 'https://download.pytorch.org/models/resnet50-19c8e357.pth'
+_MAPS_DTYPES = {torch.bfloat16: _lib.MAPS_BF16, torch.float16: _lib.MAPS_FP16}
 
 
 def pyramid_splits(num_split):
@@ -208,7 +209,8 @@ class VMGN(nn.Module):
         return hit[1]
 
     def head(self, x4_1, x4_2, adj, seq_len, return_nodes=False, out=None):
-        """vmgn.py:296-321 on the GPU: (B*S,C,h,w) x2 + (B,V,V) -> (B, 2C).
+        """vmgn.py:296-321 on the GPU: (B*S,C,h,w) x2 + (B,V,V) -> (B, 2C) fp32.  The maps may be fp32, or both bf16 /
+        both fp16 (a backbone under torch.autocast): those are read without an fp32 copy, same result as ``.float()``.
         ``out``: optional preallocated (B, 2C) fp32 CUDA tensor (unit column stride) to write into."""
         lib = _lib.require_device()
         if not x4_1.is_cuda:
@@ -225,11 +227,21 @@ class VMGN(nn.Module):
         nhwc = (x4_1.dim() == 4 and C % 4 == 0 and not x4_1.is_contiguous()
                 and x4_1.is_contiguous(memory_format=torch.channels_last)
                 and x4_2.is_contiguous(memory_format=torch.channels_last))
+        # bf16 / fp16 maps (a backbone under torch.autocast) are pooled as they are, without an fp32 copy: the kernels
+        # convert exactly on load, so the result has the bits of the .float() route.  Channels-last pooling needs maps
+        # aligned to four elements; every other case keeps the .float() route.
+        maps_dtype = _MAPS_DTYPES.get(x4_1.dtype) if x4_2.dtype == x4_1.dtype else None
         if nhwc:
-            x4_1, x4_2 = x4_1.float(), x4_2.float()                  # .float() keeps the memory format
+            native = (x4_1.data_ptr() | x4_2.data_ptr()) % 8 == 0
         else:
-            x4_1 = x4_1.float().contiguous()
-            x4_2 = x4_2.float().contiguous()
+            native = x4_1.is_contiguous() and x4_2.is_contiguous()
+        if maps_dtype is None or not native:
+            maps_dtype = _lib.MAPS_FP32
+            if nhwc:
+                x4_1, x4_2 = x4_1.float(), x4_2.float()              # .float() keeps the memory format
+            else:
+                x4_1 = x4_1.float().contiguous()
+                x4_2 = x4_2.float().contiguous()
         compact = False
         if self.use_pose:
             # adj: the reference's dense (B, V, V) fp32 graph, or the three part-membership masks per tracklet it is
@@ -243,7 +255,7 @@ class VMGN(nn.Module):
         with torch.cuda.device(dev):
             stream = torch.cuda.current_stream(dev).cuda_stream
             P, tensors, key = self._head_params()
-            P.maps_nhwc = int(nhwc)
+            P.maps_nhwc, P.maps_dtype = int(nhwc), maps_dtype
             prepared = self._prepared(lib, P, key, dev, stream)
             wsb = lib.agrl_head_workspace_bytes(ctypes.byref(P), B, seq_len)
             ws = self._ws.get((dev, stream))                         # one workspace per (device, stream)

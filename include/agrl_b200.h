@@ -312,13 +312,22 @@ typedef struct agrl_head_params {
                                      (needs C % 512 == 0; else this is ignored).  Changes the workspace size.          */
     int32_t pool_register_loads;  /* 1: the register-load pooling kernel even where the bulk-copy (TMA ring) kernel
                                      applies (16x8 maps, 16-byte aligned)                                             */
-    int32_t pool_stages;          /* 16 KiB ring stages per pooling CTA, 2..12; 0 = 4                                  */
+    int32_t pool_stages;          /* ring stages per pooling CTA, 2..12 (16 KiB each at fp32, 8 KiB at 16 bits);
+                                     0 = 4 at fp32, 12 at 16 bits                                                     */
     int32_t pool_no_l2_hint;      /* 1: no evict-first L2 hint on the pooling bulk copies                              */
     int32_t gemm_no_pair;         /* AGRL_SPLIT_FP16_E4M3 only.  Default: the layer GEMMs run as CTA pairs (tcgen05
                                      cta_group::2, 256 x 256 tiles, each CTA loads half of the W tile: a third less L2 -> SM
                                      traffic, which is what bounds this mode; 16.0 -> 12.7 ms per 11310-tracklet pass).
                                      1: one CTA per 128 x 256 tile.  Bit-identical results either way.                   */
+    int32_t maps_dtype;           /* element type of x4_1 / x4_2: AGRL_MAPS_FP32 (0, default), AGRL_MAPS_BF16 (1),
+                                     AGRL_MAPS_FP16 (2) -- the maps of a backbone run under autocast, read as they are
+                                     (half the bytes of fp32) and summed in fp32: the same bits as their fp32 copy gives.
+                                     Prepared buffer and workspace sizes do not depend on it.                          */
 } agrl_head_params;
+
+#define AGRL_MAPS_FP32 0
+#define AGRL_MAPS_BF16 1
+#define AGRL_MAPS_FP16 2
 
 /* bytes of the persistent, weight-derived buffer (bf16 planes of W, folded BN scale/shift) */
 AGRL_API size_t agrl_head_prepared_bytes(const agrl_head_params *p);
@@ -328,8 +337,9 @@ AGRL_API int    agrl_head_prepare_dev(const agrl_head_params *p, void *prepared_
 AGRL_API size_t agrl_head_workspace_bytes(const agrl_head_params *p, int64_t batch, int32_t seq_len);
 
 /*
- *   x4_1_dev, x4_2_dev  (batch*seq_len, C, h, w) fp32 NCHW contiguous (layer4_1 / layer4_2 outputs), or the same
- *                       tensors in channels-last memory when p->maps_nhwc (16-byte aligned)
+ *   x4_1_dev, x4_2_dev  (batch*seq_len, C, h, w) NCHW contiguous (layer4_1 / layer4_2 outputs), or the same
+ *                       tensors in channels-last memory when p->maps_nhwc (aligned to 4 elements); the pointers are
+ *                       typed float but point to elements of p->maps_dtype (fp32, bf16 or fp16)
  *   adj_dev             (batch, V, V) fp32, V = seq_len * 7 (dataset_loader.py:345-388); may be NULL
  *                       when use_pose == 0
  *   out_dev             (batch, 2*C) fp32, row stride ld_out: [BN(global mean) | BN(attention feature)]
