@@ -86,6 +86,13 @@ _SIGNATURES = {
     'agrl_rerank_workspace_bytes': (c_sz, [c_i64, c_i64, c_i64, c_i64]),
     'agrl_rerank_dev': (c_int, [c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_i64, c_i64, c_i64, c_i64, ctypes.c_double,
                                 c_vp, c_i64, c_vp, c_sz, c_vp]),
+    'agrl_rerank_shard_workspace_bytes': (c_sz, [c_i64, c_i64, c_i64, c_i64, c_i64]),
+    'agrl_rerank_shard_rows_dev': (c_int, [c_vp, c_i64, c_vp, c_i64, c_vp, c_i64, c_i64, c_i64, c_i64, c_i64, c_i64, c_i64,
+                                           c_i64, c_i64, c_vp, c_vp, c_sz, c_vp]),
+    'agrl_rerank_shard_expand_dev': (c_int, [c_vp, c_i64, c_i64, c_i64, c_i64, c_i64, c_i64, c_vp, c_vp, c_vp,
+                                             c_vp, c_sz, c_vp]),
+    'agrl_rerank_shard_finish_dev': (c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_i64, c_i64, c_i64, c_i64,
+                                             ctypes.c_double, c_vp, c_i64, c_vp, c_sz, c_vp]),
     'agrl_clip_pool_dev': (c_int, [c_vp, c_i64, c_i64, c_i64, c_i64, c_int, c_vp, c_i64, c_vp]),
     'agrl_head_prepared_bytes': (c_sz, [ctypes.POINTER(HeadParams)]),
     'agrl_head_prepare_dev': (c_int, [ctypes.POINTER(HeadParams), c_vp, c_sz, c_vp]),

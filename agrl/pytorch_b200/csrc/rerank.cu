@@ -12,6 +12,11 @@
 //   jaccard     per query the sum over shared columns of min(V[i,c], V[j,c]) through an inverted index of
 //               the gallery rows, in ascending column order, then 1 - t/(2-t) and the lambda blend         (:76-91)
 //
+// The kernels work on a set of *local* rows: all num_q queries, then a contiguous run of gallery rows that starts at
+// global gallery index goff.  Local row l is global row glob(l) = l (l < nq) or l + goff.  The single-device entry
+// uses goff = 0 (local == global); the gallery-sharded entries (agrl_rerank_shard_*) give each rank its own gallery
+// rows, so that D is held as (nq + n_own) x N rows and rank / V tables are exchanged between the three phases.
+//
 // Index work (ranks, sets) is exact; values are float32 with the reference's operation order (numpy's pairwise
 // sum for the weight normalisation, rows added in rank order for the mean, columns in ascending order for the
 // Jaccard sums).  The only departure is expf vs numpy's float32 exp (<= 2 ulp), so results agree to ~1e-6, not
@@ -20,24 +25,30 @@
 
 namespace agrl {
 
+__device__ __forceinline__ int glob_row(int l, int nq, int goff) { return l < nq ? l : l + goff; }
+
 struct RerankGeom {
     const float *qg, *qq, *gg;
     int64_t ld_qg, ld_qq, ld_gg;
     int nq, ng, N;
-    // element (r, c) of the block matrix [[qq, qg], [qg^T, gg]]
+    int goff;                          // local row l >= nq is global row l + goff
+    int gcol0;                         // gallery index of gg's first column (gg may hold a column slab only)
+    // element (r, c) of the block matrix [[qq, qg], [qg^T, gg]], global indices
     __device__ __forceinline__ float orig(int r, int c) const {
         if (r < nq) return c < nq ? qq[static_cast<size_t>(r) * ld_qq + c] : qg[static_cast<size_t>(r) * ld_qg + (c - nq)];
-        return c < nq ? qg[static_cast<size_t>(c) * ld_qg + (r - nq)] : gg[static_cast<size_t>(r - nq) * ld_gg + (c - nq)];
+        return c < nq ? qg[static_cast<size_t>(c) * ld_qg + (r - nq)] : gg[static_cast<size_t>(r - nq) * ld_gg + (c - nq - gcol0)];
     }
 };
 
 // ---- column maxima of orig^2 (non-negative floats: unsigned order == float order) ----------------------------
-__global__ void rr_colmax_kernel(RerankGeom g, unsigned int *colmax_bits) {
+// columns glob(l) of orig for local rows l in [row0, row1); colmax_bits is indexed by l
+__global__ void rr_colmax_kernel(RerankGeom g, int row0, int row1, unsigned int *colmax_bits) {
     __shared__ float part[8][33];
-    const int c = blockIdx.x * 32 + threadIdx.x;
+    const int l = row0 + blockIdx.x * 32 + threadIdx.x;
     const int r0 = blockIdx.y * 256;
     float m = 0.f;
-    if (c < g.N) {
+    if (l < row1) {
+        const int c = glob_row(l, g.nq, g.goff);
         const int r1 = min(r0 + 256, g.N);
         for (int r = r0 + threadIdx.y; r < r1; r += 8) {
             const float v = g.orig(r, c);
@@ -46,38 +57,38 @@ __global__ void rr_colmax_kernel(RerankGeom g, unsigned int *colmax_bits) {
     }
     part[threadIdx.y][threadIdx.x] = m;
     __syncthreads();
-    if (threadIdx.y == 0 && c < g.N) {
+    if (threadIdx.y == 0 && l < row1) {
 #pragma unroll
         for (int k = 1; k < 8; ++k) m = fmaxf(m, part[k][threadIdx.x]);
-        atomicMax(colmax_bits + c, __float_as_uint(m));
+        atomicMax(colmax_bits + l, __float_as_uint(m));
     }
 }
 
-// ---- D[i][j] = orig[j][i]^2 / colmax[i]: tiled transpose ------------------------------------------------------
-__global__ void rr_normalise_kernel(RerankGeom g, const float *colmax, float *D) {
+// ---- D[l][j] = orig[j][glob(l)]^2 / colmax[l] for local rows l in [row0, row1): tiled transpose -------------------
+__global__ void rr_normalise_kernel(RerankGeom g, int row0, int row1, const float *colmax, float *D) {
     __shared__ float tile[32][33];
-    const int i0 = blockIdx.y * 32, j0 = blockIdx.x * 32;
-    for (int k = threadIdx.y; k < 32; k += 8) {                 // read orig[j0+k][i0+tx]: coalesced along i
+    const int i0 = row0 + blockIdx.y * 32, j0 = blockIdx.x * 32;
+    for (int k = threadIdx.y; k < 32; k += 8) {                 // read orig[j0+k][glob(i0+tx)]: coalesced along i
         const int j = j0 + k, i = i0 + threadIdx.x;
         float v = 0.f;
-        if (j < g.N && i < g.N) { v = g.orig(j, i); v = __fmul_rn(v, v); }
+        if (j < g.N && i < row1) { v = g.orig(j, glob_row(i, g.nq, g.goff)); v = __fmul_rn(v, v); }
         tile[k][threadIdx.x] = v;
     }
     __syncthreads();
     for (int k = threadIdx.y; k < 32; k += 8) {                 // write D[i0+k][j0+tx]
         const int i = i0 + k, j = j0 + threadIdx.x;
-        if (i < g.N && j < g.N) D[static_cast<size_t>(i) * g.N + j] = __fdiv_rn(tile[threadIdx.x][k], colmax[i]);
+        if (i < row1 && j < g.N) D[static_cast<size_t>(i) * g.N + j] = __fdiv_rn(tile[threadIdx.x][k], colmax[i]);
     }
 }
 
-// ---- initial ranking: first K columns of every row, ties by index ------------------------------------------------
+// ---- initial ranking: first K columns of every row (local rows row0 + blockIdx.x), ties by index ------------------
 __global__ void __launch_bounds__(kRankThreads)
-rr_topk_kernel(const float *D, int N, int K, int buf_len, int32_t *rank) {
+rr_topk_kernel(const float *D, int N, int K, int buf_len, int row0, int32_t *rank) {
     extern __shared__ __align__(16) unsigned char rr_smem[];
     uint64_t *buf = reinterpret_cast<uint64_t *>(rr_smem);
     __shared__ int s_cnt;
     __shared__ unsigned long long s_thr;
-    const int i = blockIdx.x, tid = threadIdx.x;
+    const int i = row0 + blockIdx.x, tid = threadIdx.x;
     if (tid == 0) { s_cnt = 0; s_thr = kKeyMax; }
     __syncthreads();
     const int valid = select_topk(D + static_cast<size_t>(i) * N, N, K, buf_len, buf, &s_cnt, &s_thr, tid);
@@ -110,14 +121,16 @@ __device__ float np_pairwise_sum(const float *a, int n) {
     return __fadd_rn(np_pairwise_sum(a, n2), np_pairwise_sum(a + n2, n - n2));
 }
 
-// ---- k-reciprocal expansion + weights: one warp per row ---------------------------------------------------------
-// rank: (N, K) with K >= k1 + 1; entries < 0 mean "row shorter than K" (N < K).
+// ---- k-reciprocal expansion + weights: one warp per local row ---------------------------------------------------
+// rank: (N, K) with K >= k1 + 1, all global rows; entries < 0 mean "row shorter than K" (N < K).
+// D, idx, val, cnt: local rows [0, rows).
 struct ExpandArgs {
     const float *D;
     const int32_t *rank;
     int N, K, k1p, half;               // k1p = k1 + 1, half = round(k1 / 2) + 1 (both clipped to N)
     int cap;                           // capacity of a sparse row
     int32_t *idx; float *val; int32_t *cnt;
+    int rows, nq, goff;                // local rows and their global indices (glob_row)
 };
 
 constexpr int kExpandWarps = 4;
@@ -140,12 +153,13 @@ rr_expand_kernel(ExpandArgs a) {
     float *w = reinterpret_cast<float *>(reinterpret_cast<uint64_t *>(rr_smem) + static_cast<size_t>(kExpandWarps) * a.cap) +
                static_cast<size_t>(warp) * a.cap;
     __shared__ int32_t s_recip[kExpandWarps][32];
-    if (i >= a.N) return;
-    const int32_t *my = a.rank + static_cast<size_t>(i) * a.K;
+    if (i >= a.rows) return;
+    const int gi = glob_row(i, a.nq, a.goff);
+    const int32_t *my = a.rank + static_cast<size_t>(gi) * a.K;
 
     // k-reciprocal neighbours (:50-53), in rank order
     int f = lane < a.k1p ? my[lane] : -1;
-    const bool is_recip = f >= 0 && in_first(a.rank, a.K, f, a.k1p, i);
+    const bool is_recip = f >= 0 && in_first(a.rank, a.K, f, a.k1p, gi);
     const unsigned rmask = __ballot_sync(0xffffffffu, is_recip);
     const int n_recip = __popc(rmask);
     if (is_recip) s_recip[warp][__popc(rmask & ((1u << lane) - 1u))] = f;
@@ -203,9 +217,10 @@ rr_expand_kernel(ExpandArgs a) {
 // ---- query expansion: V_qe[i] = mean over i's first k2 neighbours' rows (:69-74) --------------------------------
 struct AverageArgs {
     const int32_t *rank; int N, K, k2;
-    const int32_t *idx; const float *val; const int32_t *cnt; int cap;          // input rows
-    int32_t *oidx; float *oval; int32_t *ocnt; int ocap;                        // output rows
+    const int32_t *idx; const float *val; const int32_t *cnt; int cap;          // input rows: all N, global
+    int32_t *oidx; float *oval; int32_t *ocnt; int ocap;                        // output rows: local
     int sort_len;                                                               // power of two >= k2 * cap
+    int nq, goff;                                                               // local row -> global (glob_row)
 };
 
 constexpr int kAvgThreads = 128;
@@ -218,7 +233,7 @@ rr_average_kernel(AverageArgs a) {
     const int i = blockIdx.x, tid = threadIdx.x;
     if (tid == 0) { s_n = 0; s_rows = 0; }
     __syncthreads();
-    const int32_t *my = a.rank + static_cast<size_t>(i) * a.K;
+    const int32_t *my = a.rank + static_cast<size_t>(glob_row(i, a.nq, a.goff)) * a.K;
     int rows = 0;
     for (int r = 0; r < a.k2; ++r) {
         const int nb = my[r];
@@ -269,11 +284,11 @@ rr_average_kernel(AverageArgs a) {
     if (tid == 0) a.ocnt[i] = out_n;
 }
 
-// ---- inverted index over the gallery rows (:76-78) ---------------------------------------------------------------
+// ---- inverted index over the gallery rows (:76-78): sparse rows row0 + blockIdx.x are gallery columns blockIdx.x --
 struct SparseRows { const int32_t *idx; const float *val; const int32_t *cnt; int cap; };
 
-__global__ void rr_inv_count_kernel(SparseRows v, int nq, int N, int32_t *col_cnt) {
-    const int j = nq + blockIdx.x;
+__global__ void rr_inv_count_kernel(SparseRows v, int row0, int32_t *col_cnt) {
+    const int j = row0 + blockIdx.x;
     const int c = v.cnt[j];
     for (int t = threadIdx.x; t < c; t += blockDim.x) atomicAdd(col_cnt + v.idx[static_cast<size_t>(j) * v.cap + t], 1);
 }
@@ -300,23 +315,24 @@ rr_scan_kernel(const int32_t *cnt, int n, int32_t *off) {
     if (tid == 1023) off[n] = s_part[1023];
 }
 
-__global__ void rr_inv_fill_kernel(SparseRows v, int nq, const int32_t *col_off, int32_t *col_cur,
+__global__ void rr_inv_fill_kernel(SparseRows v, int row0, const int32_t *col_off, int32_t *col_cur,
                                    int32_t *inv_row, float *inv_val) {
-    const int j = nq + blockIdx.x;
+    const int j = row0 + blockIdx.x;
     const int c = v.cnt[j];
     for (int t = threadIdx.x; t < c; t += blockDim.x) {
         const int col = v.idx[static_cast<size_t>(j) * v.cap + t];
         const int pos = col_off[col] + atomicAdd(col_cur + col, 1);      // order inside a column is irrelevant:
-        inv_row[pos] = j - nq;                                           // its entries touch distinct gallery rows
+        inv_row[pos] = blockIdx.x;                                       // its entries touch distinct gallery rows
         inv_val[pos] = v.val[static_cast<size_t>(j) * v.cap + t];
     }
 }
 
 // ---- Jaccard distance + blend: one CTA per query (:80-91) ------------------------------------------------------------
+// v rows 0..nq are the queries; the output block has ng columns, blended with D[i][dcol0 + j] (D row stride N)
 struct JaccardArgs {
     SparseRows v;
     const int32_t *col_off, *inv_row; const float *inv_val;
-    const float *D; int nq, ng, N;
+    const float *D; int dcol0, ng, N;
     float keep, lam;                   // (float)(1 - lambda), (float)lambda
     float *out; int64_t ld_out;
 };
@@ -339,7 +355,7 @@ rr_jaccard_kernel(JaccardArgs a) {
         }
         __syncthreads();
     }
-    const float *Drow = a.D + static_cast<size_t>(i) * a.N + a.nq;
+    const float *Drow = a.D + static_cast<size_t>(i) * a.N + a.dcol0;
     for (int j = tid; j < a.ng; j += kRankThreads) {
         const float tm = t_min[j];
         const float jac = __fsub_rn(1.0f, __fdiv_rn(tm, __fsub_rn(2.0f, tm)));
@@ -365,21 +381,23 @@ struct RerankWs {
     size_t bytes;
 };
 
-static RerankWs carve_rerank(void *buf, int64_t nq, int64_t ng, int k1, int k2) {
+// rows: local rows of D (all N on one device); n_inv: gallery rows of the inverted index; own_tables: the rank table
+// and the expansion rows live in the workspace (single device) rather than in caller buffers (sharded)
+static RerankWs carve_rerank(void *buf, int64_t rows, int64_t N, int64_t n_inv, int k1, int k2, bool own_tables) {
     Carver c(buf);
     RerankWs w;
-    const size_t N = static_cast<size_t>(nq + ng);
+    const size_t R = static_cast<size_t>(rows), T = own_tables ? static_cast<size_t>(N) : 0;
     const int half = round_half_even_half(k1) + 1;
     w.K = (k1 + 1 > k2) ? k1 + 1 : k2;
     w.cap1 = pow2_at_least((k1 + 1) * (half + 1));
     w.capq = (k2 == 1) ? w.cap1 : k2 * (k1 + 1) * (half + 1);
-    w.colmax = c.take<unsigned int>(N);
-    w.D = c.take<float>(N * N);
-    w.rank = c.take<int32_t>(N * w.K);
-    w.v1_idx = c.take<int32_t>(N * w.cap1); w.v1_val = c.take<float>(N * w.cap1); w.v1_cnt = c.take<int32_t>(N);
-    w.vq_idx = c.take<int32_t>(N * w.capq); w.vq_val = c.take<float>(N * w.capq); w.vq_cnt = c.take<int32_t>(N);
+    w.colmax = c.take<unsigned int>(R);
+    w.D = c.take<float>(R * N);
+    w.rank = c.take<int32_t>(T * w.K);
+    w.v1_idx = c.take<int32_t>(T * w.cap1); w.v1_val = c.take<float>(T * w.cap1); w.v1_cnt = c.take<int32_t>(T);
+    w.vq_idx = c.take<int32_t>(R * w.capq); w.vq_val = c.take<float>(R * w.capq); w.vq_cnt = c.take<int32_t>(R);
     w.col_cnt = c.take<int32_t>(N + 1); w.col_off = c.take<int32_t>(N + 1); w.col_cur = c.take<int32_t>(N + 1);
-    w.inv_row = c.take<int32_t>(static_cast<size_t>(ng) * w.capq); w.inv_val = c.take<float>(static_cast<size_t>(ng) * w.capq);
+    w.inv_row = c.take<int32_t>(static_cast<size_t>(n_inv) * w.capq); w.inv_val = c.take<float>(static_cast<size_t>(n_inv) * w.capq);
     w.bytes = c.total();
     return w;
 }
@@ -391,13 +409,96 @@ static int rerank_args_ok(int64_t nq, int64_t ng, int64_t k1, int64_t k2) {
     return AGRL_OK;
 }
 
+// Per-rank limits of the sharded form.  Positions into D are 64-bit; the column-maximum grid has (N + 255) / 256 rows
+// (<= 65535), t_min holds n_own floats in shared memory, and the inverted index (<= n_own * k2 * 527 entries) has
+// int32 offsets.
+constexpr int64_t kShardMaxN = 16000000;
+constexpr int64_t kShardMaxOwn = 50000;
+
+static int shard_args_ok(int64_t nq, int64_t ng, int64_t n_own, int64_t k1, int64_t k2) {
+    if (nq < 1 || ng < 1 || n_own < 0 || n_own > ng || k1 < 1 || k2 < 1) return AGRL_E_INVALID;
+    if (k1 > 30 || k2 > 8) return AGRL_E_UNSUPPORTED;
+    if (n_own > kShardMaxOwn || nq + ng > kShardMaxN) return AGRL_E_UNSUPPORTED;
+    return AGRL_OK;
+}
+
+// ---- the three stages, shared by the single-device and the sharded entries -----------------------------------------
+// D rows and the initial ranking of local rows [row0, row1); rank is indexed by local row, row stride K
+static int launch_rows(const RerankGeom &g, int row0, int row1, int K, unsigned int *colmax, float *D, int32_t *rank,
+                       cudaStream_t st) {
+    const int n = row1 - row0, N = g.N;
+    if (n == 0) return AGRL_OK;
+    AGRL_CUDA_TRY(cudaMemsetAsync(colmax + row0, 0, sizeof(unsigned int) * n, st));
+    rr_colmax_kernel<<<dim3((n + 31) / 32, (N + 255) / 256), dim3(32, 8), 0, st>>>(g, row0, row1, colmax);
+    AGRL_LAUNCH_CHECK(st, "rr_colmax");
+    rr_normalise_kernel<<<dim3((N + 31) / 32, (n + 31) / 32), dim3(32, 8), 0, st>>>(g, row0, row1,
+                                                                                    reinterpret_cast<const float *>(colmax), D);
+    AGRL_LAUNCH_CHECK(st, "rr_normalise");
+    int buf_len = pow2_at_least(2 * K);
+    if (buf_len < 2 * kMarsTile) buf_len = 2 * kMarsTile;
+    rr_topk_kernel<<<n, kRankThreads, static_cast<size_t>(buf_len) * 8, st>>>(D, N, K, buf_len, row0, rank);
+    AGRL_LAUNCH_CHECK(st, "rr_topk");
+    return AGRL_OK;
+}
+
+// k-reciprocal rows of the local rows [0, rows) from the full rank table
+static int launch_expand(const float *D, const int32_t *rank, int N, int K, int k1, int rows, int nq, int goff,
+                         int cap1, int32_t *idx, float *val, int32_t *cnt, cudaStream_t st) {
+    if (rows == 0) return AGRL_OK;
+    const int half = round_half_even_half(k1) + 1;
+    ExpandArgs ea{D, rank, N, K, k1 + 1 < N ? k1 + 1 : N, half < N ? half : N, cap1, idx, val, cnt, rows, nq, goff};
+    const size_t esmem = static_cast<size_t>(kExpandWarps) * cap1 * (8 + 4);
+    AGRL_CUDA_TRY(cudaFuncSetAttribute(rr_expand_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(esmem)));
+    rr_expand_kernel<<<(rows + kExpandWarps - 1) / kExpandWarps, 32 * kExpandWarps, esmem, st>>>(ea);
+    AGRL_LAUNCH_CHECK(st, "rr_expand");
+    return AGRL_OK;
+}
+
+// query expansion of the local rows, inverted index over the n_own local gallery rows, Jaccard + blend of every query
+// against them.  rank and v1 hold all N rows (global); D and the workspace's vq rows are local.
+static int launch_finish(const RerankWs &w, const int32_t *rank, SparseRows v1, int N, int nq, int goff, int n_own,
+                         int k2, double lambda_value, float *out, int64_t ld_out, cudaStream_t st) {
+    const int rows = nq + n_own;
+    SparseRows v = v1;
+    int inv_row0 = nq + goff;
+    if (k2 != 1) {
+        const int sort_len = pow2_at_least(k2 * w.cap1);
+        AverageArgs aa{rank, N, w.K, k2, v1.idx, v1.val, v1.cnt, v1.cap,
+                       w.vq_idx, w.vq_val, w.vq_cnt, w.capq, sort_len, nq, goff};
+        const size_t asmem = static_cast<size_t>(sort_len) * 8;
+        AGRL_CUDA_TRY(cudaFuncSetAttribute(rr_average_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(asmem)));
+        rr_average_kernel<<<rows, kAvgThreads, asmem, st>>>(aa);
+        AGRL_LAUNCH_CHECK(st, "rr_average");
+        v = SparseRows{w.vq_idx, w.vq_val, w.vq_cnt, w.capq};
+        inv_row0 = nq;
+    }
+    if (n_own == 0) return AGRL_OK;
+
+    AGRL_CUDA_TRY(cudaMemsetAsync(w.col_cnt, 0, sizeof(int32_t) * (N + 1), st));
+    AGRL_CUDA_TRY(cudaMemsetAsync(w.col_cur, 0, sizeof(int32_t) * (N + 1), st));
+    rr_inv_count_kernel<<<n_own, 128, 0, st>>>(v, inv_row0, w.col_cnt);
+    AGRL_LAUNCH_CHECK(st, "rr_inv_count");
+    rr_scan_kernel<<<1, 1024, 0, st>>>(w.col_cnt, N, w.col_off);
+    AGRL_LAUNCH_CHECK(st, "rr_scan");
+    rr_inv_fill_kernel<<<n_own, 128, 0, st>>>(v, inv_row0, w.col_off, w.col_cur, w.inv_row, w.inv_val);
+    AGRL_LAUNCH_CHECK(st, "rr_inv_fill");
+
+    JaccardArgs ja{v, w.col_off, w.inv_row, w.inv_val, w.D, nq + goff, n_own, N,
+                   static_cast<float>(1.0 - lambda_value), static_cast<float>(lambda_value), out, ld_out};
+    const size_t jsmem = static_cast<size_t>(n_own) * 4;
+    AGRL_CUDA_TRY(cudaFuncSetAttribute(rr_jaccard_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(jsmem)));
+    rr_jaccard_kernel<<<nq, kRankThreads, jsmem, st>>>(ja);
+    AGRL_LAUNCH_CHECK(st, "rr_jaccard");
+    return AGRL_OK;
+}
+
 }  // namespace agrl
 
 using namespace agrl;
 
 extern "C" size_t agrl_rerank_workspace_bytes(int64_t num_q, int64_t num_g, int64_t k1, int64_t k2) {
     if (rerank_args_ok(num_q, num_g, k1, k2)) return 0;
-    return carve_rerank(nullptr, num_q, num_g, static_cast<int>(k1), static_cast<int>(k2)).bytes;
+    return carve_rerank(nullptr, num_q + num_g, num_q + num_g, num_g, static_cast<int>(k1), static_cast<int>(k2), true).bytes;
 }
 
 extern "C" int agrl_rerank_dev(const float *q_g, int64_t ld_qg, const float *q_q, int64_t ld_qq,
@@ -409,58 +510,75 @@ extern "C" int agrl_rerank_dev(const float *q_g, int64_t ld_qg, const float *q_q
     if (rc) return rc;
     if (ld_qg < num_g || ld_qq < num_q || ld_gg < num_g || ld_out < num_g) return AGRL_E_INVALID;
     if ((rc = agrl_device_ok())) return rc;
-    RerankWs w = carve_rerank(ws, num_q, num_g, static_cast<int>(k1), static_cast<int>(k2));
+    RerankWs w = carve_rerank(ws, num_q + num_g, num_q + num_g, num_g, static_cast<int>(k1), static_cast<int>(k2), true);
     if (!ws || ws_bytes < w.bytes) return AGRL_E_WORKSPACE;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const int nq = static_cast<int>(num_q), ng = static_cast<int>(num_g), N = nq + ng;
-    RerankGeom g{q_g, q_q, g_g, ld_qg, ld_qq, ld_gg, nq, ng, N};
+    RerankGeom g{q_g, q_q, g_g, ld_qg, ld_qq, ld_gg, nq, ng, N, 0, 0};
+    if ((rc = launch_rows(g, 0, N, w.K, w.colmax, w.D, w.rank, st))) return rc;
+    if ((rc = launch_expand(w.D, w.rank, N, w.K, static_cast<int>(k1), N, nq, 0, w.cap1, w.v1_idx, w.v1_val, w.v1_cnt, st)))
+        return rc;
+    return launch_finish(w, w.rank, SparseRows{w.v1_idx, w.v1_val, w.v1_cnt, w.cap1}, N, nq, 0, ng, static_cast<int>(k2),
+                         lambda_value, out, ld_out, st);
+}
 
-    AGRL_CUDA_TRY(cudaMemsetAsync(w.colmax, 0, sizeof(unsigned int) * N, st));
-    rr_colmax_kernel<<<dim3((N + 31) / 32, (N + 255) / 256), dim3(32, 8), 0, st>>>(g, w.colmax);
-    AGRL_LAUNCH_CHECK(st, "rr_colmax");
-    rr_normalise_kernel<<<dim3((N + 31) / 32, (N + 31) / 32), dim3(32, 8), 0, st>>>(g, reinterpret_cast<const float *>(w.colmax), w.D);
-    AGRL_LAUNCH_CHECK(st, "rr_normalise");
+// ---- gallery-sharded re-ranking (include/agrl_b200.h; the decomposition is DESIGN.md section 8) -------------------------
+extern "C" size_t agrl_rerank_shard_workspace_bytes(int64_t num_q, int64_t num_g, int64_t n_own, int64_t k1, int64_t k2) {
+    if (shard_args_ok(num_q, num_g, n_own, k1, k2)) return 0;
+    return carve_rerank(nullptr, num_q + n_own, num_q + num_g, n_own, static_cast<int>(k1), static_cast<int>(k2), false).bytes;
+}
 
-    const int K = w.K;
-    int buf_len = pow2_at_least(2 * K);
-    if (buf_len < 2 * kMarsTile) buf_len = 2 * kMarsTile;
-    rr_topk_kernel<<<N, kRankThreads, static_cast<size_t>(buf_len) * 8, st>>>(w.D, N, K, buf_len, w.rank);
-    AGRL_LAUNCH_CHECK(st, "rr_topk");
-
-    const int half = round_half_even_half(static_cast<int>(k1)) + 1;
-    ExpandArgs ea{w.D, w.rank, N, K, static_cast<int>(k1) + 1 < N ? static_cast<int>(k1) + 1 : N, half < N ? half : N, w.cap1,
-                  w.v1_idx, w.v1_val, w.v1_cnt};
-    const size_t esmem = static_cast<size_t>(kExpandWarps) * w.cap1 * (8 + 4);
-    AGRL_CUDA_TRY(cudaFuncSetAttribute(rr_expand_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(esmem)));
-    rr_expand_kernel<<<(N + kExpandWarps - 1) / kExpandWarps, 32 * kExpandWarps, esmem, st>>>(ea);
-    AGRL_LAUNCH_CHECK(st, "rr_expand");
-
-    SparseRows v{w.v1_idx, w.v1_val, w.v1_cnt, w.cap1};
-    if (k2 != 1) {
-        const int sort_len = pow2_at_least(static_cast<int>(k2) * w.cap1);
-        AverageArgs aa{w.rank, N, K, static_cast<int>(k2), w.v1_idx, w.v1_val, w.v1_cnt, w.cap1,
-                       w.vq_idx, w.vq_val, w.vq_cnt, w.capq, sort_len};
-        const size_t asmem = static_cast<size_t>(sort_len) * 8;
-        AGRL_CUDA_TRY(cudaFuncSetAttribute(rr_average_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(asmem)));
-        rr_average_kernel<<<N, kAvgThreads, asmem, st>>>(aa);
-        AGRL_LAUNCH_CHECK(st, "rr_average");
-        v = SparseRows{w.vq_idx, w.vq_val, w.vq_cnt, w.capq};
-    }
-
-    AGRL_CUDA_TRY(cudaMemsetAsync(w.col_cnt, 0, sizeof(int32_t) * (N + 1), st));
-    AGRL_CUDA_TRY(cudaMemsetAsync(w.col_cur, 0, sizeof(int32_t) * (N + 1), st));
-    rr_inv_count_kernel<<<ng, 128, 0, st>>>(v, nq, N, w.col_cnt);
-    AGRL_LAUNCH_CHECK(st, "rr_inv_count");
-    rr_scan_kernel<<<1, 1024, 0, st>>>(w.col_cnt, N, w.col_off);
-    AGRL_LAUNCH_CHECK(st, "rr_scan");
-    rr_inv_fill_kernel<<<ng, 128, 0, st>>>(v, nq, w.col_off, w.col_cur, w.inv_row, w.inv_val);
-    AGRL_LAUNCH_CHECK(st, "rr_inv_fill");
-
-    JaccardArgs ja{v, w.col_off, w.inv_row, w.inv_val, w.D, nq, ng, N,
-                   static_cast<float>(1.0 - lambda_value), static_cast<float>(lambda_value), out, ld_out};
-    const size_t jsmem = static_cast<size_t>(ng) * 4;
-    AGRL_CUDA_TRY(cudaFuncSetAttribute(rr_jaccard_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(jsmem)));
-    rr_jaccard_kernel<<<nq, kRankThreads, jsmem, st>>>(ja);
-    AGRL_LAUNCH_CHECK(st, "rr_jaccard");
+static int shard_common(int64_t num_q, int64_t num_g, int64_t g_off, int64_t n_own, int64_t k1, int64_t k2,
+                        void *ws, size_t ws_bytes, RerankWs *w) {
+    int rc = shard_args_ok(num_q, num_g, n_own, k1, k2);
+    if (rc) return rc;
+    if (g_off < 0 || g_off + n_own > num_g) return AGRL_E_INVALID;
+    if ((rc = agrl_device_ok())) return rc;
+    *w = carve_rerank(ws, num_q + n_own, num_q + num_g, n_own, static_cast<int>(k1), static_cast<int>(k2), false);
+    if (!ws || ws_bytes < w->bytes) return AGRL_E_WORKSPACE;
     return AGRL_OK;
+}
+
+extern "C" int agrl_rerank_shard_rows_dev(const float *q_g, int64_t ld_qg, const float *q_q, int64_t ld_qq,
+                                          const float *g_cols, int64_t ld_gc, int64_t num_q, int64_t num_g,
+                                          int64_t g_off, int64_t n_own, int64_t row0, int64_t row1, int64_t k1, int64_t k2,
+                                          int32_t *rank_rows, void *ws, size_t ws_bytes, void *stream) {
+    if (!q_g || !q_q || !rank_rows) return AGRL_E_INVALID;
+    if (row0 < 0 || row1 < row0 || row1 > num_q + n_own || ld_qg < num_g || ld_qq < num_q) return AGRL_E_INVALID;
+    const int64_t gal0 = row0 > num_q ? row0 : num_q;                      // first local gallery row of the range
+    if (row1 > num_q && (!g_cols || ld_gc < row1 - gal0)) return AGRL_E_INVALID;
+    RerankWs w;
+    int rc = shard_common(num_q, num_g, g_off, n_own, k1, k2, ws, ws_bytes, &w);
+    if (rc) return rc;
+    const int nq = static_cast<int>(num_q), N = static_cast<int>(num_q + num_g);
+    RerankGeom g{q_g, q_q, g_cols, ld_qg, ld_qq, ld_gc, nq, static_cast<int>(num_g), N, static_cast<int>(g_off),
+                 static_cast<int>(g_off + gal0 - num_q)};
+    return launch_rows(g, static_cast<int>(row0), static_cast<int>(row1), w.K, w.colmax, w.D, rank_rows,
+                       static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int agrl_rerank_shard_expand_dev(const int32_t *rank_all, int64_t num_q, int64_t num_g, int64_t g_off,
+                                            int64_t n_own, int64_t k1, int64_t k2, int32_t *v_idx, float *v_val,
+                                            int32_t *v_cnt, void *ws, size_t ws_bytes, void *stream) {
+    if (!rank_all || !v_idx || !v_val || !v_cnt) return AGRL_E_INVALID;
+    RerankWs w;
+    int rc = shard_common(num_q, num_g, g_off, n_own, k1, k2, ws, ws_bytes, &w);
+    if (rc) return rc;
+    const int nq = static_cast<int>(num_q), N = static_cast<int>(num_q + num_g);
+    return launch_expand(w.D, rank_all, N, w.K, static_cast<int>(k1), nq + static_cast<int>(n_own), nq, static_cast<int>(g_off),
+                         w.cap1, v_idx, v_val, v_cnt, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int agrl_rerank_shard_finish_dev(const int32_t *rank_all, const int32_t *v_idx_all, const float *v_val_all,
+                                            const int32_t *v_cnt_all, int64_t num_q, int64_t num_g, int64_t g_off,
+                                            int64_t n_own, int64_t k1, int64_t k2, double lambda_value,
+                                            float *out, int64_t ld_out, void *ws, size_t ws_bytes, void *stream) {
+    if (!rank_all || !v_idx_all || !v_val_all || !v_cnt_all || (n_own > 0 && (!out || ld_out < n_own))) return AGRL_E_INVALID;
+    RerankWs w;
+    int rc = shard_common(num_q, num_g, g_off, n_own, k1, k2, ws, ws_bytes, &w);
+    if (rc) return rc;
+    const int N = static_cast<int>(num_q + num_g);
+    return launch_finish(w, rank_all, SparseRows{v_idx_all, v_val_all, v_cnt_all, w.cap1}, N, static_cast<int>(num_q),
+                         static_cast<int>(g_off), static_cast<int>(n_own), static_cast<int>(k2), lambda_value, out, ld_out,
+                         static_cast<cudaStream_t>(stream));
 }

@@ -10,9 +10,15 @@ one-shot collectives of NVSwitch are the right shape.  The graph head needs no c
 
     cmc, mAP = evaluate_mars_sharded(qf, gf_local, q_pids, g_pids_local, q_camids, g_camids_local)
 
+k-reciprocal re-ranking shards too (``re_ranking_sharded``, or ``re_rank=True`` above): every rank holds all
+features after one all-gather, computes the D rows of its queries + gallery rows, and two all-gathers of sparse
+tables (rank lists, k-reciprocal rows) later produces its (num_q x num_g_r) block of the re-ranked matrix.
+
 ``ops`` lets the tests drive the same plumbing with CPU stand-ins under gloo; the product default is
 the CUDA implementation and there is no fallback.
 """
+from types import SimpleNamespace
+
 import numpy as np
 import torch
 import torch.distributed as dist
@@ -202,6 +208,67 @@ class CudaOps(object):
         _raise_status(int(host.view(torch.int32)[1]) | st_parts)
         return cmc.cpu().numpy(), float(host[0])
 
+    # ---- gallery-sharded k-reciprocal re-ranking (agrl_rerank_shard_*) ----------------------------------------------
+    def rerank_rows(self, qg, qq, gg_slabs, offset, n_own, max_own, k1, k2):
+        """Phase A.  ``gg_slabs`` yields (s0, g_g[:, offset + s0 : offset + s0 + w]) in order; each slab is released
+        once consumed.  Returns (state for the next two phases, int32 rank rows (num_q + n_own, K))."""
+        lib, dev = self.lib, qg.device
+        nq, ng = qg.shape
+        if lib.agrl_rerank_shard_workspace_bytes(nq, ng, max_own, k1, k2) == 0:      # the same verdict on every rank
+            _lib.check(_lib.E_UNSUPPORTED)
+        wsb = lib.agrl_rerank_shard_workspace_bytes(nq, ng, n_own, k1, k2)
+        K, _ = rerank_row_dims(k1, k2)
+        st = SimpleNamespace(ws=torch.empty(wsb, dtype=torch.uint8, device=dev), wsb=wsb, nq=nq, ng=ng, offset=offset,
+                             n_own=n_own, k1=k1, k2=k2)
+        rank_rows = torch.empty(nq + n_own, K, dtype=torch.int32, device=dev)
+        with torch.cuda.device(dev):
+            stream = torch.cuda.current_stream(dev).cuda_stream
+
+            def rows(slab, r0, r1):
+                _lib.check(lib.agrl_rerank_shard_rows_dev(
+                    qg.data_ptr(), qg.stride(0), qq.data_ptr(), qq.stride(0), slab.data_ptr() if slab is not None else None,
+                    slab.stride(0) if slab is not None else 0, nq, ng, offset, n_own, r0, r1, k1, k2, rank_rows.data_ptr(),
+                    st.ws.data_ptr(), wsb, stream))
+            rows(None, 0, nq)
+            for s0, slab in gg_slabs:
+                rows(slab.contiguous(), nq + s0, nq + s0 + slab.shape[1])
+        return st, rank_rows
+
+    def rerank_expand(self, st, rank_all):
+        """Phase B: this rank's k-reciprocal rows (idx int32, val fp32 (num_q + n_own, cap); cnt int32 (num_q + n_own))."""
+        dev = rank_all.device
+        _, cap = rerank_row_dims(st.k1, st.k2)
+        rows = st.nq + st.n_own
+        idx = torch.empty(rows, cap, dtype=torch.int32, device=dev)
+        val = torch.empty(rows, cap, dtype=torch.float32, device=dev)
+        cnt = torch.empty(rows, dtype=torch.int32, device=dev)
+        with torch.cuda.device(dev):
+            _lib.check(self.lib.agrl_rerank_shard_expand_dev(
+                rank_all.data_ptr(), st.nq, st.ng, st.offset, st.n_own, st.k1, st.k2, idx.data_ptr(), val.data_ptr(),
+                cnt.data_ptr(), st.ws.data_ptr(), st.wsb, torch.cuda.current_stream(dev).cuda_stream))
+        return idx, val, cnt
+
+    def rerank_finish(self, st, rank_all, idx_all, val_all, cnt_all, lambda_value):
+        """Phase C: this rank's (num_q, n_own) block of the re-ranked distance matrix."""
+        dev = rank_all.device
+        out = torch.empty(st.nq, st.n_own, dtype=torch.float32, device=dev)
+        with torch.cuda.device(dev):
+            _lib.check(self.lib.agrl_rerank_shard_finish_dev(
+                rank_all.data_ptr(), idx_all.data_ptr(), val_all.data_ptr(), cnt_all.data_ptr(), st.nq, st.ng, st.offset,
+                st.n_own, st.k1, st.k2, float(lambda_value), out.data_ptr() if st.n_own else None, max(st.n_own, 1),
+                st.ws.data_ptr(), st.wsb, torch.cuda.current_stream(dev).cuda_stream))
+        return out
+
+
+def rerank_row_dims(k1, k2):
+    """(K, cap): widths of the rank-table rows and of the k-reciprocal rows exchanged by the sharded re-ranking
+    (include/agrl_b200.h): K = max(k1 + 1, k2), cap = least power of two >= (k1 + 1)(round(k1 / 2) + 2)."""
+    need = (k1 + 1) * (int(np.around(k1 / 2.)) + 2)
+    cap = 2
+    while cap < need:
+        cap *= 2
+    return max(k1 + 1, k2), cap
+
 
 def _as_dev_i64(x, dev):
     if isinstance(x, torch.Tensor):
@@ -232,13 +299,65 @@ def _broadcast_queries(qf, qp, qc, group):
     """rank 0's query features and labels to every rank: two collectives (features; both label vectors packed)"""
     src = dist.get_global_rank(group, 0) if group is not None else 0
     dist.broadcast(qf, src=src, group=group)
+    if qp is None:
+        return
     lab = torch.stack([qp, qc])
     dist.broadcast(lab, src=src, group=group)
     qp.copy_(lab[0]); qc.copy_(lab[1])
 
 
+def _gather_shard_rows(t, head, counts, rank, group):
+    """t[:head] followed by every rank's rows t[head:] in rank order (one all-gather, padded to the largest shard)."""
+    world = len(counts)
+    if world == 1:
+        return t
+    most = max(counts)
+    pad = t.new_zeros((most,) + tuple(t.shape[1:]))
+    pad[:counts[rank]] = t[head:]
+    buf = t.new_empty((world * most,) + tuple(t.shape[1:]))
+    dist.all_gather_into_tensor(buf, pad, group=group)
+    return torch.cat([t[:head]] + [buf[r * most:r * most + c] for r, c in enumerate(counts)])
+
+
+RERANK_SLAB_BYTES = 1 << 31      # largest g_g column slab (num_g x columns fp32) alive at a time
+
+
+def re_ranking_sharded(qf, gf_local, metric='euclidean', k1=20, k2=6, lambda_value=0.3, group=None,
+                       broadcast_queries=True, ops=None, gallery_counts=None):
+    """k-reciprocal re-ranking (utils/re_ranking.py:30-94) of ``qf`` against the union of every rank's gallery shard.
+
+    Returns this rank's (num_q, num_g_r) block of the re-ranked distance matrix as a CUDA tensor: bit-identical to
+    ``re_ranking_dev(qg, qq, gg)[:, off:off + num_g_r]`` with the three matrices from ``compute_distance_matrix`` on
+    the whole sets and ``off`` the global index of this rank's first gallery row.  Arguments as in
+    evaluate_mars_sharded.  Exchanges: the gallery features (all-gather), then the gallery rows of the rank table
+    (num_g x K int32) and of the k-reciprocal rows (num_g x cap x 8 B + counts).  Per-rank limits: k1 <= 30, k2 <= 8,
+    num_g_r <= 50000 (agrl_rerank_shard_workspace_bytes); the D rows take 4 (num_q + num_g_r)(num_q + num_g) bytes.
+    """
+    if metric not in ('euclidean', 'cosine'):
+        raise ValueError('Unknown distance metric: {}. Please choose either "euclidean" or "cosine"'.format(metric))
+    world = dist.get_world_size(group) if dist.is_initialized() else 1
+    ops = ops or CudaOps()
+    qf, gf_own = qf.contiguous(), gf_local.contiguous()
+    if world > 1 and broadcast_queries:
+        _broadcast_queries(qf, None, None, group)
+    counts, rank = _shard_layout(gf_own.shape[0], qf.device, world, group, gallery_counts)
+    nq, ng, n_own, offset = qf.shape[0], sum(counts), counts[rank], sum(counts[:rank])
+    gf_all = _gather_shard_rows(gf_own, 0, counts, rank, group)
+    # the operand roles of the single-device path: qq = d(q, q), qg = d(q, g), gg[:, own] = d(g, g_own)
+    qq = ops.distance(qf, qf, metric)
+    qg = ops.distance(qf, gf_all, metric)
+    width = max(1, RERANK_SLAB_BYTES // (4 * ng))
+    slabs = ((s0, ops.distance(gf_all, gf_own[s0:s0 + width], metric)) for s0 in range(0, n_own, width))
+    st, rank_rows = ops.rerank_rows(qg, qq, slabs, offset, n_own, max(counts), k1, k2)
+    del qq, qg, gf_all
+    rank_all = _gather_shard_rows(rank_rows, nq, counts, rank, group)
+    v_all = [_gather_shard_rows(t, nq, counts, rank, group) for t in ops.rerank_expand(st, rank_all)]
+    return ops.rerank_finish(st, rank_all, v_all[0], v_all[1], v_all[2], lambda_value)
+
+
 def evaluate_mars_sharded(qf, gf_local, q_pids, g_pids_local, q_camids, g_camids_local, metric='euclidean',
-                          max_rank=50, group=None, broadcast_queries=True, ops=None, fused=None, gallery_counts=None):
+                          max_rank=50, group=None, broadcast_queries=True, ops=None, fused=None, gallery_counts=None,
+                          re_rank=False, k1=20, k2=6, lambda_value=0.3):
     """MARS-metric CMC/mAP (rank.py:160-212) of ``qf`` against the union of every rank's gallery shard.
 
     qf (num_q, d) and the query labels must be the same on every rank (``broadcast_queries`` copies
@@ -247,6 +366,9 @@ def evaluate_mars_sharded(qf, gf_local, q_pids, g_pids_local, q_camids, g_camids
     ``gallery_counts``: rows of every rank's shard when the caller knows them (skips one all-gather and its host sync).
     ``fused``: distance -> top-k in the GEMM epilogue, no (num_q x num_g_r) matrix (default: from FUSED_MIN_GALLERY
     gallery rows per shard on; same result either way).
+    ``re_rank``: rank the k-reciprocal re-ranked distances (re_ranking_sharded with k1, k2, lambda_value) instead,
+    through the per-shard top-k + merge (``fused`` does not apply): the CMC/mAP of re_ranking_dev followed by
+    evaluate_rank(use_metric_mars=True) on one device.
     Returns (numpy.float64[max_rank], numpy.float64) on every rank.
     """
     world = dist.get_world_size(group) if dist.is_initialized() else 1
@@ -266,7 +388,11 @@ def evaluate_mars_sharded(qf, gf_local, q_pids, g_pids_local, q_camids, g_camids
 
     if fused is None:
         fused = gf_local.shape[0] >= FUSED_MIN_GALLERY and hasattr(ops, 'topk_fused') and max_rank <= 256
-    if fused:
+    if re_rank:
+        d = re_ranking_sharded(qf, gf_local, metric, k1, k2, lambda_value, group=group, broadcast_queries=False, ops=ops,
+                               gallery_counts=counts)
+        keys, cls, ngood, status = ops.partial(d, qp, gp, qc, gc, max_rank, offset)
+    elif fused:
         from .metrics.distance import PreparedOperand
         keys, cls, ngood, status = ops.topk_fused(PreparedOperand(qf, metric, ops.split), PreparedOperand(gf_local, metric, ops.split),
                                                   qp, gp, qc, gc, max_rank, offset)

@@ -395,6 +395,40 @@ AGRL_API int    agrl_rerank_dev(const float *q_g_dev, int64_t ld_qg, const float
                        int64_t k1, int64_t k2, double lambda_value,
                        float *out_dev, int64_t ld_out, void *workspace_dev, size_t workspace_bytes, void *stream);
 
+/* ---- gallery-sharded k-reciprocal re-ranking: the same output split over ranks ------------------------------------
+ * Rank r owns the gallery rows [g_off, g_off + n_own) of the global gallery (num_g rows, N = num_q + num_g).  Its
+ * n_loc = num_q + n_own *local rows* are all queries, then its gallery rows: local row l is global row l (l < num_q)
+ * or l + g_off.  Three calls, with exchanges between them, give its block out[:, j] = re-ranked distance of every query
+ * to gallery item g_off + j, bit-identical to agrl_rerank_dev on the whole problem given the same distance bits.
+ *   rows    D rows (N fp32 each, in the workspace) and the stable top-K of the local rows [row0, row1) -> rank_rows.
+ *           q_g (num_q, num_g) and q_q (num_q, num_q) whole; g_cols (num_g, row1 - max(row0, num_q)), row stride ld_gc,
+ *           holds the g_g columns of the range's gallery rows: column t = distances of all gallery items to gallery item
+ *           g_off + max(row0, num_q) - num_q + t (NULL when row1 <= num_q).  Call it for any partition of [0, n_loc)
+ *           into ranges, e.g. the queries and then one call per column slab.
+ *   expand  after every rank's rows: rank_all (N, K) = the query rows (identical on every rank) and every rank's
+ *           gallery rows, in global order.  Writes this rank's k-reciprocal rows v_idx / v_val (n_loc, cap) and v_cnt
+ *           (n_loc): global column indices ascending, weights summing to 1.
+ *   finish  after every rank's expand: v_*_all = the query rows and every rank's gallery rows of v_*, (N, cap) and
+ *           (N), in global order.  Writes out (num_q, n_own), row stride ld_out (out may be NULL when n_own == 0).
+ * K = max(k1 + 1, k2) and cap = the least power of two >= (k1 + 1)(round_half_even(k1 / 2) + 2), both row strides.
+ * The workspace carries the per-rank state (D rows, query expansion, inverted index) from rows to finish: pass the
+ * same buffer to all three calls.  Its size is 4 n_loc N + 8 n_loc cap_q + 8 n_own cap_q + 12 (N + 1) + 8 n_loc bytes
+ * (+ alignment), cap_q = cap when k2 == 1 else k2 (k1 + 1)(round_half_even(k1 / 2) + 2): the D rows dominate.
+ * Limits per rank: 1 <= k1 <= 30, 1 <= k2 <= 8, 0 <= n_own <= 50000, N <= 16 000 000 (AGRL_E_UNSUPPORTED beyond;
+ * the workspace query returns 0).  Positions into D are 64-bit. */
+AGRL_API size_t agrl_rerank_shard_workspace_bytes(int64_t num_q, int64_t num_g, int64_t n_own, int64_t k1, int64_t k2);
+AGRL_API int    agrl_rerank_shard_rows_dev(const float *q_g_dev, int64_t ld_qg, const float *q_q_dev, int64_t ld_qq,
+                       const float *g_cols_dev, int64_t ld_gc, int64_t num_q, int64_t num_g, int64_t g_off, int64_t n_own,
+                       int64_t row0, int64_t row1, int64_t k1, int64_t k2, int32_t *rank_rows_dev,
+                       void *workspace_dev, size_t workspace_bytes, void *stream);
+AGRL_API int    agrl_rerank_shard_expand_dev(const int32_t *rank_all_dev, int64_t num_q, int64_t num_g, int64_t g_off,
+                       int64_t n_own, int64_t k1, int64_t k2, int32_t *v_idx_dev, float *v_val_dev, int32_t *v_cnt_dev,
+                       void *workspace_dev, size_t workspace_bytes, void *stream);
+AGRL_API int    agrl_rerank_shard_finish_dev(const int32_t *rank_all_dev, const int32_t *v_idx_all_dev,
+                       const float *v_val_all_dev, const int32_t *v_cnt_all_dev, int64_t num_q, int64_t num_g,
+                       int64_t g_off, int64_t n_own, int64_t k1, int64_t k2, double lambda_value,
+                       float *out_dev, int64_t ld_out, void *workspace_dev, size_t workspace_bytes, void *stream);
+
 /* Clip pooling of the `dense` / `skipdense` test sampling (train_vidreid_xent_htri.py:461-476):
  * feats (tracklets * clips, dim) with the clips of a tracklet consecutive -> out (tracklets, dim),
  * torch.mean(features, 0) (AVG) or torch.max(features, 0) values (MAX) over the clip axis. */
