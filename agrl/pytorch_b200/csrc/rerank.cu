@@ -21,6 +21,8 @@
 // sum for the weight normalisation, rows added in rank order for the mean, columns in ascending order for the
 // Jaccard sums).  The only departure is expf vs numpy's float32 exp (<= 2 ulp), so results agree to ~1e-6, not
 // bit for bit.  One CTA / warp per row; no atomics on floating-point data, so runs are reproducible.
+// NaN propagates as in numpy: a NaN in column c of the block matrix makes the column maximum NaN (np.max), so D row c
+// is all NaN, and the Jaccard minimum of a NaN weight is NaN (np.minimum).
 #include "topk.cuh"
 
 namespace agrl {
@@ -41,26 +43,29 @@ struct RerankGeom {
 };
 
 // ---- column maxima of orig^2 (non-negative floats: unsigned order == float order) ----------------------------
-// columns glob(l) of orig for local rows l in [row0, row1); colmax_bits is indexed by l
+// columns glob(l) of orig for local rows l in [row0, row1); colmax_bits is indexed by l.  A NaN square is kept as the
+// canonical NaN 0x7fffffff, which beats +inf (0x7f800000) in the unsigned maximum: NaN propagates as in np.max.
+__device__ __forceinline__ unsigned int colmax_bits_of(float sq) { return sq != sq ? 0x7fffffffu : __float_as_uint(sq); }
+
 __global__ void rr_colmax_kernel(RerankGeom g, int row0, int row1, unsigned int *colmax_bits) {
-    __shared__ float part[8][33];
+    __shared__ unsigned int part[8][33];
     const int l = row0 + blockIdx.x * 32 + threadIdx.x;
     const int r0 = blockIdx.y * 256;
-    float m = 0.f;
+    unsigned int m = 0u;
     if (l < row1) {
         const int c = glob_row(l, g.nq, g.goff);
         const int r1 = min(r0 + 256, g.N);
         for (int r = r0 + threadIdx.y; r < r1; r += 8) {
             const float v = g.orig(r, c);
-            m = fmaxf(m, __fmul_rn(v, v));
+            m = max(m, colmax_bits_of(__fmul_rn(v, v)));
         }
     }
     part[threadIdx.y][threadIdx.x] = m;
     __syncthreads();
     if (threadIdx.y == 0 && l < row1) {
 #pragma unroll
-        for (int k = 1; k < 8; ++k) m = fmaxf(m, part[k][threadIdx.x]);
-        atomicMax(colmax_bits + l, __float_as_uint(m));
+        for (int k = 1; k < 8; ++k) m = max(m, part[k][threadIdx.x]);
+        atomicMax(colmax_bits + l, m);
     }
 }
 
@@ -351,7 +356,8 @@ rr_jaccard_kernel(JaccardArgs a) {
         const int lo = a.col_off[c], hi = a.col_off[c + 1];
         for (int e = lo + tid; e < hi; e += kRankThreads) {
             const int j = a.inv_row[e];
-            t_min[j] = __fadd_rn(t_min[j], fminf(vi, a.inv_val[e]));
+            const float vj = a.inv_val[e];                        // np.minimum: NaN if either is NaN
+            t_min[j] = __fadd_rn(t_min[j], (vi != vi || vj != vj) ? __uint_as_float(0x7fffffffu) : fminf(vi, vj));
         }
         __syncthreads();
     }

@@ -35,13 +35,26 @@ def single_device(qf, gf, metric='euclidean', k1=20, k2=6, lam=0.3):
 def run_shards(qf, gf, bounds, metric='euclidean', k1=20, k2=6, lam=0.3, slab_cols=None):
     """every shard's phases A, B, C in sequence, with the exchanges as concatenations; returns the blocks side by side"""
     ops = sharded.CudaOps()
-    nq, ng = qf.shape[0], gf.shape[0]
+    outs, _, _ = run_phases(lambda: (ops.distance(qf, gf, metric), ops.distance(qf, qf, metric)),
+                            lambda c0, c1: ops.distance(gf, gf[c0:c1], metric), bounds, k1, k2, [lam], slab_cols,
+                            ops)
+    return outs[0]
+
+
+def run_phases(q_dists, gg_cols, bounds, k1=20, k2=6, lams=(0.3,), slab_cols=None, ops=None):
+    """phases A, B, C of every shard on the block matrix [[qq, qg], [qg^T, gg]]: q_dists() gives (qg, qq) and
+    gg_cols(c0, c1) gives gg[:, c0:c1].  The references to qg and qq taken here are dropped after phase A, so the two
+    matrices are freed then unless the caller keeps its own (run_shards keeps none).  Returns ([the blocks side by
+    side, one matrix per lambda of ``lams``, all from the same phase A / B state], the exchanged rank table (N, K),
+    the exchanged k-reciprocal rows [idx (N, cap), val (N, cap), cnt (N)])."""
+    ops = ops or sharded.CudaOps()
+    qg, qq = q_dists()
+    nq, ng = qg.shape
     counts = [hi - lo for lo, hi in bounds]
-    qq, qg = ops.distance(qf, qf, metric), ops.distance(qf, gf, metric)
     width = slab_cols or max(1, sharded.RERANK_SLAB_BYTES // (4 * ng))
     states, ranks = [], []
     for lo, hi in bounds:
-        slabs = ((s0, ops.distance(gf, gf[lo + s0:min(hi, lo + s0 + width)], metric)) for s0 in range(0, hi - lo, width))
+        slabs = ((s0, gg_cols(lo + s0, min(hi, lo + s0 + width))) for s0 in range(0, hi - lo, width))
         st, rr = ops.rerank_rows(qg, qq, slabs, lo, hi - lo, max(counts), k1, k2)
         states.append(st)
         ranks.append(rr)
@@ -53,11 +66,15 @@ def run_shards(qf, gf, bounds, metric='euclidean', k1=20, k2=6, lam=0.3, slab_co
     vs = [ops.rerank_expand(st, rank_all) for st in states]
     v_all = [torch.cat([vs[0][k][:nq]] + [v[k][nq:] for v in vs]) for k in range(3)]
     del vs
-    blocks = [ops.rerank_finish(st, rank_all, v_all[0], v_all[1], v_all[2], lam) for st in states]
-    for st, blk, (lo, hi) in zip(states, blocks, bounds):
-        assert tuple(blk.shape) == (nq, hi - lo)
+    outs = []
+    for lam in lams:
+        blocks = [ops.rerank_finish(st, rank_all, v_all[0], v_all[1], v_all[2], lam) for st in states]
+        for blk, (lo, hi) in zip(blocks, bounds):
+            assert tuple(blk.shape) == (nq, hi - lo)
+        outs.append(torch.cat(blocks, dim=1))
+        del blocks
     del states
-    return torch.cat(blocks, dim=1)
+    return outs, rank_all, v_all
 
 
 def bits_equal(a, b):

@@ -1,7 +1,7 @@
 """Gallery-sharded k-reciprocal re-ranking (sharded.re_ranking_sharded, evaluate_mars_sharded(re_rank=True)) under gloo
 on CPU, world sizes 2 and 3.
 
-The three per-rank phases are CPU stand-ins restated from oracle/rerank.py on the rank's own rows, with the same
+The three per-rank phases are CPU stand-ins built from oracle/rerank.py's per-row pieces on the rank's own rows, with the same
 exchange contract as csrc/rerank.cu (rank rows (n_loc, K) padded with -1, k-reciprocal rows (n_loc, cap) + counts).
 Features lie on a coarse integer grid, so every fp32 distance is exact and splitting the gallery cannot move a bit:
 the concatenated blocks and the re-ranked CMC/mAP must equal the oracle on the whole gallery.  This checks the
@@ -33,8 +33,7 @@ class CpuRerankOps(CpuOps):
             slab = slab.numpy()
             cols += [np.concatenate([qg[:, offset + s0 + t], slab[:, t]]) for t in range(slab.shape[1])]
         assert len(cols) == nq + n_own
-        sq = np.power(np.stack(cols), 2).astype(np.float32)                                # normalised_dist, own rows
-        D = 1. * sq / np.max(sq, axis=1, keepdims=True)
+        D = np.stack([orr.d_row(c) for c in cols])                                         # own rows of D
         K, _ = sharded.rerank_row_dims(k1, k2)
         rank = np.full((nq + n_own, K), -1, np.int32)
         top = orr.initial_rank(D, K)
@@ -55,17 +54,9 @@ class CpuRerankOps(CpuOps):
         _, cap = sharded.rerank_row_dims(k1, st['k2'])
         rows = D.shape[0]
         idx, val, cnt = np.zeros((rows, cap), np.int32), np.zeros((rows, cap), np.float32), np.zeros(rows, np.int32)
-        half = int(np.around(k1 / 2.)) + 1
-        for l in range(rows):                                                              # oracle.sparse_weights
-            recip = orr.reciprocal_row(rank, self._glob(st, l), k1 + 1)
-            expansion = recip
-            for cand in recip:
-                cr = orr.reciprocal_row(rank, cand, half)
-                if len(np.intersect1d(cr, recip)) > 2. / 3 * len(cr):
-                    expansion = np.append(expansion, cr)
-            ix = np.unique(expansion)
-            w = np.exp(-D[l, ix])
-            idx[l, :len(ix)], val[l, :len(ix)], cnt[l] = ix, (1. * w / np.sum(w)).astype(np.float32), len(ix)
+        for l in range(rows):
+            ix = orr.expansion_row(rank, self._glob(st, l), k1)
+            idx[l, :len(ix)], val[l, :len(ix)], cnt[l] = ix, orr.expansion_weights(D[l], ix), len(ix)
         return torch.from_numpy(idx), torch.from_numpy(val), torch.from_numpy(cnt)
 
     def rerank_finish(self, st, rank_all, idx_all, val_all, cnt_all, lambda_value):
@@ -79,12 +70,7 @@ class CpuRerankOps(CpuOps):
             if k2 == 1:
                 rows.append(V[g])
                 continue
-            dense = np.zeros((k2, N), np.float32)                                         # oracle.query_expansion
-            for r, n in enumerate(rank[g, :k2]):
-                dense[r, V[n][0]] = V[n][1]
-            acc = np.mean(dense[:len(rank[g, :k2])], axis=0)
-            nz = np.where(acc != 0)[0]
-            rows.append((nz, acc[nz]))
+            rows.append(orr.qe_row([V[n] for n in rank[g, :k2]]))
         inv = {}                                                                           # over the own gallery rows
         for j in range(n_own):
             for c, v in zip(*rows[nq + j]):
