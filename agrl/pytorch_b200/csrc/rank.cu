@@ -54,12 +54,17 @@ __global__ void narrow_labels_kernel(LabelArrays a, uint32_t *status) {
     if (__any_sync(0xffffffffu, bad) && (threadIdx.x & 31) == 0) atomicOr(status, AGRL_ST_LABEL_RANGE);
 }
 
+// elements in front of the row's first 16-byte boundary
+__device__ __forceinline__ int row_head(const float *row, int n) {
+    const int head = static_cast<int>(((16u - (reinterpret_cast<uintptr_t>(row) & 15u)) & 15u) >> 2);
+    return head < n ? head : n;
+}
+
 // visit every element of a row once, 16-byte vector loads over the aligned body
 template <class F>
 __device__ __forceinline__ void for_each_in_row(const float *__restrict__ row, int n, int tid,
                                                 int nthreads, F &&f) {
-    int head = static_cast<int>(((16u - (reinterpret_cast<uintptr_t>(row) & 15u)) & 15u) >> 2);
-    if (head > n) head = n;
+    const int head = row_head(row, n);
     if (tid < head) f(row[tid], tid);
     const int nvec = (n - head) >> 2;
     const float4 *v4 = reinterpret_cast<const float4 *>(row + head);
@@ -71,6 +76,14 @@ __device__ __forceinline__ void for_each_in_row(const float *__restrict__ row, i
     }
     const int tail0 = head + (nvec << 2);
     if (tail0 + tid < n) f(row[tail0 + tid], tail0 + tid);     // < 4 leftovers
+}
+
+// the most elements one thread visits in for_each_in_row: thread 0 takes the head element, the
+// largest share of the vectors and a tail element
+__device__ __forceinline__ int row_max_per_thread(const float *row, int n, int nthreads) {
+    const int head = row_head(row, n);
+    const int nvec = (n - head) >> 2;
+    return (head > 0) + 4 * ((nvec + nthreads - 1) / nthreads) + (((n - head) & 3) != 0);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -152,9 +165,13 @@ rank_market_kernel(MarketArgs a) {
     }
 
     // ---- phase B: sort the short list --------------------------------------------------------
-    const bool fast = (m <= kFastBins - 2) && (ng <= 65535 * kRankThreads);   // u16 private counters
+    // u16 private counters: no thread may bin more than 65535 elements.  The bound is the busiest
+    // thread's count, not ng / kRankThreads: thread 0 can take up to 5 elements more than that.
+    const bool fast = (m <= kFastBins - 2) && (row_max_per_thread(row, ng, kRankThreads) <= 65535);
+    // No pad entry is needed: every binned key is < list[m - 1], so the search below counts at most
+    // m - 1 <= n2 - 1 list keys.  Hence n2 <= kListCap: the list never reaches into the histogram region.
     int n2 = kFastBins;
-    while (n2 < m + 1) n2 <<= 1;           // at least one pad entry
+    while (n2 < m) n2 <<= 1;
     for (int i = m + tid; i < n2; i += kRankThreads) list[i] = kKeyMax;
     if (fast) {
 #pragma unroll 8
