@@ -86,18 +86,61 @@ __device__ __forceinline__ int row_max_per_thread(const float *row, int n, int n
     return (head > 0) + 4 * ((nvec + nthreads - 1) / nthreads) + (((n - head) & 3) != 0);
 }
 
+// visit the gallery items labelled `pid`, f(j) for each, int4 loads over the labels; kRankThreads threads
+template <class F>
+__device__ __forceinline__ void for_each_same_pid(const int32_t *__restrict__ g_pid, int ng, int pid, int tid, F &&f) {
+    const int nvec = ng >> 2;
+    const int4 *p4 = reinterpret_cast<const int4 *>(g_pid);
+    for (int v = tid; v < nvec; v += kRankThreads) {
+        const int4 p = __ldg(p4 + v);
+        if (p.x == pid) f(4 * v);
+        if (p.y == pid) f(4 * v + 1);
+        if (p.z == pid) f(4 * v + 2);
+        if (p.w == pid) f(4 * v + 3);
+    }
+    const int j = (nvec << 2) + tid;
+    if (j < ng && g_pid[j] == pid) f(j);
+}
+
+__device__ __forceinline__ float div_rn(float x, float y) { return __fdiv_rn(x, y); }
+__device__ __forceinline__ double div_rn(double x, double y) { return __ddiv_rn(x, y); }
+
+// cmc[r] = (number of first hits <= r) / div for r < R, from the first-hit histogram; one warp, inclusive scan over r
+// in chunks of 32
+template <class T>
+__device__ __forceinline__ void cmc_from_hist(const int32_t *hist, int R, T div, T *cmc, int lane) {
+    int carry = 0;
+    for (int base = 0; base < R; base += 32) {
+        const int r = base + lane;
+        int x = r < R ? hist[r] : 0;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int n = __shfl_up_sync(0xffffffffu, x, o);
+            if (lane >= o) x += n;
+        }
+        if (r < R) cmc[r] = div_rn(static_cast<T>(carry + x), div);
+        carry += __shfl_sync(0xffffffffu, x, 31);
+    }
+}
+
 // ------------------------------------------------------------------------------------------------
 // market1501: one CTA per query
 // ------------------------------------------------------------------------------------------------
-struct MarketArgs {
-    const float   *dist;
-    int64_t        ld;
-    const int32_t *q_pid, *q_cam, *g_pid, *g_cam;
-    int            num_q, num_g, rank_len;        // rank_len = min(max_rank, num_g)
+// what rank_market_finish_kernel reads: sizes and the per-query results of the rank kernels
+struct MarketResults {
+    int            num_q, rank_len;                // rank_len = min(max_rank, num_g)
     float         *ap;                             // [num_q]
     int32_t       *first_hit;                      // [num_q] kept-rank of the best positive, INT_MAX if invalid
     int32_t       *kept;                           // [num_q] gallery size after the junk filter
     uint32_t      *flags;                          // bit0: some valid query has kept < rank_len (stale cmc tail)
+};
+
+struct MarketArgs {
+    const float   *dist;
+    int64_t        ld;
+    const int32_t *q_pid, *q_cam, *g_pid, *g_cam;
+    int            num_g;
+    MarketResults  res;
     int32_t       *overflow_list;                  // queries whose same-pid list exceeds kListCap
     int32_t       *overflow_count;
 };
@@ -108,6 +151,51 @@ __device__ __forceinline__ float ap_from_terms(const double *terms, int npos) {
     float acc = 0.f;
     for (int i = 0; i < npos; ++i) acc = __double2float_rn(__dadd_rn(static_cast<double>(acc), terms[i]));
     return __fdiv_rn(acc, static_cast<float>(npos));
+}
+
+// Kept ranks of one query's sorted same-pid list of m items, npos of them positives, by one warp.  count(i): row
+// elements sorting between item i - 1 and item i; junk(i): item i has the query's camera.  The prefix sum of the counts
+// is item i's full rank, minus the junk items in front of it its kept rank.  Each positive's AP term goes to
+// terms[positives in front of it]; terms may alias the list, it is written behind the read cursor.  Lane 0 stores the AP
+// to *ap; returns the best positive's kept rank in every lane.
+template <class Count, class Junk>
+__device__ __forceinline__ int market_kept_ranks(int m, int npos, int lane, double *terms, Count count, Junk junk,
+                                                 float *ap) {
+    int carry_rank = 0, carry_junk = 0, carry_pos = 0;
+    int first_hit = INT_MAX;
+    for (int base = 0; base < m; base += 32) {
+        const int i = base + lane;
+        const bool in = i < m;
+        const int cnt = in ? count(i) : 0;
+        const bool is_junk = in && junk(i);
+        const bool is_pos = in && !is_junk;
+        // inclusive scan of cnt, exclusive counts of junk / positives in front of item i
+        int incl = cnt;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int n = __shfl_up_sync(0xffffffffu, incl, o);
+            if (lane >= o) incl += n;
+        }
+        const uint32_t jm = __ballot_sync(0xffffffffu, is_junk);
+        const uint32_t pm = __ballot_sync(0xffffffffu, is_pos);
+        const uint32_t below = (1u << lane) - 1u;
+        const int full_rank = carry_rank + incl;                       // #{j : key_j < key_i}
+        const int kept_rank = full_rank - (carry_junk + __popc(jm & below));
+        const int pos_before = carry_pos + __popc(pm & below);
+        __syncwarp();
+        if (is_pos) {
+            terms[pos_before] = __ddiv_rn(static_cast<double>(pos_before + 1),
+                                          static_cast<double>(kept_rank + 1));
+            if (pos_before == 0) first_hit = kept_rank;
+        }
+        carry_rank += __shfl_sync(0xffffffffu, incl, 31);
+        carry_junk += __popc(jm);
+        carry_pos += __popc(pm);
+        __syncwarp();
+    }
+    first_hit = __reduce_min_sync(0xffffffffu, first_hit);
+    if (lane == 0) *ap = ap_from_terms(terms, npos);
+    return first_hit;
 }
 
 __global__ void __launch_bounds__(kRankThreads)
@@ -129,37 +217,24 @@ rank_market_kernel(MarketArgs a) {
     __syncthreads();
 
     // ---- phase A: gather the gallery items of the query's identity (labels only) ------------
-    {
-        const int nvec = ng >> 2;
-        const int4 *p4 = reinterpret_cast<const int4 *>(a.g_pid);
-        auto hit = [&](int j) {
-            const bool junk = (a.g_cam[j] == cam);
-            atomicAdd(junk ? &s_njunk : &s_npos, 1);
-            const int slot = atomicAdd(&s_m, 1);
-            if (slot < kListCap) list[slot] = rank_key(row[j], static_cast<uint32_t>(j));
-        };
-        for (int v = tid; v < nvec; v += kRankThreads) {
-            const int4 p = __ldg(p4 + v);
-            if (p.x == pid) hit(4 * v);
-            if (p.y == pid) hit(4 * v + 1);
-            if (p.z == pid) hit(4 * v + 2);
-            if (p.w == pid) hit(4 * v + 3);
-        }
-        const int j = (nvec << 2) + tid;
-        if (j < ng && a.g_pid[j] == pid) hit(j);
-    }
+    for_each_same_pid(a.g_pid, ng, pid, tid, [&](int j) {
+        const bool junk = (a.g_cam[j] == cam);
+        atomicAdd(junk ? &s_njunk : &s_npos, 1);
+        const int slot = atomicAdd(&s_m, 1);
+        if (slot < kListCap) list[slot] = rank_key(row[j], static_cast<uint32_t>(j));
+    });
     __syncthreads();
     const int m = s_m, njunk = s_njunk, npos = s_npos;
     const int kept = ng - njunk;
     if (npos == 0) {                       // identity absent from the gallery: query skipped (pyx:203-205)
-        if (tid == 0) { a.ap[q] = 0.f; a.first_hit[q] = INT_MAX; a.kept[q] = kept; }
+        if (tid == 0) { a.res.ap[q] = 0.f; a.res.first_hit[q] = INT_MAX; a.res.kept[q] = kept; }
         return;
     }
     if (m > kListCap) {                    // rare: handled by rank_market_overflow_kernel
         if (tid == 0) {
             a.overflow_list[atomicAdd(a.overflow_count, 1)] = q;
-            a.kept[q] = kept;
-            if (kept < a.rank_len) atomicOr(a.flags, 1u);
+            a.res.kept[q] = kept;
+            if (kept < a.res.rank_len) atomicOr(a.res.flags, 1u);
         }
         return;
     }
@@ -227,49 +302,14 @@ rank_market_kernel(MarketArgs a) {
         __syncthreads();
     }
     if (tid >= 32) return;
-    {
-        const int lane = tid;
-        double *terms = reinterpret_cast<double *>(list);     // overwritten behind the read cursor
-        int carry_rank = 0, carry_junk = 0, carry_pos = 0;
-        int first_hit = INT_MAX;
-        for (int base = 0; base < m; base += 32) {
-            const int i = base + lane;
-            const bool in = i < m;
-            const int cnt = in ? (fast ? s_cnt[i] : static_cast<int>(hist32[i])) : 0;
-            const uint32_t idx = in ? static_cast<uint32_t>(list[i]) : 0u;
-            const bool is_junk = in && (a.g_cam[idx] == cam);
-            const bool is_pos = in && !is_junk;
-            // inclusive scan of cnt, exclusive counts of junk / positives in front of item i
-            int incl = cnt;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                const int n = __shfl_up_sync(0xffffffffu, incl, o);
-                if (lane >= o) incl += n;
-            }
-            const uint32_t jm = __ballot_sync(0xffffffffu, is_junk);
-            const uint32_t pm = __ballot_sync(0xffffffffu, is_pos);
-            const uint32_t below = (1u << lane) - 1u;
-            const int full_rank = carry_rank + incl;                       // #{j : key_j < key_i}
-            const int kept_rank = full_rank - (carry_junk + __popc(jm & below));
-            const int pos_before = carry_pos + __popc(pm & below);
-            __syncwarp();
-            if (is_pos) {
-                terms[pos_before] = __ddiv_rn(static_cast<double>(pos_before + 1),
-                                              static_cast<double>(kept_rank + 1));
-                if (pos_before == 0) first_hit = kept_rank;
-            }
-            carry_rank += __shfl_sync(0xffffffffu, incl, 31);
-            carry_junk += __popc(jm);
-            carry_pos += __popc(pm);
-            __syncwarp();
-        }
-        first_hit = __reduce_min_sync(0xffffffffu, first_hit);
-        if (lane == 0) {
-            a.ap[q] = ap_from_terms(terms, npos);
-            a.first_hit[q] = first_hit;
-            a.kept[q] = kept;
-            if (kept < a.rank_len) atomicOr(a.flags, 1u);
-        }
+    const int first_hit = market_kept_ranks(
+        m, npos, tid, reinterpret_cast<double *>(list),
+        [&](int i) { return fast ? s_cnt[i] : static_cast<int>(hist32[i]); },
+        [&](int i) { return a.g_cam[static_cast<uint32_t>(list[i])] == cam; }, &a.res.ap[q]);
+    if (tid == 0) {
+        a.res.first_hit[q] = first_hit;
+        a.res.kept[q] = kept;
+        if (kept < a.res.rank_len) atomicOr(a.res.flags, 1u);
     }
 }
 
@@ -320,8 +360,8 @@ rank_market_overflow_kernel(MarketArgs a, uint64_t *slab_keys, double *slab_term
         if (tid == 0) {
             for (int i = 0; i < m; ++i)
                 npos_total += (a.g_cam[static_cast<uint32_t>(keys[i])] != cam);
-            a.ap[q] = ap_from_terms(terms, npos_total);
-            a.first_hit[q] = s_first;
+            a.res.ap[q] = ap_from_terms(terms, npos_total);
+            a.res.first_hit[q] = s_first;
         }
         __syncthreads();
     }
@@ -329,7 +369,7 @@ rank_market_overflow_kernel(MarketArgs a, uint64_t *slab_keys, double *slab_term
 
 // One CTA: averages in the reference's order (rank_cy.pyx:230-239).
 __global__ void __launch_bounds__(1024)
-rank_market_finish_kernel(MarketArgs a, int32_t *hist /*[rank_len+1], zeroed here*/,
+rank_market_finish_kernel(MarketResults a, int32_t *hist /*[rank_len+1], zeroed here*/,
                           float *cmc_out, float *map_out, int64_t *num_valid_out, uint32_t *status) {
     __shared__ int s_valid;
     const int tid = threadIdx.x, nthr = blockDim.x;
@@ -356,20 +396,7 @@ rank_market_finish_kernel(MarketArgs a, int32_t *hist /*[rank_len+1], zeroed her
             if (fh != INT_MAX) atomicAdd(&hist[fh < R ? fh : R], 1);
         }
         __syncthreads();
-        if (tid < 32) {                                    // inclusive scan over r, chunks of 32
-            int carry = 0;
-            for (int base = 0; base < R; base += 32) {
-                const int r = base + tid;
-                int x = r < R ? hist[r] : 0;
-#pragma unroll
-                for (int o = 1; o < 32; o <<= 1) {
-                    const int n = __shfl_up_sync(0xffffffffu, x, o);
-                    if (tid >= o) x += n;
-                }
-                if (r < R) cmc_out[r] = __fdiv_rn(static_cast<float>(carry + x), fvalid);
-                carry += __shfl_sync(0xffffffffu, x, 31);
-            }
-        }
+        if (tid < 32) cmc_from_hist(hist, R, fvalid, cmc_out, tid);
     } else {
         // rank_cy never clears its `cmc` scratch (pyx:177): positions >= kept keep what the last
         // valid query that reached them left there.  Replay that per rank position, in query order.
@@ -447,24 +474,13 @@ rank_market_gather_kernel(MarketShardArgs a) {
     if (tid == 0) { s_m = 0; s_njunk = 0; s_npos = 0; }
     if (!kCountOnly) for (int i = tid; i < a.cap; i += kRankThreads) out[i] = kKeyMax;
     __syncthreads();
-    const int nvec = ng >> 2;
-    const int4 *p4 = reinterpret_cast<const int4 *>(a.g_pid);
-    auto hit = [&](int j) {
+    for_each_same_pid(a.g_pid, ng, pid, tid, [&](int j) {
         const int slot = atomicAdd(&s_m, 1);
         if (kCountOnly) return;
         const bool junk = (a.g_cam[j] == cam);
         atomicAdd(junk ? &s_njunk : &s_npos, 1);
         if (slot < a.cap) out[slot] = shard_key(row[j], a.index_offset + static_cast<uint32_t>(j), junk ? 1u : 0u);
-    };
-    for (int v = tid; v < nvec; v += kRankThreads) {
-        const int4 p = __ldg(p4 + v);
-        if (p.x == pid) hit(4 * v);
-        if (p.y == pid) hit(4 * v + 1);
-        if (p.z == pid) hit(4 * v + 2);
-        if (p.w == pid) hit(4 * v + 3);
-    }
-    const int j = (nvec << 2) + tid;
-    if (j < ng && a.g_pid[j] == pid) hit(j);
+    });
     __syncthreads();
     if (tid == 0) {
         if (kCountOnly) atomicMax(a.max_count, s_m);
@@ -519,12 +535,10 @@ struct MarketFinalArgs {
     const int32_t  *cnt;                // [num_q][n2] summed over shards
     const uint64_t *sorted;             // [num_q][n2]
     const int32_t  *npos, *njunk;       // [num_q] summed over shards
-    int             num_q, n2, rank_len;
+    int             n2;
     int64_t         num_g_total;
-    float          *ap;
-    int32_t        *first_hit, *kept;
-    uint32_t       *flags;
     double         *terms;              // [num_q][n2] scratch
+    MarketResults   res;
 };
 
 // one warp per query
@@ -532,66 +546,44 @@ __global__ void __launch_bounds__(kRankThreads)
 rank_market_finalize_kernel(MarketFinalArgs a) {
     const int lane = threadIdx.x & 31;
     const int q = blockIdx.x * (kRankThreads / 32) + (threadIdx.x >> 5);
-    if (q >= a.num_q) return;
+    if (q >= a.res.num_q) return;
     const int npos = a.npos[q], njunk = a.njunk[q];
     const int kept = static_cast<int>(a.num_g_total - njunk);
     if (npos == 0) {
-        if (lane == 0) { a.ap[q] = 0.f; a.first_hit[q] = INT_MAX; a.kept[q] = kept; }
+        if (lane == 0) { a.res.ap[q] = 0.f; a.res.first_hit[q] = INT_MAX; a.res.kept[q] = kept; }
         return;
     }
-    const int m = npos + njunk;
     const int32_t *cnt = a.cnt + static_cast<size_t>(q) * a.n2;
     const uint64_t *sorted = a.sorted + static_cast<size_t>(q) * a.n2;
-    double *terms = a.terms + static_cast<size_t>(q) * a.n2;
-    int carry_rank = 0, carry_junk = 0, carry_pos = 0, first_hit = INT_MAX;
-    for (int base = 0; base < m; base += 32) {
-        const int i = base + lane;
-        const bool in = i < m;
-        const int c = in ? cnt[i] : 0;
-        const bool is_junk = in && (sorted[i] & 1ull);
-        const bool is_pos = in && !is_junk;
-        int incl = c;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const int n = __shfl_up_sync(0xffffffffu, incl, o);
-            if (lane >= o) incl += n;
-        }
-        const uint32_t jm = __ballot_sync(0xffffffffu, is_junk);
-        const uint32_t pm = __ballot_sync(0xffffffffu, is_pos);
-        const uint32_t below = (1u << lane) - 1u;
-        const int kept_rank = carry_rank + incl - (carry_junk + __popc(jm & below));
-        const int pos_before = carry_pos + __popc(pm & below);
-        if (is_pos) {
-            terms[pos_before] = __ddiv_rn(static_cast<double>(pos_before + 1), static_cast<double>(kept_rank + 1));
-            if (pos_before == 0) first_hit = kept_rank;
-        }
-        carry_rank += __shfl_sync(0xffffffffu, incl, 31);
-        carry_junk += __popc(jm);
-        carry_pos += __popc(pm);
-    }
-    first_hit = __reduce_min_sync(0xffffffffu, first_hit);
-    __syncwarp();
+    const int first_hit = market_kept_ranks(
+        npos + njunk, npos, lane, a.terms + static_cast<size_t>(q) * a.n2,
+        [&](int i) { return cnt[i]; }, [&](int i) { return (sorted[i] & 1ull) != 0; }, &a.res.ap[q]);
     if (lane == 0) {
-        a.ap[q] = ap_from_terms(terms, npos);
-        a.first_hit[q] = first_hit;
-        a.kept[q] = kept;
-        if (kept < a.rank_len) atomicOr(a.flags, 1u);
+        a.res.first_hit[q] = first_hit;
+        a.res.kept[q] = kept;
+        if (kept < a.res.rank_len) atomicOr(a.res.flags, 1u);
     }
 }
 
 // ------------------------------------------------------------------------------------------------
 // MARS metric: one CTA per query
 // ------------------------------------------------------------------------------------------------
+// what rank_mars_finish_kernel reads: sizes and the per-query results of the rank kernels
+struct MarsResults {
+    int            num_q, max_rank;
+    double        *ap;                              // [num_q]
+    int32_t       *first_pos;                       // [num_q] junk-compacted position of the first good hit
+};
+
 struct MarsArgs {
     const float   *dist;
     int64_t        ld;
     const int32_t *q_pid, *q_cam, *g_pid, *g_cam;
-    int            num_q, num_g, max_rank;
+    int            num_g;
     int            buf_len;                         // power of two >= 2*max_rank and >= 2*tile
-    double        *ap;                              // [num_q]
-    int32_t       *first_pos;                       // [num_q] junk-compacted position of the first good hit
+    MarsResults    res;
     uint32_t      *status;
-    // gallery-sharded form (rank_mars_partial_kernel): this shard's candidates instead of the AP
+    // gallery-sharded form (rank_mars_kernel<true>): this shard's candidates instead of the AP
     uint64_t      *part_keys;                       // [num_q][max_rank] keys with GLOBAL gallery index
     uint8_t       *part_cls;                        // [num_q][max_rank] bit0 good, bit1 junk
     int32_t       *part_ngood;                      // [num_q] good images in this shard
@@ -600,21 +592,18 @@ struct MarsArgs {
 
 // number of good images for the query: same pid, other camera (rank.py:166); result in *s_ngood
 __device__ __forceinline__ void mars_count_good(const MarsArgs &a, int pid, int cam, int tid, int *s_ngood) {
-    const int ng = a.num_g;
     int good = 0;
-    const int nvec = ng >> 2;
-    const int4 *p4 = reinterpret_cast<const int4 *>(a.g_pid);
-    for (int v = tid; v < nvec; v += kRankThreads) {
-        const int4 p = __ldg(p4 + v);
-        if (p.x == pid) good += (a.g_cam[4 * v] != cam);
-        if (p.y == pid) good += (a.g_cam[4 * v + 1] != cam);
-        if (p.z == pid) good += (a.g_cam[4 * v + 2] != cam);
-        if (p.w == pid) good += (a.g_cam[4 * v + 3] != cam);
-    }
-    const int j = (nvec << 2) + tid;
-    if (j < ng && a.g_pid[j] == pid) good += (a.g_cam[j] != cam);
+    for_each_same_pid(a.g_pid, a.num_g, pid, tid, [&](int j) { good += (a.g_cam[j] != cam); });
     good = warp_sum(good);
     if ((tid & 31) == 0 && good) atomicAdd(s_ngood, good);
+}
+
+// class byte of a ranked gallery item (rank.py:166-169): bit0 good (same pid, other camera), bit1 junk (pid -1, or
+// same pid and camera)
+__device__ __forceinline__ uint8_t mars_class(int gp, int gc, int pid, int cam) {
+    const bool good = (gp == pid) && (gc != cam);
+    const bool junk = (gp == -1) || ((gp == pid) && (gc == cam));
+    return static_cast<uint8_t>((good ? 1 : 0) | (junk ? 2 : 0));
 }
 
 // Compute_AP (rank.py:180-212) in Python-float (double) arithmetic, one rounding per operation.
@@ -664,7 +653,7 @@ rank_mars_kernel(MarsArgs a) {
     __shared__ unsigned long long s_thr;
 
     const int q = blockIdx.x, tid = threadIdx.x;
-    const int K = a.max_rank;
+    const int K = a.res.max_rank;
     const int pid = a.q_pid[q], cam = a.q_cam[q];
     const float *row = a.dist + static_cast<size_t>(q) * a.ld;
 
@@ -673,15 +662,11 @@ rank_mars_kernel(MarsArgs a) {
     mars_count_good(a, pid, cam, tid, &s_ngood);
     const int valid = select_topk(row, a.num_g, K, a.buf_len, buf, &s_cnt, &s_thr, tid);
 
-    // classify the ranked items: bit0 good, bit1 junk (rank.py:166-169)
     for (int n = tid; n < K; n += kRankThreads) {
         uint8_t c = 0;
         if (n < valid) {
             const uint32_t g = static_cast<uint32_t>(buf[n]);
-            const int gp = a.g_pid[g], gc = a.g_cam[g];
-            const bool good = (gp == pid) && (gc != cam);
-            const bool junk = (gp == -1) || ((gp == pid) && (gc == cam));
-            c = static_cast<uint8_t>((good ? 1 : 0) | (junk ? 2 : 0));
+            c = mars_class(a.g_pid[g], a.g_cam[g], pid, cam);
         }
         if (kPartial) {
             a.part_keys[static_cast<size_t>(q) * K + n] = (n < valid) ? buf[n] + a.index_offset : kKeyMax;
@@ -693,7 +678,7 @@ rank_mars_kernel(MarsArgs a) {
     __syncthreads();
     if (tid != 0) return;
     if (kPartial) { a.part_ngood[q] = s_ngood; return; }
-    mars_compute_ap(cls, valid, s_ngood, &a.ap[q], &a.first_pos[q], a.status);
+    mars_compute_ap(cls, valid, s_ngood, &a.res.ap[q], &a.res.first_pos[q], a.status);
 }
 
 // Merge of the shards' candidates: one CTA per query sorts parts*K (key, class) pairs and runs
@@ -702,16 +687,15 @@ struct MarsMergeArgs {
     const uint64_t *keys;
     const uint8_t  *cls;
     const int32_t  *ngood;              // [num_q], already summed over the shards
-    int             parts, num_q, max_rank, n2;      // n2 = power of two >= parts * max_rank
-    double         *ap;
-    int32_t        *first_pos;
+    int             parts, n2;          // n2 = power of two >= parts * max_rank
+    MarsResults     res;
     uint32_t       *status;
 };
 
 __global__ void __launch_bounds__(kRankThreads)
 rank_mars_merge_kernel(MarsMergeArgs a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    const int q = blockIdx.x, tid = threadIdx.x, K = a.max_rank;
+    const int q = blockIdx.x, tid = threadIdx.x, K = a.res.max_rank;
     const int Kp = (K + 15) & ~15;
     uint64_t *keys = reinterpret_cast<uint64_t *>(smem_raw);                                  // n2
     uint64_t *okeys = keys + a.n2;                                                            // Kp: the merged head
@@ -721,7 +705,7 @@ rank_mars_merge_kernel(MarsMergeArgs a) {
     int unsorted = 0;
     for (int i = tid; i < a.n2; i += kRankThreads) {
         if (i < total) {
-            const size_t src = (static_cast<size_t>(i / K) * a.num_q + q) * K + (i % K);
+            const size_t src = (static_cast<size_t>(i / K) * a.res.num_q + q) * K + (i % K);
             keys[i] = a.keys[src];
             cls[i] = a.cls[src];
             if ((i % K) != 0 && a.keys[src - 1] > keys[i]) unsorted = 1;
@@ -755,26 +739,13 @@ rank_mars_merge_kernel(MarsMergeArgs a) {
         __syncthreads();
     } else {
         // lists in arbitrary order: bitonic sort of the keys carrying the class byte
-        for (int k = 2; k <= a.n2; k <<= 1) {
-            for (int j = k >> 1; j > 0; j >>= 1) {
-                for (int t = tid; t < (a.n2 >> 1); t += kRankThreads) {
-                    const int lo = ((t & ~(j - 1)) << 1) | (t & (j - 1));
-                    const int hi = lo | j;
-                    const uint64_t x = keys[lo], y = keys[hi];
-                    if ((x > y) == ((lo & k) == 0)) {
-                        keys[lo] = y; keys[hi] = x;
-                        const uint8_t c = cls[lo]; cls[lo] = cls[hi]; cls[hi] = c;
-                    }
-                }
-                __syncthreads();
-            }
-        }
+        bitonic_sort_u64<false, true>(keys, a.n2, tid, kRankThreads, cls);
         hk = keys; hc = cls;
     }
     if (tid != 0) return;
     int valid = 0;
     while (valid < K && hk[valid] != kKeyMax) ++valid;
-    mars_compute_ap(hc, valid, a.ngood[q], &a.ap[q], &a.first_pos[q], a.status);
+    mars_compute_ap(hc, valid, a.ngood[q], &a.res.ap[q], &a.res.first_pos[q], a.status);
 }
 
 // numpy's pairwise float64 summation (what np.mean runs on the ap vector, rank.py:176):
@@ -803,10 +774,10 @@ __device__ double pairwise_leaf_f64(const double *x, int n) {
 }
 
 // Post-order walk of the split tree with an explicit stack (device recursion would overflow the
-// default 1 KiB thread stack).  kEnumerate: record the leaves (offset, length) in visiting order;
-// otherwise: combine the precomputed leaf sums.  Returns the number of leaves / leaves consumed.
-template <bool kEnumerate>
-__device__ int pairwise_walk(int n, int2 *leaves, const double *leaf_sum, int max_leaves, double *result) {
+// default 1 KiB thread stack).  leaf(offset, length, index) gives the sum of the index-th leaf in
+// visiting order; the walk combines the leaf sums into *result.  Returns the number of leaves.
+template <class Leaf>
+__device__ int pairwise_walk(int n, Leaf leaf, double *result) {
     constexpr int kDepth = 40;
     int off[kDepth], len[kDepth], state[kDepth];     // state: 1 waiting for left, 2 waiting for right
     double left[kDepth];
@@ -829,8 +800,7 @@ __device__ int pairwise_walk(int n, int2 *leaves, const double *leaf_sum, int ma
                 --sp;
             }
         } else if (len[t] <= 128) {
-            if (kEnumerate) { if (nleaf < max_leaves) leaves[nleaf] = make_int2(off[t], len[t]); }
-            else ret = leaf_sum[nleaf];
+            ret = leaf(off[t], len[t], nleaf);
             ++nleaf;
             have_ret = true;
             --sp;
@@ -840,21 +810,27 @@ __device__ int pairwise_walk(int n, int2 *leaves, const double *leaf_sum, int ma
             off[sp] = off[t]; len[sp] = n2; state[sp] = 0; ++sp;
         }
     }
-    if (!kEnumerate) *result = ret;
+    *result = ret;
     return nleaf;
 }
 
-constexpr int kMaxLeaves = 2048;             // covers num_q up to ~130 000 in one pass
+constexpr int kMaxLeaves = 2048;             // covers num_q up to 262 144 in one pass
 
 __global__ void __launch_bounds__(1024)
-rank_mars_finish_kernel(MarsArgs a, int32_t *hist /*[max_rank+1]*/, double *cmc_out, double *map_out) {
+rank_mars_finish_kernel(MarsResults a, int32_t *hist /*[max_rank+1]*/, double *cmc_out, double *map_out) {
     __shared__ int2 s_leaf[kMaxLeaves];
     __shared__ double s_sum[kMaxLeaves];
     __shared__ int s_nleaf;
     const int tid = threadIdx.x, nthr = blockDim.x;
     const int nq = a.num_q, R = a.max_rank;
     for (int r = tid; r <= R; r += nthr) hist[r] = 0;
-    if (tid == 32) s_nleaf = pairwise_walk<true>(nq, s_leaf, nullptr, kMaxLeaves, nullptr);
+    if (tid == 32) {                         // record the leaves
+        double unused;
+        s_nleaf = pairwise_walk(nq, [&](int off, int len, int l) {
+            if (l < kMaxLeaves) s_leaf[l] = make_int2(off, len);
+            return 0.0;
+        }, &unused);
+    }
     __syncthreads();
     for (int q = tid; q < nq; q += nthr) {
         const int fp = a.first_pos[q];
@@ -864,55 +840,13 @@ rank_mars_finish_kernel(MarsArgs a, int32_t *hist /*[max_rank+1]*/, double *cmc_
     if (nleaf <= kMaxLeaves)
         for (int l = tid; l < nleaf; l += nthr) s_sum[l] = pairwise_leaf_f64(a.ap + s_leaf[l].x, s_leaf[l].y);
     __syncthreads();
-    if (tid < 32) {
-        int carry = 0;
-        for (int base = 0; base < R; base += 32) {
-            const int r = base + tid;
-            int x = r < R ? hist[r] : 0;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                const int n = __shfl_up_sync(0xffffffffu, x, o);
-                if (tid >= o) x += n;
-            }
-            if (r < R) cmc_out[r] = __ddiv_rn(static_cast<double>(carry + x), static_cast<double>(nq));
-            carry += __shfl_sync(0xffffffffu, x, 31);
-        }
-    }
+    if (tid < 32) cmc_from_hist(hist, R, static_cast<double>(nq), cmc_out, tid);
     if (tid == 32) {
-        double total = 0.0;
-        if (nleaf <= kMaxLeaves) {
-            pairwise_walk<false>(nq, nullptr, s_sum, kMaxLeaves, &total);
-        } else {
-            // very large num_q: sequential leaves (still the same tree)
-            total = 0.0;
-            int2 one;
-            // fall back to evaluating leaves on the fly
-            constexpr int kDepth = 40;
-            int off[kDepth], len[kDepth], state[kDepth];
-            double left[kDepth];
-            int sp = 1;
-            off[0] = 0; len[0] = nq; state[0] = 0;
-            double ret = 0.0; bool have_ret = false;
-            while (sp > 0) {
-                const int t = sp - 1;
-                if (have_ret) {
-                    have_ret = false;
-                    if (state[t] == 1) {
-                        left[t] = ret; state[t] = 2;
-                        int n2 = len[t] / 2; n2 -= n2 % 8;
-                        off[sp] = off[t] + n2; len[sp] = len[t] - n2; state[sp] = 0; ++sp;
-                    } else { ret = __dadd_rn(left[t], ret); have_ret = true; --sp; }
-                } else if (len[t] <= 128) {
-                    ret = pairwise_leaf_f64(a.ap + off[t], len[t]); have_ret = true; --sp;
-                } else {
-                    state[t] = 1;
-                    int n2 = len[t] / 2; n2 -= n2 % 8;
-                    off[sp] = off[t]; len[sp] = n2; state[sp] = 0; ++sp;
-                }
-            }
-            total = ret;
-            (void)one;
-        }
+        double total;
+        if (nleaf <= kMaxLeaves)
+            pairwise_walk(nq, [&](int, int, int l) { return s_sum[l]; }, &total);
+        else                                 // very large num_q: sequential leaves (still the same tree)
+            pairwise_walk(nq, [&](int off, int len, int) { return pairwise_leaf_f64(a.ap + off, len); }, &total);
         *map_out = __ddiv_rn(total, static_cast<double>(nq));
     }
 }
@@ -948,16 +882,18 @@ static RankWorkspace carve_rank(void *ws, int64_t nq, int64_t ng, int64_t max_ra
     return w;
 }
 
-static int narrow_labels(const RankWorkspace &w, const int64_t *qp, const int64_t *gp, const int64_t *qc,
-                         const int64_t *gc, int64_t nq, int64_t ng, uint32_t *status, cudaStream_t st) {
+// the four label arrays to int32 in dst_*
+static int narrow_labels(const int64_t *qp, const int64_t *gp, const int64_t *qc, const int64_t *gc, int64_t nq,
+                         int64_t ng, int32_t *dst_qp, int32_t *dst_gp, int32_t *dst_qc, int32_t *dst_gc,
+                         uint32_t *status, cudaStream_t st) {
     LabelArrays la;
-    la.src[0] = qp; la.dst[0] = w.q_pid; la.n[0] = nq;
-    la.src[1] = qc; la.dst[1] = w.q_cam; la.n[1] = nq;
-    la.src[2] = gp; la.dst[2] = w.g_pid; la.n[2] = ng;
-    la.src[3] = gc; la.dst[3] = w.g_cam; la.n[3] = ng;
+    la.src[0] = qp; la.dst[0] = dst_qp; la.n[0] = nq;
+    la.src[1] = qc; la.dst[1] = dst_qc; la.n[1] = nq;
+    la.src[2] = gp; la.dst[2] = dst_gp; la.n[2] = ng;
+    la.src[3] = gc; la.dst[3] = dst_gc; la.n[3] = ng;
     const int64_t nmax = nq > ng ? nq : ng;
     int blocks = static_cast<int>((nmax + 255) / 256);
-    if (blocks > 2 * kNumSMs) blocks = 2 * kNumSMs;
+    if (blocks > 4 * kNumSMs) blocks = 4 * kNumSMs;
     if (blocks < 1) blocks = 1;
     AGRL_LAUNCH_BEGIN(st);
     narrow_labels_kernel<<<dim3(blocks, 4), 256, 0, st>>>(la, status);
@@ -971,6 +907,59 @@ static int check_rank_args(const void *d, const void *a, const void *b, const vo
     if (nq < 0 || ng < 1 || max_rank < 1 || ld < ng) return AGRL_E_INVALID;
     if (nq > INT32_MAX / 2 || ng > INT32_MAX / 2) return AGRL_E_UNSUPPORTED;
     return AGRL_OK;
+}
+
+// the smallest power of two >= x, starting from the power of two `start`
+static int pow2_at_least(int64_t x, int start) {
+    int p = start;
+    while (p < x) p <<= 1;
+    return p;
+}
+
+// Set-up and launch of rank_mars_kernel<kPartial> for agrl_rank_mars_dev / _partial_dev, whose arguments are checked.
+// `a` holds the outputs; for the whole-gallery form a.res.ap == nullptr selects the workspace's AP vector.
+template <bool kPartial>
+static int launch_rank_mars(MarsArgs &a, RankWorkspace &w, const float *distmat, int64_t ld,
+                            const int64_t *q_pids, const int64_t *g_pids, const int64_t *q_camids,
+                            const int64_t *g_camids, int64_t num_q, int64_t num_g, int64_t max_rank,
+                            void *ws, size_t ws_bytes, cudaStream_t st) {
+    int rc = agrl_device_ok();
+    if (rc) return rc;
+    w = carve_rank(ws, num_q, num_g, max_rank);
+    if (!ws || ws_bytes < w.bytes) return AGRL_E_WORKSPACE;
+    AGRL_CUDA_TRY(cudaMemsetAsync(a.status, 0, sizeof(uint32_t), st));
+    rc = narrow_labels(q_pids, g_pids, q_camids, g_camids, num_q, num_g, w.q_pid, w.g_pid, w.q_cam, w.g_cam,
+                       a.status, st);
+    if (rc) return rc;
+    a.dist = distmat; a.ld = ld;
+    a.q_pid = w.q_pid; a.q_cam = w.q_cam; a.g_pid = w.g_pid; a.g_cam = w.g_cam;
+    a.num_g = static_cast<int>(num_g);
+    a.res.num_q = static_cast<int>(num_q); a.res.max_rank = static_cast<int>(max_rank);
+    if (!kPartial) {
+        if (!a.res.ap) a.res.ap = w.ap_f64;
+        a.res.first_pos = w.first;
+    }
+    const int L = pow2_at_least(2 * max_rank, 2 * kMarsTile);
+    a.buf_len = L;
+    const size_t smem = static_cast<size_t>(L) * 8 + align_up(static_cast<size_t>(max_rank), 16);
+    AGRL_CUDA_TRY(cudaFuncSetAttribute(rank_mars_kernel<kPartial>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       static_cast<int>(smem)));
+    AGRL_LAUNCH_BEGIN(st);
+    rank_mars_kernel<kPartial><<<static_cast<unsigned>(num_q), kRankThreads, smem, st>>>(a);
+    AGRL_LAUNCH_CHECK(st, kPartial ? "rank_mars_partial" : "rank_mars");
+    return AGRL_OK;
+}
+
+// labels from the workspace's narrowed copies, or none (w == nullptr) for the bin pass
+static MarketShardArgs shard_args(const RankWorkspace *w, const float *distmat, int64_t ld, int64_t num_q,
+                                  int64_t num_g, int64_t index_offset) {
+    MarketShardArgs a;
+    memset(&a, 0, sizeof(a));
+    a.dist = distmat; a.ld = ld;
+    if (w) { a.q_pid = w->q_pid; a.q_cam = w->q_cam; a.g_pid = w->g_pid; a.g_cam = w->g_cam; }
+    a.num_q = static_cast<int>(num_q); a.num_g = static_cast<int>(num_g);
+    a.index_offset = static_cast<uint32_t>(index_offset);
+    return a;
 }
 
 }  // namespace agrl
@@ -1004,16 +993,18 @@ extern "C" int agrl_rank_market1501_dev(const float *distmat, int64_t ld,
         AGRL_CUDA_TRY(cudaMemcpyAsync(status, &one, sizeof(one), cudaMemcpyHostToDevice, st));
         return AGRL_OK;
     }
-    if ((rc = narrow_labels(w, q_pids, g_pids, q_camids, g_camids, num_q, num_g, status, st))) return rc;
+    rc = narrow_labels(q_pids, g_pids, q_camids, g_camids, num_q, num_g, w.q_pid, w.g_pid, w.q_cam, w.g_cam,
+                       status, st);
+    if (rc) return rc;
 
     MarketArgs a;
     a.dist = distmat; a.ld = ld;
     a.q_pid = w.q_pid; a.q_cam = w.q_cam; a.g_pid = w.g_pid; a.g_cam = w.g_cam;
-    a.num_q = static_cast<int>(num_q); a.num_g = static_cast<int>(num_g);
-    a.rank_len = static_cast<int>(rank_len);
-    a.ap = all_ap ? all_ap : w.ap_f32;
-    a.first_hit = w.first; a.kept = w.kept;
-    a.flags = reinterpret_cast<uint32_t *>(w.counters + 1);
+    a.num_g = static_cast<int>(num_g);
+    a.res.num_q = static_cast<int>(num_q); a.res.rank_len = static_cast<int>(rank_len);
+    a.res.ap = all_ap ? all_ap : w.ap_f32;
+    a.res.first_hit = w.first; a.res.kept = w.kept;
+    a.res.flags = reinterpret_cast<uint32_t *>(w.counters + 1);
     a.overflow_list = w.overflow_list; a.overflow_count = w.counters;
 
     const size_t smem = kListCap * 8 + kFastBins * kRankThreads * 2;
@@ -1024,7 +1015,7 @@ extern "C" int agrl_rank_market1501_dev(const float *distmat, int64_t ld,
     AGRL_LAUNCH_CHECK(st, "rank_market");
     rank_market_overflow_kernel<<<kOverflowCtas, kRankThreads, 0, st>>>(a, w.slab_keys, w.slab_terms);
     AGRL_LAUNCH_CHECK(st, "rank_market_overflow");
-    rank_market_finish_kernel<<<1, 1024, 0, st>>>(a, w.hist, cmc, map, num_valid, status);
+    rank_market_finish_kernel<<<1, 1024, 0, st>>>(a.res, w.hist, cmc, map, num_valid, status);
     AGRL_LAUNCH_CHECK(st, "rank_market_finish");
     return AGRL_OK;
 }
@@ -1039,33 +1030,16 @@ extern "C" int agrl_rank_mars_dev(const float *distmat, int64_t ld,
     if (rc) return rc;
     if (!cmc || !map || !status || num_q < 1) return AGRL_E_INVALID;
     if (max_rank > num_g || max_rank > 8192) return AGRL_E_UNSUPPORTED;
-    if ((rc = agrl_device_ok())) return rc;
-    RankWorkspace w = carve_rank(ws, num_q, num_g, max_rank);
-    if (!ws || ws_bytes < w.bytes) return AGRL_E_WORKSPACE;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-
-    AGRL_CUDA_TRY(cudaMemsetAsync(status, 0, sizeof(uint32_t), st));
-    if ((rc = narrow_labels(w, q_pids, g_pids, q_camids, g_camids, num_q, num_g, status, st))) return rc;
-
     MarsArgs a;
-    a.dist = distmat; a.ld = ld;
-    a.q_pid = w.q_pid; a.q_cam = w.q_cam; a.g_pid = w.g_pid; a.g_cam = w.g_cam;
-    a.num_q = static_cast<int>(num_q); a.num_g = static_cast<int>(num_g);
-    a.max_rank = static_cast<int>(max_rank);
-    int L = 2 * kMarsTile;
-    while (L < 2 * max_rank) L <<= 1;
-    a.buf_len = L;
-    a.ap = all_ap ? all_ap : w.ap_f64;
-    a.first_pos = w.first;
+    memset(&a, 0, sizeof(a));
+    a.res.ap = all_ap;
     a.status = status;
-    a.part_keys = nullptr; a.part_cls = nullptr; a.part_ngood = nullptr; a.index_offset = 0;
-
-    const size_t smem = static_cast<size_t>(L) * 8 + align_up(static_cast<size_t>(max_rank), 16);
-    AGRL_CUDA_TRY(cudaFuncSetAttribute(rank_mars_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       static_cast<int>(smem)));
-    rank_mars_kernel<false><<<static_cast<unsigned>(num_q), kRankThreads, smem, st>>>(a);
-    AGRL_LAUNCH_CHECK(st, "rank_mars");
-    rank_mars_finish_kernel<<<1, 1024, 0, st>>>(a, w.hist, cmc, map);
+    RankWorkspace w;
+    rc = launch_rank_mars<false>(a, w, distmat, ld, q_pids, g_pids, q_camids, g_camids, num_q, num_g, max_rank,
+                                 ws, ws_bytes, st);
+    if (rc) return rc;
+    rank_mars_finish_kernel<<<1, 1024, 0, st>>>(a.res, w.hist, cmc, map);
     AGRL_LAUNCH_CHECK(st, "rank_mars_finish");
     return AGRL_OK;
 }
@@ -1081,29 +1055,14 @@ extern "C" int agrl_rank_mars_partial_dev(const float *distmat, int64_t ld,
     if (rc) return rc;
     if (!keys || !cls || !ngood || !status || num_q < 1 || index_offset < 0) return AGRL_E_INVALID;
     if (max_rank > 8192 || index_offset + num_g > 0xFFFFFFFFll) return AGRL_E_UNSUPPORTED;
-    if ((rc = agrl_device_ok())) return rc;
-    RankWorkspace w = carve_rank(ws, num_q, num_g, max_rank);
-    if (!ws || ws_bytes < w.bytes) return AGRL_E_WORKSPACE;
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    AGRL_CUDA_TRY(cudaMemsetAsync(status, 0, sizeof(uint32_t), st));
-    if ((rc = narrow_labels(w, q_pids, g_pids, q_camids, g_camids, num_q, num_g, status, st))) return rc;
     MarsArgs a;
-    a.dist = distmat; a.ld = ld;
-    a.q_pid = w.q_pid; a.q_cam = w.q_cam; a.g_pid = w.g_pid; a.g_cam = w.g_cam;
-    a.num_q = static_cast<int>(num_q); a.num_g = static_cast<int>(num_g); a.max_rank = static_cast<int>(max_rank);
-    int L = 2 * kMarsTile;
-    while (L < 2 * max_rank) L <<= 1;
-    a.buf_len = L;
-    a.ap = nullptr; a.first_pos = nullptr; a.status = status;
+    memset(&a, 0, sizeof(a));
+    a.status = status;
     a.part_keys = keys; a.part_cls = cls; a.part_ngood = ngood;
     a.index_offset = static_cast<uint32_t>(index_offset);
-    const size_t smem = static_cast<size_t>(L) * 8 + align_up(static_cast<size_t>(max_rank), 16);
-    AGRL_CUDA_TRY(cudaFuncSetAttribute(rank_mars_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       static_cast<int>(smem)));
-    AGRL_LAUNCH_BEGIN(st);
-    rank_mars_kernel<true><<<static_cast<unsigned>(num_q), kRankThreads, smem, st>>>(a);
-    AGRL_LAUNCH_CHECK(st, "rank_mars_partial");
-    return AGRL_OK;
+    RankWorkspace w;
+    return launch_rank_mars<true>(a, w, distmat, ld, q_pids, g_pids, q_camids, g_camids, num_q, num_g, max_rank,
+                                  ws, ws_bytes, static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int agrl_rank_mars_merge_dev(const uint64_t *keys, const uint8_t *cls, const int32_t *ngood,
@@ -1120,12 +1079,12 @@ extern "C" int agrl_rank_mars_merge_dev(const uint64_t *keys, const uint8_t *cls
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     MarsMergeArgs m;
     m.keys = keys; m.cls = cls; m.ngood = ngood;
-    m.parts = static_cast<int>(parts); m.num_q = static_cast<int>(num_q); m.max_rank = static_cast<int>(max_rank);
-    int n2 = 2;
-    while (n2 < parts * max_rank) n2 <<= 1;
+    m.parts = static_cast<int>(parts);
+    const int n2 = pow2_at_least(parts * max_rank, 2);
     m.n2 = n2;
-    m.ap = all_ap ? all_ap : w.ap_f64;
-    m.first_pos = w.first;
+    m.res.num_q = static_cast<int>(num_q); m.res.max_rank = static_cast<int>(max_rank);
+    m.res.ap = all_ap ? all_ap : w.ap_f64;
+    m.res.first_pos = w.first;
     m.status = status;
     const size_t smem = (static_cast<size_t>(n2) + ((max_rank + 15) & ~static_cast<size_t>(15))) * 9;
     AGRL_CUDA_TRY(cudaFuncSetAttribute(rank_mars_merge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -1133,25 +1092,12 @@ extern "C" int agrl_rank_mars_merge_dev(const uint64_t *keys, const uint8_t *cls
     AGRL_LAUNCH_BEGIN(st);          // (profiling: do not charge the collectives queued ahead on this stream to the merge)
     rank_mars_merge_kernel<<<static_cast<unsigned>(num_q), kRankThreads, smem, st>>>(m);
     AGRL_LAUNCH_CHECK(st, "rank_mars_merge");
-    MarsArgs a;
-    memset(&a, 0, sizeof(a));
-    a.num_q = m.num_q; a.max_rank = m.max_rank; a.ap = m.ap; a.first_pos = m.first_pos; a.status = status;
-    rank_mars_finish_kernel<<<1, 1024, 0, st>>>(a, w.hist, cmc, map);
+    rank_mars_finish_kernel<<<1, 1024, 0, st>>>(m.res, w.hist, cmc, map);
     AGRL_LAUNCH_CHECK(st, "rank_mars_finish");
     return AGRL_OK;
 }
 
 // ---- gallery-sharded market1501 metric ---------------------------------------------------------------
-static int fill_shard_args(MarketShardArgs &a, const RankWorkspace &w, const float *distmat, int64_t ld,
-                           int64_t num_q, int64_t num_g, int64_t index_offset) {
-    memset(&a, 0, sizeof(a));
-    a.dist = distmat; a.ld = ld;
-    a.q_pid = w.q_pid; a.q_cam = w.q_cam; a.g_pid = w.g_pid; a.g_cam = w.g_cam;
-    a.num_q = static_cast<int>(num_q); a.num_g = static_cast<int>(num_g);
-    a.index_offset = static_cast<uint32_t>(index_offset);
-    return AGRL_OK;
-}
-
 extern "C" int agrl_rank_market1501_count_dev(const int64_t *q_pids, const int64_t *g_pids,
                                               const int64_t *q_camids, const int64_t *g_camids,
                                               int64_t num_q, int64_t num_g, int32_t *max_count, uint32_t *status,
@@ -1165,9 +1111,10 @@ extern "C" int agrl_rank_market1501_count_dev(const int64_t *q_pids, const int64
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     AGRL_CUDA_TRY(cudaMemsetAsync(status, 0, sizeof(uint32_t), st));
     AGRL_CUDA_TRY(cudaMemsetAsync(max_count, 0, sizeof(int32_t), st));
-    if ((rc = narrow_labels(w, q_pids, g_pids, q_camids, g_camids, num_q, num_g, status, st))) return rc;
-    MarketShardArgs a;
-    fill_shard_args(a, w, nullptr, 0, num_q, num_g, 0);
+    rc = narrow_labels(q_pids, g_pids, q_camids, g_camids, num_q, num_g, w.q_pid, w.g_pid, w.q_cam, w.g_cam,
+                       status, st);
+    if (rc) return rc;
+    MarketShardArgs a = shard_args(&w, nullptr, 0, num_q, num_g, 0);
     a.max_count = max_count;
     AGRL_LAUNCH_BEGIN(st);
     rank_market_gather_kernel<true><<<static_cast<unsigned>(num_q), kRankThreads, 0, st>>>(a);
@@ -1190,20 +1137,15 @@ extern "C" int agrl_rank_market1501_gather_dev(const float *distmat, int64_t ld,
     if (!ws || ws_bytes < w.bytes) return AGRL_E_WORKSPACE;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     AGRL_CUDA_TRY(cudaMemsetAsync(status, 0, sizeof(uint32_t), st));
-    if ((rc = narrow_labels(w, q_pids, g_pids, q_camids, g_camids, num_q, num_g, status, st))) return rc;
-    MarketShardArgs a;
-    fill_shard_args(a, w, distmat, ld, num_q, num_g, index_offset);
+    rc = narrow_labels(q_pids, g_pids, q_camids, g_camids, num_q, num_g, w.q_pid, w.g_pid, w.q_cam, w.g_cam,
+                       status, st);
+    if (rc) return rc;
+    MarketShardArgs a = shard_args(&w, distmat, ld, num_q, num_g, index_offset);
     a.cap = static_cast<int>(cap); a.keys = keys; a.npos = npos; a.njunk = njunk;
     AGRL_LAUNCH_BEGIN(st);
     rank_market_gather_kernel<false><<<static_cast<unsigned>(num_q), kRankThreads, 0, st>>>(a);
     AGRL_LAUNCH_CHECK(st, "rank_market_gather");
     return AGRL_OK;
-}
-
-static int market_n2(int64_t parts, int64_t cap) {
-    int n2 = 2;
-    while (n2 < parts * cap) n2 <<= 1;
-    return n2;
 }
 
 extern "C" int agrl_rank_market1501_bin_dev(const float *distmat, int64_t ld, int64_t num_q, int64_t num_g,
@@ -1214,11 +1156,8 @@ extern "C" int agrl_rank_market1501_bin_dev(const float *distmat, int64_t ld, in
     int rc = agrl_device_ok();
     if (rc) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    MarketShardArgs a;
-    memset(&a, 0, sizeof(a));
-    a.dist = distmat; a.ld = ld; a.num_q = static_cast<int>(num_q); a.num_g = static_cast<int>(num_g);
-    a.index_offset = static_cast<uint32_t>(index_offset);
-    a.cap = static_cast<int>(cap); a.parts = static_cast<int>(parts); a.n2 = market_n2(parts, cap);
+    MarketShardArgs a = shard_args(nullptr, distmat, ld, num_q, num_g, index_offset);
+    a.cap = static_cast<int>(cap); a.parts = static_cast<int>(parts); a.n2 = pow2_at_least(parts * cap, 2);
     a.keys = const_cast<uint64_t *>(keys_all); a.cnt = cnt; a.sorted = sorted;
     const size_t smem = static_cast<size_t>(a.n2) * 8 + (static_cast<size_t>(a.n2) + 1) * 4;
     AGRL_CUDA_TRY(cudaFuncSetAttribute(rank_market_bin_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
@@ -1230,7 +1169,7 @@ extern "C" int agrl_rank_market1501_bin_dev(const float *distmat, int64_t ld, in
 
 extern "C" int64_t agrl_rank_market1501_list_len(int64_t parts, int64_t cap) {
     if (parts < 1 || cap < 1 || parts * cap > 8192) return 0;
-    return market_n2(parts, cap);
+    return pow2_at_least(parts * cap, 2);
 }
 
 extern "C" int agrl_rank_market1501_finalize_dev(const int32_t *cnt_total, const uint64_t *sorted,
@@ -1243,7 +1182,7 @@ extern "C" int agrl_rank_market1501_finalize_dev(const int32_t *cnt_total, const
     int rc = agrl_device_ok();
     if (rc) return rc;
     const int64_t rank_len = max_rank < num_g_total ? max_rank : num_g_total;
-    const int n2 = market_n2(parts, cap);
+    const int n2 = pow2_at_least(parts * cap, 2);
     Carver c(ws);
     RankWorkspace w = carve_rank(ws, num_q, 0, rank_len);
     c.off = w.bytes;
@@ -1253,26 +1192,22 @@ extern "C" int agrl_rank_market1501_finalize_dev(const int32_t *cnt_total, const
     AGRL_CUDA_TRY(cudaMemsetAsync(w.counters, 0, 4 * sizeof(int32_t), st));
     MarketFinalArgs f;
     f.cnt = cnt_total; f.sorted = sorted; f.npos = npos_total; f.njunk = njunk_total;
-    f.num_q = static_cast<int>(num_q); f.n2 = n2; f.rank_len = static_cast<int>(rank_len);
-    f.num_g_total = num_g_total;
-    f.ap = all_ap ? all_ap : w.ap_f32; f.first_hit = w.first; f.kept = w.kept;
-    f.flags = reinterpret_cast<uint32_t *>(w.counters + 1);
-    f.terms = terms;
+    f.n2 = n2; f.num_g_total = num_g_total; f.terms = terms;
+    f.res.num_q = static_cast<int>(num_q); f.res.rank_len = static_cast<int>(rank_len);
+    f.res.ap = all_ap ? all_ap : w.ap_f32; f.res.first_hit = w.first; f.res.kept = w.kept;
+    f.res.flags = reinterpret_cast<uint32_t *>(w.counters + 1);
     const int wpb = kRankThreads / 32;
     AGRL_LAUNCH_BEGIN(st);
     rank_market_finalize_kernel<<<static_cast<unsigned>((num_q + wpb - 1) / wpb), kRankThreads, 0, st>>>(f);
     AGRL_LAUNCH_CHECK(st, "rank_market_finalize");
-    MarketArgs a;
-    memset(&a, 0, sizeof(a));
-    a.num_q = f.num_q; a.rank_len = f.rank_len; a.ap = f.ap; a.first_hit = f.first_hit; a.kept = f.kept; a.flags = f.flags;
-    rank_market_finish_kernel<<<1, 1024, 0, st>>>(a, w.hist, cmc, map, num_valid, status);
+    rank_market_finish_kernel<<<1, 1024, 0, st>>>(f.res, w.hist, cmc, map, num_valid, status);
     AGRL_LAUNCH_CHECK(st, "rank_market_finish");
     return AGRL_OK;
 }
 
 extern "C" size_t agrl_rank_market1501_finalize_workspace_bytes(int64_t num_q, int64_t parts, int64_t cap, int64_t max_rank) {
     if (num_q < 1 || parts < 1 || cap < 1 || max_rank < 1 || parts * cap > 8192) return 0;
-    return carve_rank(nullptr, num_q, 0, max_rank).bytes + align_up(static_cast<size_t>(num_q) * market_n2(parts, cap) * 8, 256) + 256;
+    return carve_rank(nullptr, num_q, 0, max_rank).bytes + align_up(static_cast<size_t>(num_q) * pow2_at_least(parts * cap, 2) * 8, 256) + 256;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1296,8 +1231,7 @@ static ClassifyWorkspace carve_classify(void *ws, int64_t nq, int64_t ng) {
     ClassifyWorkspace w;
     w.q_pid = c.take<int32_t>(nq); w.q_cam = c.take<int32_t>(nq);
     w.g_pid = c.take<int32_t>(ng); w.g_cam = c.take<int32_t>(ng);
-    int slots = 64;
-    while (slots < 4 * nq) slots <<= 1;
+    const int slots = pow2_at_least(4 * nq, 64);
     w.slots = slots;
     w.tab_p = c.take<int32_t>(4 * static_cast<size_t>(slots));      // tab_p | tab_pc | cnt_p | cnt_pc, contiguous
     w.tab_pc = w.tab_p ? w.tab_p + slots : nullptr;
@@ -1315,36 +1249,46 @@ __device__ __forceinline__ uint32_t hash_pid_cam(int pid, int cam) {
     return hash_u32(static_cast<uint32_t>(pid) * 0x9E3779B1U + hash_u32(static_cast<uint32_t>(cam) + 0x85EBCA6BU));
 }
 
+// Linear probing in `tab` from slot `hash`: walks until the slot is empty or holds a query that match()es; returns
+// that slot, or -1 at an empty slot.  kClaim: an empty slot is taken for query q (atomicCAS), which ends the walk.
+template <bool kClaim, class Match>
+__device__ __forceinline__ int probe(int32_t *tab, uint32_t hash, int slots, int q, Match match) {
+    const uint32_t mask = static_cast<uint32_t>(slots - 1);
+    for (uint32_t h = hash & mask;; h = (h + 1) & mask) {
+        const int cur = kClaim ? atomicCAS(&tab[h], -1, q) : tab[h];
+        if (cur == -1) return -1;
+        if (match(cur)) return static_cast<int>(h);
+    }
+}
+
+// slot of pid in tab_p / of (pid, cam) in tab_pc, -1 if absent; kClaim inserts query q
+template <bool kClaim>
+__device__ __forceinline__ int probe_pid(const ClassifyWorkspace &w, int pid, int q = -1) {
+    return probe<kClaim>(w.tab_p, hash_u32(static_cast<uint32_t>(pid)), w.slots, q,
+                         [&](int r) { return w.q_pid[r] == pid; });
+}
+template <bool kClaim>
+__device__ __forceinline__ int probe_pid_cam(const ClassifyWorkspace &w, int pid, int cam, int q = -1) {
+    return probe<kClaim>(w.tab_pc, hash_pid_cam(pid, cam), w.slots, q,
+                         [&](int r) { return w.q_pid[r] == pid && w.q_cam[r] == cam; });
+}
+
 __global__ void classify_insert_kernel(ClassifyWorkspace w, int nq) {
     const int q = blockIdx.x * blockDim.x + threadIdx.x;
     if (q >= nq) return;
     const int pid = w.q_pid[q], cam = w.q_cam[q];
-    const uint32_t mask = static_cast<uint32_t>(w.slots - 1);
-    for (uint32_t h = hash_u32(static_cast<uint32_t>(pid)) & mask;; h = (h + 1) & mask) {
-        const int cur = atomicCAS(&w.tab_p[h], -1, q);
-        if (cur == -1 || w.q_pid[cur] == pid) break;
-    }
-    for (uint32_t h = hash_pid_cam(pid, cam) & mask;; h = (h + 1) & mask) {
-        const int cur = atomicCAS(&w.tab_pc[h], -1, q);
-        if (cur == -1 || (w.q_pid[cur] == pid && w.q_cam[cur] == cam)) break;
-    }
+    probe_pid<true>(w, pid, q);
+    probe_pid_cam<true>(w, pid, cam, q);
 }
 
 __global__ void classify_count_kernel(ClassifyWorkspace w, int64_t ng) {
-    const uint32_t mask = static_cast<uint32_t>(w.slots - 1);
     for (int64_t j = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; j < ng;
          j += static_cast<int64_t>(gridDim.x) * blockDim.x) {
         const int pid = w.g_pid[j], cam = w.g_cam[j];
-        for (uint32_t h = hash_u32(static_cast<uint32_t>(pid)) & mask;; h = (h + 1) & mask) {
-            const int cur = w.tab_p[h];
-            if (cur == -1) break;
-            if (w.q_pid[cur] == pid) { atomicAdd(&w.cnt_p[h], 1); break; }
-        }
-        for (uint32_t h = hash_pid_cam(pid, cam) & mask;; h = (h + 1) & mask) {
-            const int cur = w.tab_pc[h];
-            if (cur == -1) break;
-            if (w.q_pid[cur] == pid && w.q_cam[cur] == cam) { atomicAdd(&w.cnt_pc[h], 1); break; }
-        }
+        const int hp = probe_pid<false>(w, pid);
+        if (hp >= 0) atomicAdd(&w.cnt_p[hp], 1);
+        const int hpc = probe_pid_cam<false>(w, pid, cam);
+        if (hpc >= 0) atomicAdd(&w.cnt_pc[hpc], 1);
     }
 }
 
@@ -1359,28 +1303,12 @@ __global__ void classify_keys_kernel(ClassifyWorkspace w, const uint64_t *__rest
     uint8_t c = 0;
     if (key != kKeyMax) {
         const int64_t g = static_cast<int64_t>(static_cast<uint32_t>(key)) - index_offset;
-        if (g >= 0 && g < ng) {
-            const int gp = w.g_pid[g], gc = w.g_cam[g];
-            const bool good = (gp == pid) && (gc != cam);
-            const bool junk = (gp == -1) || ((gp == pid) && (gc == cam));
-            c = static_cast<uint8_t>((good ? 1 : 0) | (junk ? 2 : 0));
-        }
+        if (g >= 0 && g < ng) c = mars_class(w.g_pid[g], w.g_cam[g], pid, cam);
     }
     cls[i] = c;
     if (n == 0) {
-        const uint32_t mask = static_cast<uint32_t>(w.slots - 1);
-        int same_pid = 0, same_both = 0;
-        for (uint32_t h = hash_u32(static_cast<uint32_t>(pid)) & mask;; h = (h + 1) & mask) {
-            const int cur = w.tab_p[h];
-            if (cur == -1) break;
-            if (w.q_pid[cur] == pid) { same_pid = w.cnt_p[h]; break; }
-        }
-        for (uint32_t h = hash_pid_cam(pid, cam) & mask;; h = (h + 1) & mask) {
-            const int cur = w.tab_pc[h];
-            if (cur == -1) break;
-            if (w.q_pid[cur] == pid && w.q_cam[cur] == cam) { same_both = w.cnt_pc[h]; break; }
-        }
-        ngood[q] = same_pid - same_both;
+        const int hp = probe_pid<false>(w, pid), hpc = probe_pid_cam<false>(w, pid, cam);
+        ngood[q] = (hp >= 0 ? w.cnt_p[hp] : 0) - (hpc >= 0 ? w.cnt_pc[hpc] : 0);
     }
 }
 
@@ -1404,17 +1332,9 @@ extern "C" int agrl_rank_mars_classify_dev(const uint64_t *keys, const int64_t *
     ClassifyWorkspace w = carve_classify(ws, num_q, num_g);
     if (!ws || ws_bytes < w.bytes) return AGRL_E_WORKSPACE;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    LabelArrays la;
-    la.src[0] = q_pids; la.dst[0] = w.q_pid; la.n[0] = num_q;
-    la.src[1] = q_camids; la.dst[1] = w.q_cam; la.n[1] = num_q;
-    la.src[2] = g_pids; la.dst[2] = w.g_pid; la.n[2] = num_g;
-    la.src[3] = g_camids; la.dst[3] = w.g_cam; la.n[3] = num_g;
-    const int64_t nmax = num_q > num_g ? num_q : num_g;
-    int blocks = static_cast<int>((nmax + 255) / 256);
-    if (blocks > 4 * kNumSMs) blocks = 4 * kNumSMs;
-    AGRL_LAUNCH_BEGIN(st);
-    narrow_labels_kernel<<<dim3(blocks, 4), 256, 0, st>>>(la, status);
-    AGRL_LAUNCH_CHECK(st, "narrow_labels");
+    rc = narrow_labels(q_pids, g_pids, q_camids, g_camids, num_q, num_g, w.q_pid, w.g_pid, w.q_cam, w.g_cam,
+                       status, st);
+    if (rc) return rc;
     AGRL_CUDA_TRY(cudaMemsetAsync(w.tab_p, 0xFF, sizeof(int32_t) * 2 * w.slots, st));       // both tables: empty (-1)
     AGRL_CUDA_TRY(cudaMemsetAsync(w.cnt_p, 0, sizeof(int32_t) * 2 * w.slots, st));
     const int nq = static_cast<int>(num_q);

@@ -10,10 +10,12 @@ constexpr int kRankThreads = 256;
 constexpr uint64_t kKeyMax = 0xFFFFFFFFFFFFFFFFull;
 
 // ------------------------------------------------------------------------------------------------
-// shared-memory bitonic sort of n2 (power of two) uint64 keys by `nthreads` cooperating threads
+// shared-memory bitonic sort of n2 (power of two) uint64 keys by `nthreads` cooperating threads;
+// kPayload: payload[i] is swapped along with keys[i]
 // ------------------------------------------------------------------------------------------------
-template <bool kWarpOnly>
-__device__ __forceinline__ void bitonic_sort_u64(uint64_t *keys, int n2, int tid, int nthreads) {
+template <bool kWarpOnly, bool kPayload = false>
+__device__ __forceinline__ void bitonic_sort_u64(uint64_t *keys, int n2, int tid, int nthreads,
+                                                 uint8_t *payload = nullptr) {
     for (int k = 2; k <= n2; k <<= 1) {
         for (int j = k >> 1; j > 0; j >>= 1) {
             for (int t = tid; t < (n2 >> 1); t += nthreads) {
@@ -21,7 +23,10 @@ __device__ __forceinline__ void bitonic_sort_u64(uint64_t *keys, int n2, int tid
                 const int hi = lo | j;
                 const uint64_t a = keys[lo], b = keys[hi];
                 const bool up = ((lo & k) == 0);
-                if ((a > b) == up) { keys[lo] = b; keys[hi] = a; }
+                if ((a > b) == up) {
+                    keys[lo] = b; keys[hi] = a;
+                    if (kPayload) { const uint8_t c = payload[lo]; payload[lo] = payload[hi]; payload[hi] = c; }
+                }
             }
             // (CTA-wide barriers only around the steps that cross 64-element blocks, __syncwarp elsewhere: measured, no gain)
             if (kWarpOnly) __syncwarp(); else __syncthreads();

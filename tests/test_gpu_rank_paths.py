@@ -432,7 +432,9 @@ def test_mars_errors(evaluate_mars):
             evaluate_mars(dist, qp, gp2, qc, gc2, 16)
 
 
-MAP_NQ = [1, 7, 8, 9, 127, 128, 129, 136, 1024, 8191, 8192, 8193, 100003]
+# 262 144 / 262 145: 2048 / 2049 leaves of the pairwise sum, either side of the leaf table of rank_mars_finish_kernel
+# (kMaxLeaves); above it the leaves are summed during the tree walk
+MAP_NQ = [1, 7, 8, 9, 127, 128, 129, 136, 1024, 8191, 8192, 8193, 100003, 262144, 262145]
 
 
 @gpu
