@@ -1237,13 +1237,19 @@ struct HeadWorkspace {
     float *z;                          // (batch, 4S, C) low-rank first layer: Q.W^T
     float *gt;                         // (batch, V, 4S) low-rank first layer: G.T
     float *y_unscale;                  // (batch) scaled fp16 modes
-    float *row_sumsq;                  // (batch*V, 32) partial row norms of the last layer's output
+    float *row_sumsq;                  // (batch*V, sumsq_slots_of) partial row norms of the last layer's output
     size_t bytes;
 };
 
 // the first layer runs low-rank (G.X.W^T = (G.T).(Q.W^T) on the 4S quarter-strip rows) unless switched off or impossible
 static bool lowrank_enabled(const agrl_head_params *p, int S) {
     return !p->lowrank_off && p->num_layers > 0 && p->channels % (2 * kHeadThreads) == 0 && S * kParts <= kMaxNodes;
+}
+
+// partial row sums of squares that the last layer's GEMM epilogue leaves for the attention: one per (column tile, half)
+static int sumsq_slots_of(const agrl_head_params *p) {
+    const int bn = p->split == AGRL_SPLIT_BF16X3 ? 128 : 256;
+    return 2 * ((p->channels + bn - 1) / bn);
 }
 
 static HeadWorkspace carve_head(const agrl_head_params *p, void *ws, int64_t batch, int32_t S) {
@@ -1254,7 +1260,9 @@ static HeadWorkspace carve_head(const agrl_head_params *p, void *ws, int64_t bat
     w.x[1] = c.take<float>(n);
     w.y_planes = c.take<__nv_bfloat16>(static_cast<size_t>(planes_of(p->split)) * n);
     w.y_unscale = c.take<float>(static_cast<size_t>(batch));
-    w.row_sumsq = c.take<float>(static_cast<size_t>(batch) * S * kParts * 32);
+    // no fewer than 32 floats per row, so that the workspace size of every split at C <= 2048 stays what callers allocate
+    const int sumsq_room = sumsq_slots_of(p) > 32 ? sumsq_slots_of(p) : 32;
+    w.row_sumsq = c.take<float>(static_cast<size_t>(batch) * S * kParts * sumsq_room);
     const bool lowrank = lowrank_enabled(p, S);
     w.z = lowrank ? c.take<float>(static_cast<size_t>(batch) * S * 4 * p->channels) : nullptr;
     w.gt = lowrank ? c.take<float>(static_cast<size_t>(batch) * S * kParts * S * 4) : nullptr;
@@ -1472,8 +1480,8 @@ static int launch_layers(const agrl_head_params *p, const Prepared &pr, HeadWork
         }
         AGRL_LAUNCH_BEGIN(st);
         if ((rc = launch_graph(ga, n, st))) return rc;
-        const int sumsq_slots = 2 * ((C + bn - 1) / bn);                 // (column tile, half) pairs of the direct epilogue
-        float *sumsq = (l == L - 1 && C % bn == 0) ? hwk.row_sumsq + row0 * 32 : nullptr;
+        const int sumsq_slots = sumsq_slots_of(p);
+        float *sumsq = (l == L - 1 && C % bn == 0) ? hwk.row_sumsq + row0 * sumsq_slots : nullptr;
         if (sumsq) { attn_sumsq = sumsq; attn_slots = sumsq_slots; }
         gemm::EpiGraphLayer e2{x[cur], pr.scale[l], pr.shift[l], dst, C, C, p->gamma, p->leaky_slope, nullptr, nullptr, V};
         gemm::EpiGraphLayerF16 e1{x[cur], pr.scale[l], pr.shift[l], dst, C, C, p->gamma, p->leaky_slope,

@@ -219,6 +219,14 @@ class VMGN(nn.Module):
             _lib.check(_lib.E_UNSUPPORTED)
         dev = x4_1.device
         BS, C, h, w = x4_1.shape
+        # the library takes C from the module and reads both maps with x4_1's geometry: a mismatch would be read with the
+        # wrong layout (or past the end of x4_2), and frames beyond the last whole tracklet would be dropped
+        if C != self.feature_dim:
+            raise ValueError('x4_1 has %d channels; this module is built for %d' % (C, self.feature_dim))
+        if tuple(x4_2.shape) != tuple(x4_1.shape):
+            raise ValueError('x4_2 must have the shape of x4_1: %s vs %s' % (tuple(x4_2.shape), tuple(x4_1.shape)))
+        if BS % seq_len != 0:
+            raise ValueError('B*S = %d maps is not a multiple of seq_len = %d' % (BS, seq_len))
         B, V = BS // seq_len, seq_len * self.total_split
         if B == 0:                                                   # empty loader batch: nothing to launch
             empty = torch.empty(0, 2 * C, dtype=torch.float32, device=dev) if out is None else out

@@ -280,7 +280,7 @@ AGRL_API int agrl_distance_host(const float *q_host, const float *g_host, float 
  *     stays on stock cuDNN in the caller.
  *
  *     Canonical geometry only: pyramid strips of num_split = 4 ([4,2,1] -> P = 7 parts,
- *     utils/reidtools.py:13-15), feature-map height h divisible by 4, C divisible by 64,
+ *     utils/reidtools.py:13-15), feature-map height h divisible by 4, C divisible by 128,
  *     S*P <= 64 nodes per tracklet.  Anything else returns AGRL_E_UNSUPPORTED.
  * ============================================================================================= */
 #define AGRL_HEAD_MAX_LAYERS 4
