@@ -132,7 +132,7 @@ def load(build_if_missing=True):
 
 
 def planes_of_distance_split(split):
-    """16-bit planes per row of a prepared distance operand (csrc/distance.cu planes_of)."""
+    """16-bit planes per row of a prepared distance operand (csrc/planes.cuh count)."""
     return 2 if split == SPLIT_FP16X2 else int(split)
 
 

@@ -3,9 +3,10 @@
 //   euclidean : out[i,j] = (|q_i|^2 + |g_j|^2) - 2 q_i.g_j      (no clamp, no sqrt; distance.py:70-72)
 //   cosine    : out[i,j] = 1 - q^_i . g^_j,  x^ = x / max(|x|_2, 1e-12)   (distance.py:86-88)
 //
-// Pipeline: split.cu turns both operands into bf16 planes (and norms / normalised rows) in one
+// Pipeline: split.cu turns both operands into operand planes (planes.cuh; and norms / normalised rows) in one
 // pass each, then one persistent tcgen05 GEMM (gemm_sm100.cuh) with the distance epilogue fused.
 #include "gemm_sm100.cuh"
+#include "planes.cuh"
 #include "topk.cuh"
 
 namespace agrl {
@@ -17,30 +18,31 @@ struct Operand {
     size_t bytes;
 };
 
-static int planes_of(int split) { return split == AGRL_SPLIT_FP16X2 ? 2 : split; }
-
 static Operand carve_operand(void *buf, int64_t rows, int64_t dim, int split) {
     Carver c(buf);
     Operand o;
-    o.planes = c.take<__nv_bfloat16>(static_cast<size_t>(planes_of(split)) * rows * gemm::pad_k(dim));
+    o.planes = c.take<__nv_bfloat16>(static_cast<size_t>(planes::count(split)) * rows * gemm::pad_k(dim));
     o.sumsq = c.take<float>(rows);
     o.unscale = c.take<float>(rows);
     o.bytes = c.total();
     return o;
 }
 
-static bool split_ok(int split) { return split == AGRL_SPLIT_BF16X2 || split == AGRL_SPLIT_BF16X3 || split == AGRL_SPLIT_FP16X2; }
-
-// fp16 x 2: one CTA per 128 x 128 tile, the two-MMA k-step of gemm_sm100.cuh (kWideB).  (CTA pairs on 256 x 128 tiles were
-// measured as well: 0.397 against 0.383 ms at 1980 x 9330 x 4096 -- not kept.)
-template <class Epi>
-static int launch_f16x2(const void *q_planes, int64_t num_q, const void *g_planes, int64_t g_rows, int64_t g_plane_rows,
-                        int kp, const Epi &epi, cudaStream_t st) {
-    CUtensorMap map_q, map_g;
-    int rc;
-    if ((rc = gemm::make_plane_tensor_map(&map_q, q_planes, num_q, kp, 2, gemm::BM, num_q))) return rc;
-    if ((rc = gemm::make_plane_tensor_map(&map_g, g_planes, g_rows, kp, 2, 128, g_plane_rows))) return rc;
-    return gemm::launch_split_gemm<2, 128, true>(map_q, map_g, static_cast<int>(num_q), static_cast<int>(g_rows), kp, epi, st);
+// q x (g_rows rows of the gallery planes, g_plane_rows rows apart) on the split's GEMM: one CTA per 128 x 128 tile (for
+// fp16 x 2 the two-MMA k-step of gemm_sm100.cuh, kWideB; CTA pairs on 256 x 128 tiles were measured as well: 0.397
+// against 0.383 ms at 1980 x 9330 x 4096 -- not kept).  make(mode) builds the epilogue of that mode.
+template <class Make>
+static int launch_distance_gemm(int split, const void *q_planes, int64_t num_q, const void *g_planes, int64_t g_rows,
+                                int64_t g_plane_rows, int kp, Make make, cudaStream_t st) {
+    return planes::with_distance_mode(split, [&](auto mode) {
+        using M = decltype(mode);
+        CUtensorMap map_q, map_g;
+        int rc;
+        if ((rc = gemm::make_plane_tensor_map(&map_q, q_planes, num_q, kp, M::kP, gemm::BM, num_q))) return rc;
+        if ((rc = gemm::make_plane_tensor_map(&map_g, g_planes, g_rows, kp, M::kP, 128, g_plane_rows))) return rc;
+        return gemm::launch_split_gemm<M::kP, 128, true>(map_q, map_g, static_cast<int>(num_q), static_cast<int>(g_rows), kp,
+                                                         make(mode), st);
+    });
 }
 
 static bool metric_ok(int metric) { return metric == AGRL_METRIC_EUCLIDEAN || metric == AGRL_METRIC_COSINE; }
@@ -50,14 +52,14 @@ static bool metric_ok(int metric) { return metric == AGRL_METRIC_EUCLIDEAN || me
 using namespace agrl;
 
 extern "C" size_t agrl_distance_operand_bytes(int64_t rows, int64_t dim, int split) {
-    if (rows < 0 || dim < 1 || !split_ok(split)) return 0;
+    if (rows < 0 || dim < 1 || !planes::distance_ok(split)) return 0;
     return carve_operand(nullptr, rows, dim, split).bytes;
 }
 
 extern "C" int agrl_distance_prepare_operand_dev(const float *x, int64_t ld, int64_t rows, int64_t dim,
                                                  int metric, int split, void *operand, size_t operand_bytes,
                                                  void *stream) {
-    if (!x || rows < 0 || dim < 1 || ld < dim || !metric_ok(metric) || !split_ok(split)) return AGRL_E_INVALID;
+    if (!x || rows < 0 || dim < 1 || ld < dim || !metric_ok(metric) || !planes::distance_ok(split)) return AGRL_E_INVALID;
     if (rows > (1 << 30) || dim > (1 << 24)) return AGRL_E_UNSUPPORTED;
     int rc = agrl_device_ok();
     if (rc) return rc;
@@ -65,38 +67,30 @@ extern "C" int agrl_distance_prepare_operand_dev(const float *x, int64_t ld, int
     if (!operand || operand_bytes < o.bytes) return AGRL_E_WORKSPACE;
     const int normalize = (metric == AGRL_METRIC_COSINE);
     gemm::SplitArgs sa{x, ld, o.planes, normalize ? nullptr : o.sumsq, rows, static_cast<int>(dim),
-                       static_cast<int>(gemm::pad_k(dim)), planes_of(split), normalize};
-    if (split == AGRL_SPLIT_FP16X2) { sa.fp16x2 = 1; sa.unscale = o.unscale; }
+                       static_cast<int>(gemm::pad_k(dim)), split, normalize};
+    sa.unscale = o.unscale;
     return gemm::launch_split_planes(sa, static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int agrl_distance_prepared_dev(const void *q_operand, int64_t num_q, const void *g_operand, int64_t num_g,
                                           int64_t dim, int metric, int split, float *out, int64_t ld_out, void *stream) {
     if (!q_operand || !g_operand || !out || num_q < 0 || num_g < 0 || dim < 1 || ld_out < num_g) return AGRL_E_INVALID;
-    if (!metric_ok(metric) || !split_ok(split)) return AGRL_E_INVALID;
+    if (!metric_ok(metric) || !planes::distance_ok(split)) return AGRL_E_INVALID;
     if (num_q > (1 << 30) || num_g > (1 << 30) || dim > (1 << 24)) return AGRL_E_UNSUPPORTED;
     int rc = agrl_device_ok();
     if (rc) return rc;
     if (num_q == 0 || num_g == 0) return AGRL_OK;
     Operand q = carve_operand(const_cast<void *>(q_operand), num_q, dim, split);
     Operand g = carve_operand(const_cast<void *>(g_operand), num_g, dim, split);
-    const int kp = static_cast<int>(gemm::pad_k(dim));
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (split == AGRL_SPLIT_FP16X2) {
-        gemm::EpiDistanceF16x2 epi{q.sumsq, g.sumsq, out, ld_out, metric, q.unscale, g.unscale};
-        return launch_f16x2(q.planes, num_q, g.planes, num_g, num_g, kp, epi, st);
-    }
-    CUtensorMap map_q, map_g;
-    if ((rc = gemm::make_plane_tensor_map(&map_q, q.planes, num_q, kp, split, gemm::BM, num_q))) return rc;
-    if ((rc = gemm::make_plane_tensor_map(&map_g, g.planes, num_g, kp, split, 128, num_g))) return rc;
-    gemm::EpiDistance epi{q.sumsq, g.sumsq, out, ld_out, metric, nullptr, nullptr};
-    const int nq = static_cast<int>(num_q), ng = static_cast<int>(num_g);
-    if (split == AGRL_SPLIT_BF16X3) return gemm::launch_split_gemm<3, 128, true>(map_q, map_g, nq, ng, kp, epi, st);
-    return gemm::launch_split_gemm<2, 128, true>(map_q, map_g, nq, ng, kp, epi, st);
+    return launch_distance_gemm(split, q.planes, num_q, g.planes, num_g, num_g, static_cast<int>(gemm::pad_k(dim)),
+                                [&](auto mode) {
+                                    return gemm::EpiDistanceT<decltype(mode)::kRowScaled>{q.sumsq, g.sumsq, out, ld_out, metric,
+                                                                                          q.unscale, g.unscale};
+                                }, static_cast<cudaStream_t>(stream));
 }
 
 extern "C" size_t agrl_distance_workspace_bytes(int64_t num_q, int64_t num_g, int64_t dim, int split) {
-    if (num_q < 0 || num_g < 0 || dim < 1 || !split_ok(split)) return 0;
+    if (num_q < 0 || num_g < 0 || dim < 1 || !planes::distance_ok(split)) return 0;
     return agrl_distance_operand_bytes(num_q, dim, split) + agrl_distance_operand_bytes(num_g, dim, split);
 }
 
@@ -105,7 +99,7 @@ extern "C" int agrl_distance_dev(const float *q, int64_t ld_q, const float *g, i
                                  int metric, int split, void *ws, size_t ws_bytes, void *stream) {
     if (!q || !g || !out) return AGRL_E_INVALID;
     if (num_q < 0 || num_g < 0 || dim < 1 || ld_q < dim || ld_g < dim || ld_out < num_g) return AGRL_E_INVALID;
-    if (!metric_ok(metric) || !split_ok(split)) return AGRL_E_INVALID;
+    if (!metric_ok(metric) || !planes::distance_ok(split)) return AGRL_E_INVALID;
     int rc = agrl_device_ok();
     if (rc) return rc;
     if (num_q == 0 || num_g == 0) return AGRL_OK;
@@ -120,7 +114,7 @@ extern "C" int agrl_distance_dev(const float *q, int64_t ld_q, const float *g, i
 // ------------------------------------------------------------------------------------------------
 // Fused distance -> top-k (retrieval against a large gallery; SURVEY.md section 7 step 6, section 8d "ranking"):
 // the (num_q x num_g) matrix is never materialised.  The gallery columns are processed in launches of growing width
-// (384, then `growth` x what has been seen so far); the GEMM epilogue (EpiTopK) appends every key below the row's
+// (384, then `growth` x what has been seen so far); the GEMM epilogue (EpiTopKT) appends every key below the row's
 // threshold -- fixed during a launch -- to the row's candidate list, topk_compact_kernel keeps the K smallest and tightens
 // the threshold.  With the columns in an order unrelated to the distances a launch adds about growth x K candidates per
 // row (binomial); growth is chosen so that K + growth K + 6 sigma stays below the list capacity kTopkCap.  A list that
@@ -187,7 +181,7 @@ extern "C" int agrl_distance_topk_dev(const void *q_operand, int64_t num_q, cons
                                       int64_t dim, int metric, int split, int64_t max_rank, int64_t index_offset,
                                       uint64_t *keys, uint32_t *status, void *ws, size_t ws_bytes, void *stream) {
     if (!q_operand || !g_operand || !keys || !status || num_q < 0 || num_g < 0 || dim < 1 || index_offset < 0) return AGRL_E_INVALID;
-    if (!metric_ok(metric) || !split_ok(split) || max_rank < 1) return AGRL_E_INVALID;
+    if (!metric_ok(metric) || !planes::distance_ok(split) || max_rank < 1) return AGRL_E_INVALID;
     if (max_rank > 256 || num_q > (1 << 30) || dim > (1 << 24) || index_offset + num_g > 0xFFFFFFFFll) return AGRL_E_UNSUPPORTED;
     int rc = agrl_device_ok();
     if (rc) return rc;
@@ -202,8 +196,6 @@ extern "C" int agrl_distance_topk_dev(const void *q_operand, int64_t num_q, cons
     Operand q = carve_operand(const_cast<void *>(q_operand), num_q, dim, split);
     Operand g = carve_operand(const_cast<void *>(g_operand), num_g, dim, split);
     const int kp = static_cast<int>(gemm::pad_k(dim));
-    CUtensorMap map_q, map_g;
-    if (split != AGRL_SPLIT_FP16X2 && (rc = gemm::make_plane_tensor_map(&map_q, q.planes, num_q, kp, split, gemm::BM, num_q))) return rc;
     int64_t c0 = 0;
     // expected candidates per row and launch: growth * K (+ the K kept ones); leave 30 % of the list for the spread
     int growth = static_cast<int>(0.7 * (kTopkCap - K) / K);
@@ -217,17 +209,10 @@ extern "C" int agrl_distance_topk_dev(const void *q_operand, int64_t num_q, cons
         // the first launch may keep everything it sees (kTopkFirst <= capacity); later ones add ~growth * K per row
         int64_t width = c0 == 0 ? kTopkFirst : growth * c0;
         if (c0 + width > num_g || num_g - (c0 + width) < width / 8) width = num_g - c0;      // no tiny tail launch
-        if (split == AGRL_SPLIT_FP16X2) {
-            gemm::EpiTopKF16x2 epi{q.sumsq, g.sumsq + c0, metric, w.tau, w.cnt, w.cand, kTopkCap, static_cast<uint32_t>(index_offset + c0),
-                                   q.unscale, g.unscale + c0};
-            rc = launch_f16x2(q.planes, num_q, g.planes + c0 * kp, width, num_g, kp, epi, st);
-        } else {
-            if ((rc = gemm::make_plane_tensor_map(&map_g, g.planes + c0 * kp, width, kp, split, 128, num_g))) return rc;
-            gemm::EpiTopK epi{q.sumsq, g.sumsq + c0, metric, w.tau, w.cnt, w.cand, kTopkCap, static_cast<uint32_t>(index_offset + c0),
-                              nullptr, nullptr};
-            rc = split == AGRL_SPLIT_BF16X3 ? gemm::launch_split_gemm<3, 128, true>(map_q, map_g, nq, static_cast<int>(width), kp, epi, st)
-                                            : gemm::launch_split_gemm<2, 128, true>(map_q, map_g, nq, static_cast<int>(width), kp, epi, st);
-        }
+        rc = launch_distance_gemm(split, q.planes, num_q, g.planes + c0 * kp, width, num_g, kp, [&](auto mode) {
+            return gemm::EpiTopKT<decltype(mode)::kRowScaled>{q.sumsq, g.sumsq + c0, metric, w.tau, w.cnt, w.cand, kTopkCap,
+                                                              static_cast<uint32_t>(index_offset + c0), q.unscale, g.unscale + c0};
+        }, st);
         if (rc) return rc;
         c0 += width;
         topk_compact_kernel<<<nq, kCompactThreads, 0, st>>>(w, K, c0 >= num_g ? 1 : 0, keys, status);

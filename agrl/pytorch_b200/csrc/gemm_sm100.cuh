@@ -270,7 +270,7 @@ struct EpiDistanceT {           // distance.py:59-73 / :76-89
 };
 
 // Distance -> per-query top-k candidates, fused (SURVEY 7 step 6: the num_q x num_g matrix is never written).  Same
-// accumulation and the same final expression as EpiDistance, so every distance has the bits the matrix would hold; the
+// accumulation and the same final expression as EpiDistanceT, so every distance has the bits the matrix would hold; the
 // thread that owns (row, 64 columns) turns them into ranking keys (order-preserving distance bits << 32 | GLOBAL gallery
 // index) and appends the ones below the row's threshold -- the K-th smallest key of the columns seen by earlier
 // launches -- to the row's candidate list.  Launches cover growing column ranges; topk_compact_kernel (distance.cu) cuts
@@ -315,15 +315,11 @@ struct EpiTopKT {
         }
     }
 };
-using EpiDistance = EpiDistanceT<false>;
-using EpiDistanceF16x2 = EpiDistanceT<true>;
-using EpiTopK = EpiTopKT<false>;
-using EpiTopKF16x2 = EpiTopKT<true>;
 
 // kScaled: single-plane fp16 operands (AGRL_SPLIT_FP16X1).  Both operands were multiplied by powers of two to sit
 // in the middle of the fp16 range (per tracklet for Y, per layer for W); the epilogue undoes that exactly.
 // kFp8 (with kScaled): AGRL_SPLIT_FP16_E4M3 -- plane 0 is the scaled fp16 operand, plane 1 holds, per 64-element k-block,
-// 64 E4M3 residuals and 64 E4M3 copies of the values (see split.cu): one fp16 product + one K-concatenated 8-bit product.
+// 64 E4M3 residuals and 64 E4M3 copies of the values (planes.cuh): one fp16 product + one K-concatenated 8-bit product.
 template <bool kScaled, bool kFp8_ = false>
 struct EpiGraphLayerT {         // vmgn.py:169-172: gamma * LeakyReLU(BN(acc)) + (1-gamma) * x
     static constexpr const char *kName = "gemm_graph_layer";
@@ -427,9 +423,6 @@ struct EpiPlainT {
     }
     __device__ __forceinline__ void store_sumsq(int, int, float) const {}
 };
-using EpiGraphLayer = EpiGraphLayerT<false>;
-using EpiGraphLayerF16 = EpiGraphLayerT<true>;
-using EpiGraphLayerF16E4 = EpiGraphLayerT<true, true>;
 
 // ---- the kernel --------------------------------------------------------------------------------
 // kPair: the CTA pair (cluster of 2, tcgen05 cta_group::2) owns a 256 x BN tile.  Every CTA loads its own 128 rows of A
@@ -867,19 +860,16 @@ int launch_split_gemm(const CUtensorMap &map_a, const CUtensorMap &map_b, int M,
     return AGRL_OK;
 }
 
-// fp32 rows -> bf16 planes (+ optional squared norms / L2 normalisation); see split.cu
+// fp32 rows -> operand planes of one split format (+ optional squared norms / L2 normalisation); see split.cu
 struct SplitArgs {
     const float *src; int64_t ld;      // (rows, dim) fp32
     __nv_bfloat16 *planes;             // [P][rows][k_pad]
     float *sumsq;                      // optional: per-row sum of squares (of the un-normalised row)
-    int64_t rows; int dim; int k_pad; int P;
+    int64_t rows; int dim; int k_pad;
+    int split;                         // AGRL_SPLIT_*: the format of the planes (planes.cuh)
     int normalize;                     // 1: split x / max(||x||, 1e-12) instead of x (cosine_distance)
-    int fp16 = 0;                      // 1: ONE fp16 plane of x * (*prescale) instead of bf16 planes
-    const float *prescale = nullptr;   // device, a power of two (fp16 mode)
-    int fp16x2 = 0;                    // 1: AGRL_SPLIT_FP16X2 -- planes fp16(x s), fp16((x s - fp16(x s)) 2^11), s = 2^k per row, 1 / s -> unscale[row]
-    float *unscale = nullptr;
-    int fp8 = 0;                       // with fp16: a second plane of E4M3 pairs for the B operand of the fp16 + e4m3 GEMM --
-                                       // per 64-element k-block 64 bytes e4m3(x s 2^-6), then 64 bytes e4m3((x s - fp16(x s)) 2^6)
+    const float *prescale = nullptr;   // device, the power of two of the tensor (AGRL_SPLIT_FP16X1 / AGRL_SPLIT_FP16_E4M3)
+    float *unscale = nullptr;          // AGRL_SPLIT_FP16X2: 1 / s per row
 };
 int launch_split_planes(const SplitArgs &a, cudaStream_t st);
 

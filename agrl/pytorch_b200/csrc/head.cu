@@ -21,19 +21,13 @@
 //   attn_kernel        temporal attention (vmgn.py:276-277), part mean, BN neck -> out[:, C:] (:317-321).
 //   clip_pool_kernel   mean / max over the clips of a tracklet (train_vidreid_xent_htri.py:471-476).
 #include "gemm_sm100.cuh"
-
-#include <cuda_fp16.h>
-#include <cuda_fp8.h>
+#include "planes.cuh"
 
 namespace agrl {
 
 constexpr int kParts = 7;              // calc_splits(4) = [4,2,1] (utils/reidtools.py:13-15)
 constexpr int kMaxNodes = 64;
 constexpr int kHeadThreads = 256;
-
-// operand planes of a GEMM mode: bf16 x2 / x3, ONE scaled fp16 plane, or the fp16 plane + one plane of E4M3 pairs
-static inline int planes_of(int split) { return split == AGRL_SPLIT_FP16_E4M3 ? 2 : split; }
-static inline bool scaled_mode(int split) { return split == AGRL_SPLIT_FP16X1 || split == AGRL_SPLIT_FP16_E4M3; }
 
 // ------------------------------------------------------------------------------------------------
 // weight preparation: folded BN vectors
@@ -55,8 +49,8 @@ __global__ void fold_bn_kernel(FoldArgs a) {
     }
 }
 
-// fp16 mode: W is multiplied by the power of two that puts max|W| just below 2^14 before it is rounded to fp16
-// (fp16 keeps 11 significant bits only between 2^-14 and 2^15), and the GEMM epilogue multiplies by its inverse.
+// scaled fp16 modes: W is multiplied by the power of two of planes::f16_scales before it is rounded to fp16, and the GEMM
+// epilogue multiplies by its inverse.
 __global__ void absmax_kernel(const float *__restrict__ w, size_t n, float *slot) {
     float m = 0.f;
     for (size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; i < n; i += static_cast<size_t>(gridDim.x) * blockDim.x) {
@@ -67,15 +61,7 @@ __global__ void absmax_kernel(const float *__restrict__ w, size_t n, float *slot
     for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
     if ((threadIdx.x & 31) == 0) atomicMax(reinterpret_cast<unsigned int *>(slot + 2), __float_as_uint(m));
 }
-__device__ __forceinline__ void pow2_scales(float bound, float *up, float *down) {
-    int e = 0;
-    if (bound > 0.f) frexpf(bound, &e);                // bound = m * 2^e, m in [0.5, 1)
-    else e = 14;
-    e = max(-100, min(100, e));
-    *up = ldexpf(1.0f, 14 - e);
-    *down = ldexpf(1.0f, e - 14);
-}
-__global__ void w_scale_kernel(float *slot) { pow2_scales(slot[2], slot, slot + 1); }
+__global__ void w_scale_kernel(float *slot) { planes::f16_scales(slot[2], slot, slot + 1); }
 
 struct Prepared {                       // layout of the caller-owned "prepared" buffer
     __nv_bfloat16 *w_planes[AGRL_HEAD_MAX_LAYERS];     // [P][C][C]
@@ -88,7 +74,7 @@ static Prepared carve_prepared(const agrl_head_params *p, void *buf) {
     Carver c(buf);
     Prepared r;
     const size_t C = static_cast<size_t>(p->channels);
-    for (int l = 0; l < p->num_layers; ++l) r.w_planes[l] = c.take<__nv_bfloat16>(planes_of(p->split) * C * C);
+    for (int l = 0; l < p->num_layers; ++l) r.w_planes[l] = c.take<__nv_bfloat16>(planes::count(p->split) * C * C);
     for (int l = 0; l < p->num_layers + 2; ++l) { r.scale[l] = c.take<float>(C); r.shift[l] = c.take<float>(C); }
     r.w_scale = c.take<float>(4 * AGRL_HEAD_MAX_LAYERS);
     r.bytes = c.total();
@@ -480,19 +466,16 @@ struct GraphArgs {
     const float *x;                    // (B, V, C) layer input
     const float *adj;                  // (B, V, V) or null
     const uint64_t *masks;             // (B, 3) part-membership masks instead of adj (pose.cu), or null
-    __nv_bfloat16 *y_planes;           // [P][B*V][C]
+    __nv_bfloat16 *y_planes;           // [P][B*V][C]: A operand of the layer GEMM
     int64_t plane_stride;              // B*V*C
-    int V, C, P;
+    int V, C;
     int use_pose, learn_graph;
-    int fp16;                          // P == 1: one fp16 plane of y * 2^k, k per tracklet
+    int split;                         // AGRL_SPLIT_* of the planes; the scaled fp16 modes scale y by 2^k, k per tracklet
     float *y_unscale;                  // (B): 2^-k
     // low-rank first layer (graph_kernel_tc only): instead of Y = G.X the kernel writes G.T (B, V, 4S) and the planes of
     // the quarter-strip rows -- y_planes / plane_stride then describe [P][B*4S][C]
     int lowrank = 0;
     float *gt = nullptr;
-    // with fp16: second plane of E4M3 pairs (AGRL_SPLIT_FP16_E4M3), per 64-channel k-block 64 bytes
-    // e4m3((y s - fp16(y s)) 2^6) then 64 bytes e4m3(y s 2^-6) -- the A-operand order, W has them swapped (split.cu)
-    int fp8 = 0;
 };
 
 // element (r, c) of the pose graph: the dense matrix, or the three membership masks it is made of
@@ -563,42 +546,37 @@ static_assert((kMaxNodes * kGLd + kMaxNodes) * 4 <= kTcRingBytes, "g[] fits the 
 
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
-// 8 fp32 -> `P` bf16 planes of 8 values (16 bytes each): p0 = bf16(x), p1 = bf16(x - p0), ...
-template <int P>
-__device__ __forceinline__ void split8(const float (&v)[8], uint4 (&out)[P]) {
-    float r[8];
-#pragma unroll
-    for (int i = 0; i < 8; ++i) r[i] = v[i];
-#pragma unroll
-    for (int p = 0; p < P; ++p) {
-        uint32_t w[4];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            const __nv_bfloat162 b = __floats2bfloat162_rn(r[2 * i], r[2 * i + 1]);
-            w[i] = *reinterpret_cast<const uint32_t *>(&b);
-            r[2 * i] = __fsub_rn(r[2 * i], __uint_as_float(w[i] << 16));
-            r[2 * i + 1] = __fsub_rn(r[2 * i + 1], __uint_as_float(w[i] & 0xffff0000u));
-        }
-        out[p] = make_uint4(w[0], w[1], w[2], w[3]);
-    }
+__device__ __forceinline__ uint4 u4(const uint32_t (&w)[4]) { return make_uint4(w[0], w[1], w[2], w[3]); }
+__device__ __forceinline__ uint2 u2(const uint16_t (&b)[4]) {
+    return make_uint2(b[0] | (static_cast<uint32_t>(b[1]) << 16), b[2] | (static_cast<uint32_t>(b[3]) << 16));
 }
 
-// 8 scaled fp32 -> 8 fp16 (16 B), their residuals x 2^6 as E4M3 (8 B), the values x 2^-6 as E4M3 (8 B)
-__device__ __forceinline__ void split8_f16e4(const float (&v)[8], uint4 &h16, uint2 &res8, uint2 &val8) {
-    uint32_t hw[4], r[4], c[4];
+// 8 values of an A-operand row, channels k..k+7 -> the layer GEMM's planes (dst: channel k of the row in plane 0), 16-byte
+// stores; s: the tracklet's 2^k in the scaled modes
+__device__ __forceinline__ void store_a8(const GraphArgs &a, __nv_bfloat16 *dst, int k, const float (&v)[8], float s) {
+    if (planes::has_e4m3(a.split)) {
+        uint32_t h[4];
+        uint16_t res[4], val[4];
+        planes::encode_f16_e4m3(v, s, h, res, val);
+        *reinterpret_cast<uint4 *>(dst) = u4(h);
+        unsigned char *row8 = reinterpret_cast<unsigned char *>(dst - k + a.plane_stride);
+        *reinterpret_cast<uint2 *>(row8 + planes::e4m3_offset(k, false, true)) = u2(res);
+        *reinterpret_cast<uint2 *>(row8 + planes::e4m3_offset(k, false, false)) = u2(val);
+    } else if (planes::scaled(a.split)) {
+        uint32_t h[4];
+        planes::encode_f16(v, s, h);
+        *reinterpret_cast<uint4 *>(dst) = u4(h);
+    } else if (a.split == AGRL_SPLIT_BF16X3) {
+        uint32_t w[3][4];
+        planes::encode_bf16<3>(v, w);
 #pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        const __half2 h = __floats2half2_rn(v[2 * i], v[2 * i + 1]);
-        hw[i] = *reinterpret_cast<const uint32_t *>(&h);
-        const float2 hf = __half22float2(h);
-        // (v - h) * 64 as ONE fma: v - h is exact in fp32 and 64 a power of two, so the result is the same number
-        r[i] = __nv_cvt_float2_to_fp8x2(make_float2(fmaf(v[2 * i], 64.0f, -64.0f * hf.x), fmaf(v[2 * i + 1], 64.0f, -64.0f * hf.y)),
-                                        __NV_SATFINITE, __NV_E4M3);
-        c[i] = __nv_cvt_float2_to_fp8x2(make_float2(v[2 * i] * 0.015625f, v[2 * i + 1] * 0.015625f), __NV_SATFINITE, __NV_E4M3);
+        for (int p = 0; p < 3; ++p) *reinterpret_cast<uint4 *>(dst + p * a.plane_stride) = u4(w[p]);
+    } else {
+        uint32_t w[2][4];
+        planes::encode_bf16<2>(v, w);
+#pragma unroll
+        for (int p = 0; p < 2; ++p) *reinterpret_cast<uint4 *>(dst + p * a.plane_stride) = u4(w[p]);
     }
-    h16 = make_uint4(hw[0], hw[1], hw[2], hw[3]);
-    res8 = make_uint2(r[0] | (r[1] << 16), r[2] | (r[3] << 16));
-    val8 = make_uint2(c[0] | (c[1] << 16), c[2] | (c[3] << 16));
 }
 
 // one 32-byte store per lane (STG.256): full 32-byte sectors instead of two half-written ones
@@ -714,11 +692,11 @@ graph_kernel_tc(const __grid_constant__ CUtensorMap map_x, GraphArgs a) {
 #pragma unroll
                         for (int i = 0; i < 8; ++i) c[i] = 0.f;
                     }
-                    uint4 pl[2];
-                    split8<2>(c, pl);
+                    uint32_t pl[2][4];
+                    planes::encode_bf16<2>(c, pl);
                     const int off = row * 128 + ((slot ^ (row & 7)) << 4);
 #pragma unroll
-                    for (int p = 0; p < 2; ++p) *reinterpret_cast<uint4 *>(dst + p * kTcPlane + off) = pl[p];
+                    for (int p = 0; p < 2; ++p) *reinterpret_cast<uint4 *>(dst + p * kTcPlane + off) = u4(pl[p]);
                 }
                 fence_proxy_async_smem();
                 __syncwarp();
@@ -811,7 +789,7 @@ graph_kernel_tc(const __grid_constant__ CUtensorMap map_x, GraphArgs a) {
     __syncthreads();
     __shared__ float s_scale[2];
     float y_scale = 1.0f;
-    if (a.fp16) {                                                      // see graph_kernel
+    if (planes::scaled(a.split)) {                                     // see graph_kernel
         if (!a.learn_graph) {
             if (worker) {
                 for (int r = warp; r < V; r += 12) {
@@ -842,7 +820,7 @@ graph_kernel_tc(const __grid_constant__ CUtensorMap map_x, GraphArgs a) {
             }
             if (lane == 0) {
                 m = (m < 3.0e38f && refn < 3.0e38f) ? sqrtf(m) + sqrtf(refn) : 0.f;
-                pow2_scales(m, &s_scale[0], &s_scale[1]);
+                planes::f16_scales(m, &s_scale[0], &s_scale[1]);
                 a.y_unscale[b] = s_scale[1];
             }
         }
@@ -868,37 +846,7 @@ graph_kernel_tc(const __grid_constant__ CUtensorMap map_x, GraphArgs a) {
                 const float4 *src = reinterpret_cast<const float4 *>(x + static_cast<size_t>(row) * C + cg * 8);
                 const float4 lo = __ldg(src), hi = __ldg(src + 1);
                 const float v[8] = {lo.x, lo.y, lo.z, lo.w, hi.x, hi.y, hi.z, hi.w};
-                __nv_bfloat16 *dst = a.y_planes + (static_cast<size_t>(b) * S4 + qr) * C + cg * 8;
-                if (a.fp8) {
-                    float vs[8];
-#pragma unroll
-                    for (int t = 0; t < 8; ++t) vs[t] = v[t] * y_scale;
-                    uint4 h16; uint2 r8, c8;
-                    split8_f16e4(vs, h16, r8, c8);
-                    *reinterpret_cast<uint4 *>(dst) = h16;
-                    unsigned char *row8 = reinterpret_cast<unsigned char *>(a.y_planes + a.plane_stride + (static_cast<size_t>(b) * S4 + qr) * C) +
-                                          (cg >> 3) * 128 + (cg & 7) * 8;
-                    *reinterpret_cast<uint2 *>(row8) = r8;
-                    *reinterpret_cast<uint2 *>(row8 + 64) = c8;
-                } else if (a.fp16) {
-                    uint32_t w[4];
-#pragma unroll
-                    for (int t = 0; t < 4; ++t) {
-                        const __half2 h = __floats2half2_rn(v[2 * t] * y_scale, v[2 * t + 1] * y_scale);
-                        w[t] = *reinterpret_cast<const uint32_t *>(&h);
-                    }
-                    *reinterpret_cast<uint4 *>(dst) = make_uint4(w[0], w[1], w[2], w[3]);
-                } else if (a.P == 3) {
-                    uint4 pl[3];
-                    split8<3>(v, pl);
-#pragma unroll
-                    for (int pp = 0; pp < 3; ++pp) *reinterpret_cast<uint4 *>(dst + pp * a.plane_stride) = pl[pp];
-                } else {
-                    uint4 pl[2];
-                    split8<2>(v, pl);
-#pragma unroll
-                    for (int pp = 0; pp < 2; ++pp) *reinterpret_cast<uint4 *>(dst + pp * a.plane_stride) = pl[pp];
-                }
+                store_a8(a, a.y_planes + (static_cast<size_t>(b) * S4 + qr) * C + cg * 8, cg * 8, v, y_scale);
             }
         }
         gemm::tc_fence_before();
@@ -914,11 +862,11 @@ graph_kernel_tc(const __grid_constant__ CUtensorMap map_x, GraphArgs a) {
             float v[8];
 #pragma unroll
             for (int i = 0; i < 8; ++i) v[i] = (row < V) ? g[row * kGLd + slot * 8 + i] : 0.f;    // columns >= V hold zeros
-            uint4 pl[2];
-            split8<2>(v, pl);
+            uint32_t pl[2][4];
+            planes::encode_bf16<2>(v, pl);
             const int off = row * 128 + ((slot ^ (row & 7)) << 4);
-            *reinterpret_cast<uint4 *>(smem + kTcGPlanes + off) = pl[0];
-            *reinterpret_cast<uint4 *>(smem + kTcGPlanes + kTcPlane + off) = pl[1];
+            *reinterpret_cast<uint4 *>(smem + kTcGPlanes + off) = u4(pl[0]);
+            *reinterpret_cast<uint4 *>(smem + kTcGPlanes + kTcPlane + off) = u4(pl[1]);
         }
         fence_proxy_async_smem();
     }
@@ -984,11 +932,11 @@ graph_kernel_tc(const __grid_constant__ CUtensorMap map_x, GraphArgs a) {
             const int row = (hh & 1) * 64 + ch;
 #pragma unroll
             for (int t = 0; t < 2; ++t) {
-                uint4 pl[2];
-                split8<2>(nx[t], pl);
+                uint32_t pl[2][4];
+                planes::encode_bf16<2>(nx[t], pl);
                 const int off = row * 128 + (((g0 + 4 * t) ^ (row & 7)) << 4);
-                *reinterpret_cast<uint4 *>(dst + off) = pl[0];
-                *reinterpret_cast<uint4 *>(dst + 2 * kTcPlane + off) = pl[1];
+                *reinterpret_cast<uint4 *>(dst + off) = u4(pl[0]);
+                *reinterpret_cast<uint4 *>(dst + 2 * kTcPlane + off) = u4(pl[1]);
             }
             // the stage may be refilled only now: the shared-memory reads above have certainly completed once their values
             // have been converted and stored (an arrive right after the loads lets the bulk copy -- another proxy -- overtake them)
@@ -1023,53 +971,37 @@ graph_kernel_tc(const __grid_constant__ CUtensorMap map_x, GraphArgs a) {
                     if (warp == 0) AGRL_TL(80 + cb);
                 }
                 if (erow < V) {
-                    __nv_bfloat16 *dst = a.y_planes + (static_cast<size_t>(b) * V + erow) * C + cb * 128 + ehalf * 64 + hq * 32;
-                    if (a.fp8) {
+                    const int k = cb * 128 + ehalf * 64 + hq * 32;
+                    __nv_bfloat16 *dst = a.y_planes + (static_cast<size_t>(b) * V + erow) * C + k;
+                    if (planes::has_e4m3(a.split)) {
                         // this thread's 64 channels are exactly k-block 2 cb + ehalf of the row
                         unsigned char *row8 = reinterpret_cast<unsigned char *>(a.y_planes + a.plane_stride + (static_cast<size_t>(b) * V + erow) * C) +
-                                              (cb * 2 + ehalf) * 128 + hq * 32;
+                                              planes::e4m3_offset(k, false, true);
                         // 32 channels: 64 bytes of fp16, 32 bytes of residuals, 32 bytes of value copies -> four 32-byte stores
-                        uint4 h16[4]; uint2 r8[4], c8[4];
+                        uint4 h16[4];
+                        uint2 r8[4], c8[4];
 #pragma unroll
                         for (int e = 0; e < 4; ++e) {
                             float v[8];
 #pragma unroll
-                            for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[0][8 * e + i]) * y_scale;
-                            split8_f16e4(v, h16[e], r8[e], c8[e]);
+                            for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[0][8 * e + i]);
+                            uint32_t h[4];
+                            uint16_t res[4], val[4];
+                            planes::encode_f16_e4m3(v, y_scale, h, res, val);
+                            h16[e] = u4(h); r8[e] = u2(res); c8[e] = u2(val);
                         }
                         st256(dst, h16[0], h16[1]);
                         st256(dst + 16, h16[2], h16[3]);
                         st256(row8, make_uint4(r8[0].x, r8[0].y, r8[1].x, r8[1].y), make_uint4(r8[2].x, r8[2].y, r8[3].x, r8[3].y));
-                        st256(row8 + 64, make_uint4(c8[0].x, c8[0].y, c8[1].x, c8[1].y), make_uint4(c8[2].x, c8[2].y, c8[3].x, c8[3].y));
-                    } else if (a.fp16) {
-#pragma unroll
-                        for (int q = 0; q < 4; ++q) {
-                            uint32_t w[4];
-#pragma unroll
-                            for (int i = 0; i < 4; ++i) {
-                                const __half2 h = __floats2half2_rn(__uint_as_float(r[0][8 * q + 2 * i]) * y_scale,
-                                                                    __uint_as_float(r[0][8 * q + 2 * i + 1]) * y_scale);
-                                w[i] = *reinterpret_cast<const uint32_t *>(&h);
-                            }
-                            reinterpret_cast<uint4 *>(dst)[q] = make_uint4(w[0], w[1], w[2], w[3]);
-                        }
+                        st256(row8 + (planes::e4m3_offset(k, false, false) - planes::e4m3_offset(k, false, true)),
+                              make_uint4(c8[0].x, c8[0].y, c8[1].x, c8[1].y), make_uint4(c8[2].x, c8[2].y, c8[3].x, c8[3].y));
                     } else {
 #pragma unroll
                         for (int q = 0; q < 4; ++q) {
                             float v[8];
 #pragma unroll
                             for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[0][8 * q + i]);
-                            if (a.P == 3) {
-                                uint4 pl[3];
-                                split8<3>(v, pl);
-#pragma unroll
-                                for (int p = 0; p < 3; ++p) reinterpret_cast<uint4 *>(dst + p * a.plane_stride)[q] = pl[p];
-                            } else {
-                                uint4 pl[2];
-                                split8<2>(v, pl);
-#pragma unroll
-                                for (int p = 0; p < 2; ++p) reinterpret_cast<uint4 *>(dst + p * a.plane_stride)[q] = pl[p];
-                            }
+                            store_a8(a, dst + 8 * q, k + 8 * q, v, y_scale);
                         }
                     }
                 }
@@ -1248,7 +1180,7 @@ static bool lowrank_enabled(const agrl_head_params *p, int S) {
 
 // partial row sums of squares that the last layer's GEMM epilogue leaves for the attention: one per (column tile, half)
 static int sumsq_slots_of(const agrl_head_params *p) {
-    const int bn = p->split == AGRL_SPLIT_BF16X3 ? 128 : 256;
+    const int bn = planes::head_bn(p->split);
     return 2 * ((p->channels + bn - 1) / bn);
 }
 
@@ -1258,7 +1190,7 @@ static HeadWorkspace carve_head(const agrl_head_params *p, void *ws, int64_t bat
     const size_t n = static_cast<size_t>(batch) * S * kParts * p->channels;
     w.x[0] = c.take<float>(n);
     w.x[1] = c.take<float>(n);
-    w.y_planes = c.take<__nv_bfloat16>(static_cast<size_t>(planes_of(p->split)) * n);
+    w.y_planes = c.take<__nv_bfloat16>(static_cast<size_t>(planes::count(p->split)) * n);
     w.y_unscale = c.take<float>(static_cast<size_t>(batch));
     // no fewer than 32 floats per row, so that the workspace size of every split at C <= 2048 stays what callers allocate
     const int sumsq_room = sumsq_slots_of(p) > 32 ? sumsq_slots_of(p) : 32;
@@ -1273,8 +1205,7 @@ static HeadWorkspace carve_head(const agrl_head_params *p, void *ws, int64_t bat
 static int check_params(const agrl_head_params *p) {
     if (!p) return AGRL_E_INVALID;
     if (p->num_layers < 0 || p->num_layers > AGRL_HEAD_MAX_LAYERS) return AGRL_E_INVALID;
-    if (p->split != AGRL_SPLIT_BF16X2 && p->split != AGRL_SPLIT_BF16X3 && p->split != AGRL_SPLIT_FP16X1 &&
-        p->split != AGRL_SPLIT_FP16_E4M3) return AGRL_E_INVALID;
+    if (!planes::head_ok(p->split)) return AGRL_E_INVALID;
     if (p->channels < kChunk || p->channels % kChunk != 0) return AGRL_E_UNSUPPORTED;
     if (!p->use_pose && !p->learn_graph) return AGRL_E_INVALID;            // vmgn.py:92 assert
     if (p->pool_stages != 0 && (p->pool_stages < 2 || p->pool_stages > 12)) return AGRL_E_INVALID;
@@ -1323,16 +1254,15 @@ extern "C" int agrl_head_prepare_dev(const agrl_head_params *p, void *prepared, 
     for (int l = 0; l < p->num_layers; ++l) {
         if (!p->linear_weight[l] || !p->bn_weight[l] || !p->bn_bias[l] || !p->bn_mean[l] || !p->bn_var[l]) return AGRL_E_INVALID;
         fa.w[l] = p->bn_weight[l]; fa.b[l] = p->bn_bias[l]; fa.mean[l] = p->bn_mean[l]; fa.var[l] = p->bn_var[l];
-        gemm::SplitArgs sa{p->linear_weight[l], C, pr.w_planes[l], nullptr, C, C, C, planes_of(p->split), 0};
-        if (scaled_mode(p->split)) {
+        gemm::SplitArgs sa{p->linear_weight[l], C, pr.w_planes[l], nullptr, C, C, C, p->split, 0};
+        if (planes::scaled(p->split)) {
             float *slot = pr.w_scale + 4 * l;
             AGRL_CUDA_TRY(cudaMemsetAsync(slot, 0, 4 * sizeof(float), st));
             absmax_kernel<<<4 * kNumSMs, 256, 0, st>>>(p->linear_weight[l], static_cast<size_t>(C) * C, slot);
             AGRL_LAUNCH_CHECK(st, "absmax");
             w_scale_kernel<<<1, 1, 0, st>>>(slot);
             AGRL_LAUNCH_CHECK(st, "w_scale");
-            sa.fp16 = 1; sa.prescale = slot;
-            sa.fp8 = p->split == AGRL_SPLIT_FP16_E4M3;
+            sa.prescale = slot;
         }
         if ((rc = gemm::launch_split_planes(sa, st))) return rc;
     }
@@ -1414,25 +1344,24 @@ static int launch_pool_any(const agrl_head_params *p, const Prepared &pr, const 
     }
 }
 
-// one GEMM of a graph layer in the caller's operand mode; Epi is built by `make(fp8)` for the scaled modes
-template <class EpiBf16, class EpiF16, class EpiF16E4>
+// one GEMM of a graph layer in the layer's operand mode; make(mode) builds the epilogue of that mode.  fp16 + E4M3 runs as
+// CTA pairs (cta_group::2, each CTA loads half of the W tile) unless `pair` is off.
+template <class Make>
 static int launch_layer_gemm(int split, bool pair, const CUtensorMap &map_a, const CUtensorMap &map_w, int rows, int C,
-                             const EpiBf16 &e2, const EpiF16 &e1, const EpiF16E4 &e4, cudaStream_t st) {
-    switch (split) {
-        case AGRL_SPLIT_FP16X1: return gemm::launch_split_gemm<1, 256, false>(map_a, map_w, rows, C, C, e1, st);
-        case AGRL_SPLIT_FP16_E4M3:
-            return pair ? gemm::launch_pair_gemm<2, 256, false>(map_a, map_w, rows, C, C, e4, st)
-                        : gemm::launch_split_gemm<2, 256, false>(map_a, map_w, rows, C, C, e4, st);
-        case AGRL_SPLIT_BF16X3: return gemm::launch_split_gemm<3, 128, false>(map_a, map_w, rows, C, C, e2, st);
-        default: return gemm::launch_split_gemm<2, 256, false>(map_a, map_w, rows, C, C, e2, st);
-    }
+                             Make make, cudaStream_t st) {
+    return planes::with_head_mode(split, [&](auto mode) {
+        using M = decltype(mode);
+        if constexpr (M::kFp8)
+            if (pair) return gemm::launch_pair_gemm<M::kP, M::kHeadBN, false>(map_a, map_w, rows, C, C, make(mode), st);
+        return gemm::launch_split_gemm<M::kP, M::kHeadBN, false>(map_a, map_w, rows, C, C, make(mode), st);
+    });
 }
 
 // graph layers + attention of `n` tracklets starting at tracklet `b0` (their nodes are in hwk.x[0])
 static int launch_layers(const agrl_head_params *p, const Prepared &pr, HeadWorkspace hwk, const float *adj,
                          const uint64_t *masks, float *out,
                          int64_t ld_out, float *nodes_out, int64_t b0, int64_t n, int64_t batch, int S, cudaStream_t st) {
-    const int C = p->channels, V = S * kParts, L = p->num_layers, P = planes_of(p->split);
+    const int C = p->channels, V = S * kParts, L = p->num_layers, P = planes::count(p->split);
     const int64_t rows = n * V, row0 = b0 * V, all_rows = batch * V;
     float *x[2] = {hwk.x[0] + row0 * C, hwk.x[1] + row0 * C};
     __nv_bfloat16 *y = hwk.y_planes + row0 * C;
@@ -1444,13 +1373,12 @@ static int launch_layers(const agrl_head_params *p, const Prepared &pr, HeadWork
     int attn_slots = 0;
     CUtensorMap map_y, map_w;
     if (L > 0 && (rc = gemm::make_plane_tensor_map(&map_y, y, rows, C, P, gemm::BM, all_rows))) return rc;
-    const int scaled = scaled_mode(p->split), fp8 = p->split == AGRL_SPLIT_FP16_E4M3;
-    const int bn = p->split == AGRL_SPLIT_BF16X3 ? 128 : 256;
-    const bool pair = fp8 && !p->gemm_no_pair;              // CTA pairs (cta_group::2): each CTA loads half of the W tile
+    const int bn = planes::head_bn(p->split);
+    const bool pair = planes::has_e4m3(p->split) && !p->gemm_no_pair;
     int cur = 0;
     for (int l = 0; l < L; ++l) {
-        GraphArgs ga{x[cur], adj, masks, y, all_rows * C, V, C, P, p->use_pose, p->learn_graph, scaled, hwk.y_unscale + b0};
-        ga.fp8 = fp8;
+        GraphArgs ga{x[cur], adj, masks, y, all_rows * C, V, C, p->use_pose, p->learn_graph, p->split, hwk.y_unscale + b0};
+        const float *w_unscale = pr.w_scale + 4 * l + 1;
         float *dst = (l == L - 1 && nodes_out) ? nodes_out : x[cur ^ 1];
         if ((rc = gemm::make_plane_tensor_map(&map_w, pr.w_planes[l], C, C, P, pair ? bn / 2 : bn, C))) return rc;
         // Low-rank first layer: only layer 0 sees nodes that are T.(quarter strips)
@@ -1465,10 +1393,11 @@ static int launch_layers(const agrl_head_params *p, const Prepared &pr, HeadWork
             CUtensorMap map_q;
             if ((rc = gemm::make_plane_tensor_map(&map_q, yq, qrows, C, P, gemm::BM, q_all))) return rc;
             AGRL_LAUNCH_BEGIN(st);
-            gemm::EpiPlainT<false> z2{z, C, nullptr, nullptr, S4};
-            gemm::EpiPlainT<true> z1{z, C, hwk.y_unscale + b0, pr.w_scale + 4 * l + 1, S4};
-            gemm::EpiPlainT<true, true> z4{z, C, hwk.y_unscale + b0, pr.w_scale + 4 * l + 1, S4};
-            if ((rc = launch_layer_gemm(p->split, pair, map_q, map_w, static_cast<int>(qrows), C, z2, z1, z4, st))) return rc;
+            rc = launch_layer_gemm(p->split, pair, map_q, map_w, static_cast<int>(qrows), C, [&](auto mode) {
+                using M = decltype(mode);
+                return gemm::EpiPlainT<M::kScaled, M::kFp8>{z, C, hwk.y_unscale + b0, w_unscale, S4};
+            }, st);
+            if (rc) return rc;
             MixArgs ma{x[cur], z, ga.gt, dst, pr.scale[l], pr.shift[l], V, S4, C, p->gamma, p->leaky_slope};
             AGRL_LAUNCH_BEGIN(st);
             if (S4 <= 32) graph_mix_kernel<32><<<dim3(C / (2 * kHeadThreads), static_cast<unsigned>(n)), kHeadThreads, 0, st>>>(ma);
@@ -1483,15 +1412,16 @@ static int launch_layers(const agrl_head_params *p, const Prepared &pr, HeadWork
         const int sumsq_slots = sumsq_slots_of(p);
         float *sumsq = (l == L - 1 && C % bn == 0) ? hwk.row_sumsq + row0 * sumsq_slots : nullptr;
         if (sumsq) { attn_sumsq = sumsq; attn_slots = sumsq_slots; }
-        gemm::EpiGraphLayer e2{x[cur], pr.scale[l], pr.shift[l], dst, C, C, p->gamma, p->leaky_slope, nullptr, nullptr, V};
-        gemm::EpiGraphLayerF16 e1{x[cur], pr.scale[l], pr.shift[l], dst, C, C, p->gamma, p->leaky_slope,
-                                  hwk.y_unscale + b0, pr.w_scale + 4 * l + 1, V};
-        gemm::EpiGraphLayerF16E4 e4{x[cur], pr.scale[l], pr.shift[l], dst, C, C, p->gamma, p->leaky_slope,
-                                    hwk.y_unscale + b0, pr.w_scale + 4 * l + 1, V};
-        e2.row_sumsq = e1.row_sumsq = e4.row_sumsq = sumsq;
-        e2.sumsq_slots = e1.sumsq_slots = e4.sumsq_slots = sumsq ? sumsq_slots : 0;
         AGRL_LAUNCH_BEGIN(st);
-        if ((rc = launch_layer_gemm(p->split, pair, map_y, map_w, static_cast<int>(rows), C, e2, e1, e4, st))) return rc;
+        rc = launch_layer_gemm(p->split, pair, map_y, map_w, static_cast<int>(rows), C, [&](auto mode) {
+            using M = decltype(mode);
+            gemm::EpiGraphLayerT<M::kScaled, M::kFp8> e{x[cur], pr.scale[l], pr.shift[l], dst, C, C, p->gamma, p->leaky_slope,
+                                                        hwk.y_unscale + b0, w_unscale, V};
+            e.row_sumsq = sumsq;
+            e.sumsq_slots = sumsq ? sumsq_slots : 0;
+            return e;
+        }, st);
+        if (rc) return rc;
         if (dst == nodes_out) x[cur ^ 1] = nodes_out;
         cur ^= 1;
     }

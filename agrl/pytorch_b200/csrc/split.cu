@@ -1,14 +1,11 @@
-// split.cu -- fp32 rows -> bf16 operand planes for the tcgen05 GEMMs, plus the TMA descriptors.
-//
-//   x = p0 + p1 (+ p2),  p0 = bf16(x), p1 = bf16(x - p0), p2 = bf16(x - p0 - p1)
-// The residuals are exact in fp32, so three planes carry all 24 significand bits of x.
+// split.cu -- fp32 rows -> operand planes for the tcgen05 GEMMs in any split format (planes.cuh), plus the TMA
+// descriptors.  Rows are B operands (and both operands of the distance GEMM); the E4M3 plane is written in B order.
 // The same pass produces what the distance epilogues need: the per-row sum of squares
 // (euclidean_squared_distance, distance.py:70-71) or the L2-normalised row x / max(||x||, 1e-12)
 // (cosine_distance, distance.py:86-87: F.normalize then mm).
 #include "gemm_sm100.cuh"
+#include "planes.cuh"
 
-#include <cuda_fp16.h>
-#include <cuda_fp8.h>
 #include <mutex>
 
 namespace agrl {
@@ -25,9 +22,10 @@ split_planes_kernel(SplitArgs a) {
     const int tid = threadIdx.x;
     const float *src = a.src + row * a.ld;
     const bool vec = ((reinterpret_cast<uintptr_t>(src) & 15u) == 0) && (a.dim % 4 == 0);
+    const bool row_scaled = planes::row_scaled(a.split);
 
     float inv = 1.0f, ps = 1.0f;
-    if (a.sumsq != nullptr || a.normalize || a.fp16x2) {
+    if (a.sumsq != nullptr || a.normalize || row_scaled) {
         float s = 0.f, m = 0.f;
         if (vec) {
             const float4 *s4 = reinterpret_cast<const float4 *>(src);
@@ -51,62 +49,44 @@ split_planes_kernel(SplitArgs a) {
             if (a.sumsq) a.sumsq[row] = t;
             const float nrm = fmaxf(sqrtf(t), 1e-12f);       // F.normalize: x / max(||x||_2, eps)
             s_inv = nrm;
-            if (a.fp16x2) {
-                // power of two that puts the row's largest (normalised) magnitude in [2^7, 2^8); rows that are all zero,
-                // or hold Inf / NaN (fmaxf drops NaNs, the sum of squares keeps them), stay unscaled
-                if (a.normalize) mx = __fdiv_rn(mx, nrm);
-                int e = 7;
-                if (mx > 0.f && mx < 3.0e38f && t == t) e = ilogbf(mx);
-                e = max(-110, min(120, e));
-                s_ps = ldexpf(1.0f, 7 - e);
-                a.unscale[row] = ldexpf(1.0f, e - 7);
-            }
+            if (row_scaled) planes::f16x2_scales(a.normalize ? __fdiv_rn(mx, nrm) : mx, t, &s_ps, a.unscale + row);
         }
         __syncthreads();
         inv = s_inv;
-        if (a.fp16x2) ps = s_ps;
+        if (row_scaled) ps = s_ps;
     }
 
     const size_t plane_stride = static_cast<size_t>(a.rows) * a.k_pad;
     __nv_bfloat16 *dst = a.planes + row * a.k_pad;
     // pairs of elements -> one 32-bit store per plane
     for (int i = 2 * tid; i < a.k_pad; i += 2 * kSplitThreads) {
-        float x0 = (i < a.dim) ? src[i] : 0.f;
-        float x1 = (i + 1 < a.dim) ? src[i + 1] : 0.f;
-        if (a.normalize) { x0 = __fdiv_rn(x0, inv); x1 = __fdiv_rn(x1, inv); }
-        if (a.fp16x2) {
-            x0 *= ps; x1 *= ps;                                   // exact
-            const __half2 h = __floats2half2_rn(x0, x1);
-            const float2 hf = __half22float2(h);
-            // (x - h is exact in fp32; 2^11 lifts the residual into fp16's normal range)
-            const __half2 l = __floats2half2_rn(__fsub_rn(x0, hf.x) * 2048.0f, __fsub_rn(x1, hf.y) * 2048.0f);
-            *reinterpret_cast<__half2 *>(dst + i) = h;
-            *reinterpret_cast<__half2 *>(dst + plane_stride + i) = l;
-            continue;
-        }
-        if (a.fp16) {
-            const float ps = __ldg(a.prescale);
-            const __half2 h = __floats2half2_rn(x0 * ps, x1 * ps);
-            *reinterpret_cast<__half2 *>(dst + i) = h;
-            if (a.fp8) {
-                // B-operand layout of the 8-bit plane: [value copies | residuals] per 64-element k-block
-                const float2 hf = __half22float2(h);
-                unsigned char *row8 = reinterpret_cast<unsigned char *>(dst + plane_stride) + (i >> 6) * 128 + (i & 63);
-                *reinterpret_cast<__nv_fp8x2_storage_t *>(row8) =
-                    __nv_cvt_float2_to_fp8x2(make_float2(x0 * ps * 0.015625f, x1 * ps * 0.015625f), __NV_SATFINITE, __NV_E4M3);
-                *reinterpret_cast<__nv_fp8x2_storage_t *>(row8 + 64) =
-                    __nv_cvt_float2_to_fp8x2(make_float2(__fsub_rn(x0 * ps, hf.x) * 64.0f, __fsub_rn(x1 * ps, hf.y) * 64.0f),
-                                             __NV_SATFINITE, __NV_E4M3);
-            }
-            continue;
-        }
+        float x[2] = {(i < a.dim) ? src[i] : 0.f, (i + 1 < a.dim) ? src[i + 1] : 0.f};
+        if (a.normalize) { x[0] = __fdiv_rn(x[0], inv); x[1] = __fdiv_rn(x[1], inv); }
+        uint32_t *w0 = reinterpret_cast<uint32_t *>(dst + i), *w1 = reinterpret_cast<uint32_t *>(dst + plane_stride + i);
+        if (row_scaled) {
+            uint32_t h[1], l[1];
+            planes::encode_f16x2(x, ps, h, l);
+            *w0 = h[0]; *w1 = l[0];
+        } else if (planes::has_e4m3(a.split)) {
+            uint32_t h[1];
+            uint16_t res[1], val[1];
+            planes::encode_f16_e4m3(x, __ldg(a.prescale), h, res, val);
+            *w0 = h[0];
+            unsigned char *row8 = reinterpret_cast<unsigned char *>(dst + plane_stride);
+            *reinterpret_cast<uint16_t *>(row8 + planes::e4m3_offset(i, true, true)) = res[0];
+            *reinterpret_cast<uint16_t *>(row8 + planes::e4m3_offset(i, true, false)) = val[0];
+        } else if (planes::scaled(a.split)) {
+            uint32_t h[1];
+            planes::encode_f16(x, __ldg(a.prescale), h);
+            *w0 = h[0];
+        } else {
 #pragma unroll
-        for (int p = 0; p < 3; ++p) {
-            if (p < a.P) {
-                const __nv_bfloat16 b0 = __float2bfloat16_rn(x0), b1 = __float2bfloat16_rn(x1);
-                *reinterpret_cast<__nv_bfloat162 *>(dst + p * plane_stride + i) = __halves2bfloat162(b0, b1);
-                x0 = __fsub_rn(x0, __bfloat162float(b0));
-                x1 = __fsub_rn(x1, __bfloat162float(b1));
+            for (int p = 0; p < 3; ++p) {
+                if (p < planes::count(a.split)) {
+                    uint32_t w[1];
+                    planes::bf16_plane(x, w);
+                    *reinterpret_cast<uint32_t *>(dst + p * plane_stride + i) = w[0];
+                }
             }
         }
     }
