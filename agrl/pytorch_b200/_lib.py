@@ -79,6 +79,9 @@ _SIGNATURES = {
     'agrl_rank_mars_classify_workspace_bytes': (c_sz, [c_i64, c_i64]),
     'agrl_rank_mars_classify_dev': (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_i64, c_i64, c_vp, c_vp, c_vp,
                                             c_vp, c_sz, c_vp]),
+    'agrl_rank_lists_dev': (c_int, [c_vp, c_i64, c_i64, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_i64, c_int, c_vp, c_vp,
+                                    c_i64, c_vp, c_vp, c_sz, c_vp]),
+    'agrl_rank_junk_depth_dev': (c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_sz, c_vp]),
     'agrl_pose_part_masks_dev': (c_int, [c_vp, c_vp, c_vp, c_i64, c_i32, c_i32, ctypes.c_double, c_vp, c_vp]),
     'agrl_pose_adjacency_dev': (c_int, [c_vp, c_i64, c_i32, c_vp, c_vp]),
     'agrl_head_forward_compact_dev': (c_int, [ctypes.POINTER(HeadParams), c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp,

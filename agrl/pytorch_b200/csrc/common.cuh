@@ -64,6 +64,11 @@ __device__ __forceinline__ uint32_t mono_key(float d) {
     uint32_t u = __float_as_uint(d + 0.0f);          // -0.0f + 0.0f == +0.0f
     return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
 }
+// Inverse of mono_key: the bits of the distance that was ranked.  A -0 was ranked as +0 and comes back as +0; every NaN
+// was ranked as 0xFFFFFFFF and comes back as the NaN 0x7FFFFFFF.
+__device__ __forceinline__ float mono_key_value(uint32_t k) {
+    return __uint_as_float((k & 0x80000000u) ? (k & 0x7FFFFFFFu) : ~k);
+}
 __device__ __forceinline__ uint64_t rank_key(float d, uint32_t idx) {
     return (static_cast<uint64_t>(mono_key(d)) << 32) | idx;
 }

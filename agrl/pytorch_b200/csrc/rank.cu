@@ -681,6 +681,22 @@ rank_mars_kernel(MarsArgs a) {
     mars_compute_ap(cls, valid, s_ngood, &a.res.ap[q], &a.res.first_pos[q], a.status);
 }
 
+// Position of `key`, entry `pos` of list p, in the merge of `parts` ascending key lists (list o at lists + o * stride) whose
+// real keys are unique: pos plus, for every other list, the number of its keys below `key` (a binary search over the
+// list's first n entries).  Positions from n on are not needed: the count stops there, and the result is then >= n.
+__device__ __forceinline__ int merged_position(const uint64_t *lists, int parts, int stride, int n, int p, int pos,
+                                               uint64_t key) {
+    int rank = pos;
+    for (int o = 0; o < parts && rank < n; ++o) {
+        if (o == p) continue;
+        const uint64_t *lst = lists + o * stride;
+        int lo = 0, hi = n;
+        while (lo < hi) { const int mid = (lo + hi) >> 1; if (lst[mid] < key) lo = mid + 1; else hi = mid; }
+        rank += lo;
+    }
+    return rank;
+}
+
 // Merge of the shards' candidates: one CTA per query sorts parts*K (key, class) pairs and runs
 // Compute_AP on the first K.  keys/cls are laid out [part][query][K].
 struct MarsMergeArgs {
@@ -726,14 +742,7 @@ rank_mars_merge_kernel(MarsMergeArgs a) {
             const uint64_t key = keys[i];
             if (key == kKeyMax) continue;
             const int p = i / K;
-            int rank = i - p * K;
-            for (int o = 0; o < a.parts && rank < K; ++o) {
-                if (o == p) continue;
-                const uint64_t *lst = keys + o * K;
-                int lo = 0, hi = K;
-                while (lo < hi) { const int mid = (lo + hi) >> 1; if (lst[mid] < key) lo = mid + 1; else hi = mid; }
-                rank += lo;
-            }
+            const int rank = merged_position(keys, a.parts, K, K, p, i - p * K, key);
             if (rank < K) { okeys[rank] = key; ocls[rank] = cls[i]; }
         }
         __syncthreads();
@@ -1312,6 +1321,103 @@ __global__ void classify_keys_kernel(ClassifyWorkspace w, const uint64_t *__rest
     }
 }
 
+// the most gallery items that share a query's pid and camera, over the queries
+__global__ void rank_junk_depth_kernel(ClassifyWorkspace w, int nq, int32_t *junk_depth) {
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= nq) return;
+    const int h = probe_pid_cam<false>(w, w.q_pid[q], w.q_cam[q]);
+    if (h >= 0) atomicMax(junk_depth, w.cnt_pc[h]);
+}
+
+// Labels to int32, the queries' identities into the two tables, one pass over the gallery labels counting into them.
+static int build_label_tables(const ClassifyWorkspace &w, const int64_t *q_pids, const int64_t *g_pids,
+                              const int64_t *q_camids, const int64_t *g_camids, int64_t num_q, int64_t num_g,
+                              uint32_t *status, cudaStream_t st) {
+    int rc = narrow_labels(q_pids, g_pids, q_camids, g_camids, num_q, num_g, w.q_pid, w.g_pid, w.q_cam, w.g_cam,
+                           status, st);
+    if (rc) return rc;
+    AGRL_CUDA_TRY(cudaMemsetAsync(w.tab_p, 0xFF, sizeof(int32_t) * 2 * w.slots, st));       // both tables: empty (-1)
+    AGRL_CUDA_TRY(cudaMemsetAsync(w.cnt_p, 0, sizeof(int32_t) * 2 * w.slots, st));
+    const int nq = static_cast<int>(num_q);
+    classify_insert_kernel<<<(nq + 255) / 256, 256, 0, st>>>(w, nq);
+    AGRL_LAUNCH_CHECK(st, "classify_insert");
+    if (num_g > 0) {
+        int cb = static_cast<int>((num_g + 255) / 256);
+        if (cb > 8 * kNumSMs) cb = 8 * kNumSMs;
+        classify_count_kernel<<<cb, 256, 0, st>>>(w, num_g);
+        AGRL_LAUNCH_CHECK(st, "classify_count");
+    }
+    return AGRL_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// Ranked lists: each query's first k gallery items and their distances, from ascending key lists laid out
+// [part][query][depth] (_partial, agrl_distance_topk_dev or the shards' lists after an all-gather).  One CTA per query:
+//   1. every list into shared memory, without the query's junk items (same pid and camera) when asked: a stable
+//      compaction, so each list stays ascending;
+//   2. the rank merge of rank_mars_merge_kernel (merged_position) places the keys that land among the first k;
+//   3. each key -> (global gallery index, distance), the tail padded with (-1, +inf).
+// Dropping junk list by list is exact when every list holds its shard's first k + J keys, J at least the number of junk
+// items any query has in that shard (agrl_rank_junk_depth_dev): an item among the first k kept ones of the whole gallery
+// is among the first k kept ones of its own shard.
+// ------------------------------------------------------------------------------------------------
+struct ListsArgs {
+    const uint64_t *keys;
+    int             parts, num_q, depth, k;
+    int64_t         num_g;
+    const int32_t  *q_pid, *q_cam, *g_pid, *g_cam;   // q_pid == nullptr: no junk exclusion
+    int64_t        *index_out;
+    float          *dist_out;
+    int64_t         ld_out;
+};
+
+__global__ void __launch_bounds__(kRankThreads)
+rank_lists_kernel(ListsArgs a) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int D = a.depth, K = a.k;
+    uint64_t *lists = reinterpret_cast<uint64_t *>(smem_raw);                 // parts * D
+    uint64_t *head = lists + static_cast<size_t>(a.parts) * D;                // K: the merged head
+    const int q = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const bool drop_junk = a.q_pid != nullptr;
+    const int pid = drop_junk ? a.q_pid[q] : 0, cam = drop_junk ? a.q_cam[q] : 0;
+    for (int p = warp; p < a.parts; p += kRankThreads / 32) {
+        const uint64_t *src = a.keys + (static_cast<size_t>(p) * a.num_q + q) * D;
+        uint64_t *dst = lists + static_cast<size_t>(p) * D;
+        int n = 0;
+        for (int base = 0; base < D; base += 32) {
+            const int j = base + lane;
+            const uint64_t key = j < D ? src[j] : kKeyMax;
+            bool keep = key != kKeyMax;
+            if (keep && drop_junk) {
+                const uint32_t g = static_cast<uint32_t>(key);
+                keep = !(g < a.num_g && a.g_pid[g] == pid && a.g_cam[g] == cam);
+            }
+            const uint32_t m = __ballot_sync(0xffffffffu, keep);
+            if (keep) dst[n + __popc(m & ((1u << lane) - 1u))] = key;
+            n += __popc(m);
+        }
+        for (int j = n + lane; j < D; j += 32) dst[j] = kKeyMax;
+    }
+    for (int i = tid; i < K; i += kRankThreads) head[i] = kKeyMax;
+    __syncthreads();
+    for (int i = tid; i < a.parts * K; i += kRankThreads) {
+        const int p = i / K, pos = i - p * K;
+        const uint64_t key = lists[static_cast<size_t>(p) * D + pos];
+        if (key == kKeyMax) continue;
+        const int rank = merged_position(lists, a.parts, D, K, p, pos, key);
+        if (rank < K) head[rank] = key;
+    }
+    __syncthreads();
+    int64_t *idx = a.index_out + static_cast<size_t>(q) * a.ld_out;
+    float *dst = a.dist_out + static_cast<size_t>(q) * a.ld_out;
+    for (int i = tid; i < K; i += kRankThreads) {
+        const uint64_t key = head[i];
+        const bool real = key != kKeyMax;
+        idx[i] = real ? static_cast<int64_t>(static_cast<uint32_t>(key)) : -1;
+        dst[i] = real ? mono_key_value(static_cast<uint32_t>(key >> 32)) : __uint_as_float(0x7F800000u);
+    }
+}
+
 }  // namespace agrl
 
 extern "C" size_t agrl_rank_mars_classify_workspace_bytes(int64_t num_q, int64_t num_g) {
@@ -1332,23 +1438,72 @@ extern "C" int agrl_rank_mars_classify_dev(const uint64_t *keys, const int64_t *
     ClassifyWorkspace w = carve_classify(ws, num_q, num_g);
     if (!ws || ws_bytes < w.bytes) return AGRL_E_WORKSPACE;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    rc = narrow_labels(q_pids, g_pids, q_camids, g_camids, num_q, num_g, w.q_pid, w.g_pid, w.q_cam, w.g_cam,
-                       status, st);
+    rc = build_label_tables(w, q_pids, g_pids, q_camids, g_camids, num_q, num_g, status, st);
     if (rc) return rc;
-    AGRL_CUDA_TRY(cudaMemsetAsync(w.tab_p, 0xFF, sizeof(int32_t) * 2 * w.slots, st));       // both tables: empty (-1)
-    AGRL_CUDA_TRY(cudaMemsetAsync(w.cnt_p, 0, sizeof(int32_t) * 2 * w.slots, st));
-    const int nq = static_cast<int>(num_q);
-    classify_insert_kernel<<<(nq + 255) / 256, 256, 0, st>>>(w, nq);
-    AGRL_LAUNCH_CHECK(st, "classify_insert");
-    if (num_g > 0) {
-        int cb = static_cast<int>((num_g + 255) / 256);
-        if (cb > 8 * kNumSMs) cb = 8 * kNumSMs;
-        classify_count_kernel<<<cb, 256, 0, st>>>(w, num_g);
-        AGRL_LAUNCH_CHECK(st, "classify_count");
-    }
     const int64_t total = num_q * max_rank;
     classify_keys_kernel<<<static_cast<unsigned>((total + 255) / 256), 256, 0, st>>>(
-        w, keys, nq, static_cast<int>(max_rank), num_g, static_cast<uint32_t>(index_offset), cls, ngood);
+        w, keys, static_cast<int>(num_q), static_cast<int>(max_rank), num_g, static_cast<uint32_t>(index_offset), cls,
+        ngood);
     AGRL_LAUNCH_CHECK(st, "classify_keys");
+    return AGRL_OK;
+}
+
+// ---- ranked lists ------------------------------------------------------------------------------------
+extern "C" int agrl_rank_junk_depth_dev(const int64_t *q_pids, const int64_t *g_pids, const int64_t *q_camids,
+                                        const int64_t *g_camids, int64_t num_q, int64_t num_g, int32_t *junk_depth,
+                                        uint32_t *status, void *ws, size_t ws_bytes, void *stream) {
+    if (!q_pids || !q_camids || !junk_depth || !status || (num_g > 0 && (!g_pids || !g_camids))) return AGRL_E_INVALID;
+    if (num_q < 1 || num_g < 0) return AGRL_E_INVALID;
+    if (num_q > (1 << 28) || num_g > INT32_MAX) return AGRL_E_UNSUPPORTED;
+    int rc = agrl_device_ok();
+    if (rc) return rc;
+    ClassifyWorkspace w = carve_classify(ws, num_q, num_g);
+    if (!ws || ws_bytes < w.bytes) return AGRL_E_WORKSPACE;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    AGRL_CUDA_TRY(cudaMemsetAsync(status, 0, sizeof(uint32_t), st));
+    AGRL_CUDA_TRY(cudaMemsetAsync(junk_depth, 0, sizeof(int32_t), st));
+    rc = build_label_tables(w, q_pids, g_pids, q_camids, g_camids, num_q, num_g, status, st);
+    if (rc) return rc;
+    const int nq = static_cast<int>(num_q);
+    rank_junk_depth_kernel<<<(nq + 255) / 256, 256, 0, st>>>(w, nq, junk_depth);
+    AGRL_LAUNCH_CHECK(st, "rank_junk_depth");
+    return AGRL_OK;
+}
+
+extern "C" int agrl_rank_lists_dev(const uint64_t *keys, int64_t parts, int64_t num_q, int64_t depth, int64_t k,
+                                   const int64_t *q_pids, const int64_t *g_pids, const int64_t *q_camids,
+                                   const int64_t *g_camids, int64_t num_g, int exclude_junk,
+                                   int64_t *index_out, float *dist_out, int64_t ld_out, uint32_t *status,
+                                   void *ws, size_t ws_bytes, void *stream) {
+    if (!keys || !index_out || !dist_out || !status) return AGRL_E_INVALID;
+    if (parts < 1 || num_q < 1 || k < 1 || depth < k || ld_out < k) return AGRL_E_INVALID;
+    if (exclude_junk && (!q_pids || !g_pids || !q_camids || !g_camids || num_g < 1)) return AGRL_E_INVALID;
+    if (depth > 8192 || parts * depth > 16384 || num_q > INT32_MAX / 2) return AGRL_E_UNSUPPORTED;
+    if (exclude_junk && num_g > 0xFFFFFFFFll) return AGRL_E_UNSUPPORTED;
+    int rc = agrl_device_ok();
+    if (rc) return rc;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    AGRL_CUDA_TRY(cudaMemsetAsync(status, 0, sizeof(uint32_t), st));
+    ListsArgs a;
+    memset(&a, 0, sizeof(a));
+    if (exclude_junk) {
+        ClassifyWorkspace w = carve_classify(ws, num_q, num_g);
+        if (!ws || ws_bytes < w.bytes) return AGRL_E_WORKSPACE;
+        rc = narrow_labels(q_pids, g_pids, q_camids, g_camids, num_q, num_g, w.q_pid, w.g_pid, w.q_cam, w.g_cam,
+                           status, st);
+        if (rc) return rc;
+        a.q_pid = w.q_pid; a.q_cam = w.q_cam; a.g_pid = w.g_pid; a.g_cam = w.g_cam;
+        a.num_g = num_g;
+    }
+    a.keys = keys;
+    a.parts = static_cast<int>(parts); a.num_q = static_cast<int>(num_q);
+    a.depth = static_cast<int>(depth); a.k = static_cast<int>(k);
+    a.index_out = index_out; a.dist_out = dist_out; a.ld_out = ld_out;
+    const size_t smem = static_cast<size_t>(parts * depth + k) * 8;
+    AGRL_CUDA_TRY(cudaFuncSetAttribute(rank_lists_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       static_cast<int>(smem)));
+    AGRL_LAUNCH_BEGIN(st);
+    rank_lists_kernel<<<static_cast<unsigned>(num_q), kRankThreads, smem, st>>>(a);
+    AGRL_LAUNCH_CHECK(st, "rank_lists");
     return AGRL_OK;
 }

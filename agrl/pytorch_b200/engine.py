@@ -89,10 +89,14 @@ def _report(say, cmc, mAP, ranks):
 
 def test(model, queryloader, galleryloader, pool='avg', use_gpu=True, ranks=(1, 5, 10, 20), return_distmat=False,
          test_sample='evenly', dist_metric='euclidean', re_rank=False, max_rank=50, args=None, verbose=True,
-         group=None, sharded_ops=None):
+         group=None, sharded_ops=None, return_ranked=None):
     """Drop-in for the reference's test(): returns ``(cmc[0], mAP)``, or the (num_query, num_gallery) distance
-    matrix as a numpy array with ``return_distmat``.  Raises what the reference raises: ``ZeroDivisionError`` for a
-    query without a cross-camera match (rank.py:203), ``ValueError`` for an unknown metric (distance.py:50-54)."""
+    matrix as a numpy array with ``return_distmat``.  ``return_ranked=k`` (without ``return_distmat``) returns
+    ``(cmc[0], mAP, indices, distances)`` instead, the first k gallery items of every query and their distances as
+    (num_query, k) CUDA tensors (metrics.rank_lists on the ranked matrix; with several processes
+    sharded.rank_lists_sharded, global gallery indices, the same on every rank).  Raises what the reference raises:
+    ``ZeroDivisionError`` for a query without a cross-camera match (rank.py:203), ``ValueError`` for an unknown metric
+    (distance.py:50-54)."""
     if not use_gpu:
         raise RuntimeError('agrl.pytorch_b200 has no CPU path: test() needs use_gpu=True and a B200')
     if args is not None:
@@ -124,6 +128,10 @@ def test(model, queryloader, galleryloader, pool='avg', use_gpu=True, ranks=(1, 
         cmc, mAP = sharded.evaluate_mars_sharded(qf, gf, q_pids, g_pids, q_camids, g_camids, metric=dist_metric,
                                                  max_rank=max_rank, group=group, ops=sharded_ops)
         _report(say, cmc, mAP, ranks)
+        if return_ranked:
+            indices, distances = sharded.rank_lists_sharded(qf, gf, return_ranked, metric=dist_metric, group=group,
+                                                            ops=sharded_ops)
+            return cmc[0], mAP, indices, distances
         return cmc[0], mAP
     distmat = metrics.compute_distance_matrix(qf, gf, dist_metric)
 
@@ -141,4 +149,6 @@ def test(model, queryloader, galleryloader, pool='avg', use_gpu=True, ranks=(1, 
 
     if return_distmat:
         return distmat.cpu().numpy() if isinstance(distmat, torch.Tensor) else distmat
+    if return_ranked:
+        return (cmc[0], mAP) + metrics.rank_lists(distmat, return_ranked)
     return cmc[0], mAP

@@ -145,6 +145,74 @@ class CudaOps(object):
         _raise_status(status)
         return host[:max_rank].numpy().copy(), np.float64(host[max_rank])
 
+    # ---- ranked lists (agrl_rank_lists_dev) ---------------------------------------------------------------------------
+    def keys(self, d, depth, offset):
+        """Each query's first ``depth`` keys of the distance block ``d`` (agrl_rank_mars_partial_dev)."""
+        qp, lab = _unlabelled(d.shape[0], d.shape[1], d.device)
+        return self.partial(d, qp, lab, qp, lab, depth, offset)[0]
+
+    def topk_keys(self, qop, gop, depth, offset, fused=True):
+        """``keys`` of the distance block of two PreparedOperand without materialising it: distance -> top-k fused into
+        the GEMM epilogue (depth <= 256); when a query's candidate list overflows, or with ``fused=False``, distance blocks
+        of at most 2 GiB + ``keys``.  The keys are the same either way."""
+        from .metrics.distance import _METRICS, distance_prepared
+        assert (qop.metric, qop.split, qop.dim, qop.device) == (gop.metric, gop.split, gop.dim, gop.device)
+        dev, nq, ng = qop.device, qop.rows, gop.rows
+        keys = torch.empty(nq, depth, dtype=torch.int64, device=dev)
+        if fused:
+            status = torch.zeros(1, dtype=torch.int32, device=dev)
+            wsb = self.lib.agrl_distance_topk_workspace_bytes(nq)
+            ws = self._workspace(dev, wsb)
+            with torch.cuda.device(dev):
+                _lib.check(self.lib.agrl_distance_topk_dev(
+                    qop.buf.data_ptr(), nq, gop.buf.data_ptr(), ng, qop.dim, _METRICS[qop.metric], qop.split, depth, offset,
+                    keys.data_ptr(), status.data_ptr(), ws.data_ptr(), wsb, torch.cuda.current_stream(dev).cuda_stream))
+            if not int(status.cpu()) & _lib.ST_TOPK_OVERFLOW:
+                return keys
+        rows = max(1, min(nq, (1 << 31) // max(4 * ng, 1)))
+        dbuf = torch.empty(rows, ng, device=dev)
+        for q0 in range(0, nq, rows):
+            q1 = min(nq, q0 + rows)
+            keys[q0:q1] = self.keys(distance_prepared(qop.rows_view(q0, q1), gop, out=dbuf[:q1 - q0]), depth, offset)
+        return keys
+
+    def junk_depth(self, q_pids, g_pids, q_camids, g_camids):
+        """(J, status) as int32 tensors of one element: the most gallery items of this shard sharing a query's pid and
+        camera, over the queries (agrl_rank_junk_depth_dev)."""
+        dev = q_pids.device
+        nq, ng = q_pids.numel(), g_pids.numel()
+        out = torch.zeros(2, dtype=torch.int32, device=dev)                   # [J, status]
+        wsb = self.lib.agrl_rank_mars_classify_workspace_bytes(nq, ng)
+        ws = self._workspace(dev, wsb)
+        with torch.cuda.device(dev):
+            _lib.check(self.lib.agrl_rank_junk_depth_dev(
+                q_pids.data_ptr(), g_pids.data_ptr(), q_camids.data_ptr(), g_camids.data_ptr(), nq, ng, out.data_ptr(),
+                out.data_ptr() + 4, ws.data_ptr(), wsb, torch.cuda.current_stream(dev).cuda_stream))
+        return out[0:1], out[1:2]
+
+    def lists(self, keys_all, k, q_pids=None, g_pids=None, q_camids=None, g_camids=None, exclude_junk=False):
+        """(indices int64, distances fp32), (num_q, k) each, from the [part][query][depth] key lists (agrl_rank_lists_dev);
+        with ``exclude_junk`` the gallery labels are indexed by global gallery index."""
+        dev = keys_all.device
+        keys_all = keys_all.contiguous()
+        parts, nq, depth = keys_all.shape
+        index = torch.empty(nq, k, dtype=torch.int64, device=dev)
+        dist_ = torch.empty(nq, k, dtype=torch.float32, device=dev)
+        status = torch.zeros(1, dtype=torch.int32, device=dev)
+        ng = g_pids.numel() if exclude_junk else 0
+        wsb = self.lib.agrl_rank_mars_classify_workspace_bytes(nq, ng) if exclude_junk else 0
+        ws = self._workspace(dev, max(wsb, 1))
+        lab = [x.data_ptr() if exclude_junk else None for x in (q_pids, g_pids, q_camids, g_camids)]
+        with torch.cuda.device(dev):
+            _lib.check(self.lib.agrl_rank_lists_dev(
+                keys_all.data_ptr(), parts, nq, depth, k, lab[0], lab[1], lab[2], lab[3], ng, int(bool(exclude_junk)),
+                index.data_ptr(), dist_.data_ptr(), k, status.data_ptr(), ws.data_ptr(), wsb,
+                torch.cuda.current_stream(dev).cuda_stream))
+            st = int(status.cpu())
+        from .metrics.rank import _raise_status
+        _raise_status(st)
+        return index, dist_
+
 
     # ---- market1501 metric -------------------------------------------------------------------------
     def market_count(self, q_pids, g_pids, q_camids, g_camids):
@@ -274,6 +342,94 @@ def _as_dev_i64(x, dev):
     if isinstance(x, torch.Tensor):
         return x.to(device=dev, dtype=torch.int64).contiguous()
     return torch.as_tensor(np.ascontiguousarray(np.asarray(x), dtype=np.int64)).to(dev)
+
+
+def _unlabelled(nq, ng, dev):
+    """query / gallery labels for a ranking that needs none: no gallery item shares a query's pid"""
+    return torch.zeros(nq, dtype=torch.int64, device=dev), torch.ones(ng, dtype=torch.int64, device=dev)
+
+
+MAX_LIST_DEPTH = 8192            # k + J per query and shard (agrl_rank_mars_partial_dev / agrl_rank_lists_dev)
+FUSED_MAX_DEPTH = 256            # deepest list the fused distance -> top-k keeps (agrl_distance_topk_dev)
+
+
+def list_depth(k, ops, labels, exclude_junk, group=None, world=1):
+    """Keys every shard must keep per query for lists of length k: k, plus with ``exclude_junk`` the most junk items
+    (same pid and camera) any query has in one shard, all-reduced (MAX) over the ranks with their status words.  Raises
+    ValueError beyond MAX_LIST_DEPTH."""
+    k = int(k)
+    if k < 1:
+        raise ValueError('k must be at least 1, got {}'.format(k))
+    J = 0
+    if exclude_junk:
+        if labels is None:
+            raise ValueError('exclude_junk needs q_pids, g_pids, q_camids and g_camids')
+        j, status = ops.junk_depth(*labels)
+        if world > 1:                     # J and the status bits in one MAX reduction
+            shifts = torch.arange(16, device=status.device, dtype=torch.int32)
+            word = torch.cat([j.to(torch.int32), (status.to(torch.int32) >> shifts) & 1])
+            dist.all_reduce(word, op=dist.ReduceOp.MAX, group=group)
+            j, status = word[0:1], (word[1:] << shifts).sum().view(1)
+        from .metrics.rank import _raise_status
+        host = torch.cat([j, status.to(j.dtype)]).cpu()
+        _raise_status(int(host[1]))
+        J = int(host[0])
+    if k + J > MAX_LIST_DEPTH:
+        raise ValueError('ranked lists reach {} keys per query (k = {} plus {} junk items of one identity and camera); '
+                         'at most {} are supported'.format(k + J, k, J, MAX_LIST_DEPTH))
+    return k + J
+
+
+def rank_lists_sharded(qf, gf_local, k, q_pids=None, g_pids_local=None, q_camids=None, g_camids_local=None,
+                       metric='euclidean', exclude_junk=False, group=None, broadcast_queries=True, ops=None,
+                       gallery_counts=None, fused=None, re_rank=False, k1=20, k2=6, lambda_value=0.3):
+    """Ranked lists of ``qf`` against the union of every rank's gallery shard: (indices int64, distances fp32) CUDA
+    tensors of shape (num_q, k), the same on every rank, bit-identical to ``metrics.rank_lists`` on the whole distance
+    matrix -- row i is np.argsort(d[i], kind='stable')[:k] with GLOBAL gallery indices, padded with (-1, +inf).
+    Arguments as in evaluate_mars_sharded; labels are only needed for ``exclude_junk`` (skip the gallery items with the
+    query's pid and camera; pid -1 distractors stay).  ``re_rank`` ranks the block of re_ranking_sharded instead.
+    Exchanges: the query broadcast and shard layout of evaluate_mars_sharded, one all-reduce(max) of the junk depth J with
+    ``exclude_junk`` (plus one all-gather of the gallery labels), and one all-gather of num_q x (k + J) keys.
+    Raises ValueError when k + J exceeds MAX_LIST_DEPTH."""
+    if metric not in ('euclidean', 'cosine'):
+        raise ValueError('Unknown distance metric: {}. Please choose either "euclidean" or "cosine"'.format(metric))
+    world = dist.get_world_size(group) if dist.is_initialized() else 1
+    dev = qf.device
+    ops = ops or CudaOps()
+    qf = qf.contiguous()
+    labels = None
+    if q_pids is not None:
+        labels = [_as_dev_i64(x, dev) for x in (q_pids, g_pids_local, q_camids, g_camids_local)]
+    if world > 1 and broadcast_queries:
+        _broadcast_queries(qf, labels[0] if labels else None, labels[2] if labels else None, group)
+    counts, rank = _shard_layout(gf_local.shape[0], dev, world, group, gallery_counts)
+    offset, n_own, nq = sum(counts[:rank]), counts[rank], qf.shape[0]
+    depth = list_depth(k, ops, labels, exclude_junk, group, world)
+    if fused is None:
+        fused = n_own >= FUSED_MIN_GALLERY and hasattr(ops, 'topk_keys') and depth <= FUSED_MAX_DEPTH
+    if re_rank:
+        d = re_ranking_sharded(qf, gf_local, metric, k1, k2, lambda_value, group=group, broadcast_queries=False, ops=ops,
+                               gallery_counts=counts)
+    if n_own == 0:                        # no candidates: an all-empty list
+        keys = torch.full((nq, depth), -1, dtype=torch.int64, device=dev)
+    elif re_rank:
+        keys = ops.keys(d, depth, offset)
+    elif fused:
+        from .metrics.distance import PreparedOperand
+        keys = ops.topk_keys(PreparedOperand(qf, metric, ops.split), PreparedOperand(gf_local, metric, ops.split), depth,
+                             offset, fused=depth <= FUSED_MAX_DEPTH)
+    else:
+        keys = ops.keys(ops.distance(qf, gf_local, metric), depth, offset)
+    if world > 1:
+        keys_all = torch.empty((world * nq, depth), dtype=keys.dtype, device=dev)
+        dist.all_gather_into_tensor(keys_all, keys.contiguous(), group=group)
+        keys_all = keys_all.view(world, nq, depth)
+        if exclude_junk:                  # the junk test needs the labels of every listed item
+            labels[1] = _gather_shard_rows(labels[1], 0, counts, rank, group)
+            labels[3] = _gather_shard_rows(labels[3], 0, counts, rank, group)
+    else:
+        keys_all = keys.unsqueeze(0)
+    return ops.lists(keys_all, k, *(labels or [None] * 4), exclude_junk=exclude_junk)
 
 
 FUSED_MIN_GALLERY = 32768        # gallery rows per shard from which the fused distance -> top-k is the default

@@ -269,6 +269,37 @@ AGRL_API int agrl_rank_mars_classify_dev(const uint64_t *keys_dev,
                                 uint8_t *cls_dev, int32_t *ngood_dev, uint32_t *status_dev,
                                 void *workspace_dev, size_t workspace_bytes, void *stream);
 
+/* Ranked lists: each query's first k gallery items, in the order of section (3) -- row i's list is
+ * numpy.argsort(d[i], kind='stable')[:k] of the (global) distance matrix -- with their distances.
+ *   keys_dev    (parts, num_q, depth) ascending key lists as _partial, agrl_distance_topk_dev or an all-gather of the
+ *               shards' lists lay them out (all-ones = empty slot).  parts == 1 is the whole gallery.
+ *   index_out   out (num_q, k) int64 global gallery indices, row stride ld_out
+ *   dist_out    out (num_q, k) fp32, row stride ld_out: the bits of the ranked distance, decoded from the key (-0 comes
+ *               back as +0, every NaN as the NaN 0x7FFFFFFF)
+ *   When fewer than k items qualify (num_g < k, or junk exclusion leaves fewer) the tail is index -1, distance +inf.
+ *   exclude_junk: skip the gallery items with the query's pid AND camera (rank_cy.pyx:197, rank.py:166-169 without the
+ *               pid == -1 distractors, which stay in the list).  Needs the labels (int64, fitting int32, else
+ *               AGRL_ST_LABEL_RANGE in *status_dev) with g_*_dev indexed by GLOBAL gallery index, num_g of them, and a
+ *               workspace of agrl_rank_mars_classify_workspace_bytes(num_q, num_g) bytes; without it the labels, num_g
+ *               and the workspace may be NULL / 0.  The result is then the stable argsort with those columns deleted, cut
+ *               to k, provided every shard's list holds its first depth = k + J keys, with J from
+ *               agrl_rank_junk_depth_dev on that shard's labels, all-reduced (MAX) over the shards.
+ *   status_dev  out, 1 uint32: zeroed, then AGRL_ST_LABEL_RANGE.
+ * Limits: 1 <= k <= depth <= 8192, parts * depth <= 16384 (AGRL_E_UNSUPPORTED beyond). */
+AGRL_API int agrl_rank_lists_dev(const uint64_t *keys_dev, int64_t parts, int64_t num_q, int64_t depth, int64_t k,
+                                 const int64_t *q_pids_dev, const int64_t *g_pids_dev,
+                                 const int64_t *q_camids_dev, const int64_t *g_camids_dev, int64_t num_g,
+                                 int exclude_junk, int64_t *index_out_dev, float *dist_out_dev, int64_t ld_out,
+                                 uint32_t *status_dev, void *workspace_dev, size_t workspace_bytes, void *stream);
+/* Junk depth of one gallery shard: *junk_depth_dev = the most gallery items of this shard sharing a query's pid and
+ * camera, over the queries (0 for an empty shard), in O(num_q + num_g) with the tables of agrl_rank_mars_classify_dev.
+ * Workspace: agrl_rank_mars_classify_workspace_bytes(num_q, num_g).  status_dev out: zeroed, then
+ * AGRL_ST_LABEL_RANGE. */
+AGRL_API int agrl_rank_junk_depth_dev(const int64_t *q_pids_dev, const int64_t *g_pids_dev,
+                                      const int64_t *q_camids_dev, const int64_t *g_camids_dev,
+                                      int64_t num_q, int64_t num_g, int32_t *junk_depth_dev, uint32_t *status_dev,
+                                      void *workspace_dev, size_t workspace_bytes, void *stream);
+
 AGRL_API int agrl_distance_host(const float *q_host, const float *g_host, float *out_host,
                        int64_t num_q, int64_t num_g, int64_t dim, int metric, int split);
 
