@@ -97,6 +97,8 @@ _SIGNATURES = {
     'agrl_rerank_shard_finish_dev': (c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_i64, c_i64, c_i64, c_i64,
                                              ctypes.c_double, c_vp, c_i64, c_vp, c_sz, c_vp]),
     'agrl_clip_pool_dev': (c_int, [c_vp, c_i64, c_i64, c_i64, c_i64, c_int, c_vp, c_i64, c_vp]),
+    'agrl_qe_mix_dev': (c_int, [c_vp, c_vp, c_i64, c_i64, c_i64, c_vp, c_i64, c_i64, c_i64, ctypes.c_float, c_vp, c_i64,
+                                c_vp]),
     'agrl_head_prepared_bytes': (c_sz, [ctypes.POINTER(HeadParams)]),
     'agrl_head_prepare_dev': (c_int, [ctypes.POINTER(HeadParams), c_vp, c_sz, c_vp]),
     'agrl_head_workspace_bytes': (c_sz, [ctypes.POINTER(HeadParams), c_i64, c_i32]),

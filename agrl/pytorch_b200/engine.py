@@ -89,20 +89,26 @@ def _report(say, cmc, mAP, ranks):
 
 def test(model, queryloader, galleryloader, pool='avg', use_gpu=True, ranks=(1, 5, 10, 20), return_distmat=False,
          test_sample='evenly', dist_metric='euclidean', re_rank=False, max_rank=50, args=None, verbose=True,
-         group=None, sharded_ops=None, return_ranked=None):
+         group=None, sharded_ops=None, return_ranked=None, aqe=False, qe_k=5, qe_times=1, qe_alpha=3.0):
     """Drop-in for the reference's test(): returns ``(cmc[0], mAP)``, or the (num_query, num_gallery) distance
     matrix as a numpy array with ``return_distmat``.  ``return_ranked=k`` (without ``return_distmat``) returns
     ``(cmc[0], mAP, indices, distances)`` instead, the first k gallery items of every query and their distances as
     (num_query, k) CUDA tensors (metrics.rank_lists on the ranked matrix; with several processes
     sharded.rank_lists_sharded, global gallery indices, the same on every rank).  Raises what the reference raises:
     ``ZeroDivisionError`` for a query without a cross-camera match (rank.py:203), ``ValueError`` for an unknown metric
-    (distance.py:50-54)."""
+    (distance.py:50-54).  ``aqe`` applies alpha query expansion (metrics.query_expansion with ``qe_k``, ``qe_times`` and
+    ``qe_alpha``; with several processes sharded.query_expansion_sharded) to the extracted features, as FastReID's
+    TEST.AQE does before its distance matrix: every later step, re-ranking included, sees the expanded features."""
     if not use_gpu:
         raise RuntimeError('agrl.pytorch_b200 has no CPU path: test() needs use_gpu=True and a B200')
     if args is not None:
         test_sample = getattr(args, 'test_sample', test_sample)
         dist_metric = getattr(args, 'dist_metric', dist_metric)
         re_rank = getattr(args, 're_rank', re_rank)
+        aqe = getattr(args, 'aqe', aqe)
+        qe_k = getattr(args, 'qe_k', qe_k)
+        qe_times = getattr(args, 'qe_times', qe_times)
+        qe_alpha = getattr(args, 'qe_alpha', qe_alpha)
     world = torch.distributed.get_world_size(group) if torch.distributed.is_initialized() else 1
     if world > 1 and torch.distributed.get_rank(group) != 0:
         verbose = False                                   # one copy of the progress lines
@@ -117,6 +123,13 @@ def test(model, queryloader, galleryloader, pool='avg', use_gpu=True, ranks=(1, 
         gf, g_pids, g_camids, tg, ng, bg = extract_features(model, galleryloader, pool, test_sample)
         say("Extracted features for gallery set, obtained {}-by-{} matrix".format(gf.size(0), gf.size(1)))
     say("==> BatchTime(s)/BatchSize(img): {:.3f}/{}".format((tq + tg) / max(nq + ng, 1), max(bq, bg)))
+
+    if aqe:
+        say('Applying alpha query expansion (qe_k={}, qe_times={}, alpha={}) ...'.format(qe_k, qe_times, qe_alpha))
+        if world > 1:
+            qf, gf = sharded.query_expansion_sharded(qf, gf, qe_k, qe_times, qe_alpha, group=group, ops=sharded_ops)
+        else:
+            qf, gf = metrics.query_expansion(qf, gf, qe_k, qe_times, qe_alpha)
 
     say('Computing distance matrix with metric={} ...'.format(dist_metric))
     if world > 1:

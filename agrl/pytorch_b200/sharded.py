@@ -17,6 +17,7 @@ tables (rank lists, k-reciprocal rows) later produces its (num_q x num_g_r) bloc
 ``ops`` lets the tests drive the same plumbing with CPU stand-ins under gloo; the product default is
 the CUDA implementation and there is no fallback.
 """
+import math
 from types import SimpleNamespace
 
 import numpy as np
@@ -212,6 +213,37 @@ class CudaOps(object):
         from .metrics.rank import _raise_status
         _raise_status(st)
         return index, dist_
+
+    # ---- alpha query expansion (agrl_qe_mix_dev) ----------------------------------------------------------------------
+    def qe_lists(self, x, ranges, k, fused=None):
+        """(indices int64, cosine distances fp32), (rows, k) each: the ranked lists of the rows x[r0:r1] of every
+        (r0, r1) in ``ranges``, in order, against all rows of x (each row's list includes itself).  x is split into
+        cosine operand planes once; a range that is not the whole of x is a rows_view of those planes.  The distance ->
+        top-k is fused into the GEMM epilogue from FUSED_MIN_GALLERY rows of x on (``fused`` overrides); the lists are
+        the same either way."""
+        from .metrics.distance import PreparedOperand
+        n, dev = x.shape[0], x.device
+        if fused is None:
+            fused = n >= FUSED_MIN_GALLERY
+        op = PreparedOperand(x, 'cosine', self.split)
+        keys = [self.topk_keys(op if (r0, r1) == (0, n) else op.rows_view(r0, r1), op, k, 0,
+                               fused=fused and k <= FUSED_MAX_DEPTH) for r0, r1 in ranges if r1 > r0]
+        if not keys:
+            return torch.empty(0, k, dtype=torch.int64, device=dev), torch.empty(0, k, dtype=torch.float32, device=dev)
+        return self.lists(torch.cat(keys).unsqueeze(0), k)
+
+    def qe_mix(self, idx, d, x, alpha):
+        """(rows, dim) fp32: row r = sum_j powf(1 - d[r, j], alpha) * x[idx[r, j]] / k, in list order
+        (agrl_qe_mix_dev)."""
+        assert idx.stride() == d.stride() and x.dtype == torch.float32 and x.stride(1) == 1
+        rows, k = idx.shape
+        dim = x.shape[1]
+        out = torch.empty(rows, dim, dtype=torch.float32, device=x.device)
+        with torch.cuda.device(x.device):
+            _lib.check(self.lib.agrl_qe_mix_dev(
+                idx.data_ptr(), d.data_ptr(), idx.stride(0), rows, k, x.data_ptr(), x.stride(0), x.shape[0], dim,
+                float(alpha), out.data_ptr(), dim, torch.cuda.current_stream(x.device).cuda_stream))
+        return out
 
 
     # ---- market1501 metric -------------------------------------------------------------------------
@@ -433,6 +465,47 @@ def rank_lists_sharded(qf, gf_local, k, q_pids=None, g_pids_local=None, q_camids
 
 
 FUSED_MIN_GALLERY = 32768        # gallery rows per shard from which the fused distance -> top-k is the default
+
+
+def check_qe_args(qe_k, qe_times, alpha, n):
+    """ValueError for alpha query expansion parameters it cannot honour on a joint set of n rows."""
+    if qe_k < 1 or qe_k > MAX_LIST_DEPTH:
+        raise ValueError('qe_k must be between 1 and {}, got {}'.format(MAX_LIST_DEPTH, qe_k))
+    if qe_k > n:
+        raise ValueError('qe_k = {} exceeds the {} query and gallery rows'.format(qe_k, n))
+    if qe_times < 1:
+        raise ValueError('qe_times must be at least 1, got {}'.format(qe_times))
+    if not math.isfinite(alpha):
+        raise ValueError('alpha must be finite, got {}'.format(alpha))
+
+
+def query_expansion_sharded(qf, gf_local, qe_k=5, qe_times=1, alpha=3.0, group=None, broadcast_queries=True, ops=None,
+                            gallery_counts=None):
+    """Alpha query expansion (metrics.query_expansion) of ``qf`` and the union of every rank's gallery shard.
+
+    Returns (qf', gf_local'): the expanded queries (the same on every rank) and this rank's expanded gallery rows,
+    bit-identical to the matching rows of metrics.query_expansion on the whole sets.  Arguments as in
+    evaluate_mars_sharded; shards may be empty.  Each iteration all-gathers the gallery rows; each rank then ranks its
+    query and gallery rows against the whole joint set and mixes them.  Raises ValueError as check_qe_args."""
+    world = dist.get_world_size(group) if dist.is_initialized() else 1
+    ops = ops or CudaOps()
+    assert qf.dim() == 2 and gf_local.dim() == 2 and qf.size(1) == gf_local.size(1)
+    dev = qf.device
+    qf = qf.detach().to(torch.float32).contiguous()
+    gf = gf_local.detach().to(device=dev, dtype=torch.float32).contiguous()
+    if world > 1 and broadcast_queries:
+        qf = qf.clone()                   # the broadcast writes into it
+        _broadcast_queries(qf, None, None, group)
+    counts, rank = _shard_layout(gf.shape[0], dev, world, group, gallery_counts)
+    nq, offset, n_own = qf.shape[0], sum(counts[:rank]), counts[rank]
+    check_qe_args(qe_k, qe_times, alpha, nq + sum(counts))
+    lo = nq + offset
+    for _ in range(qe_times):
+        x = torch.cat([qf, _gather_shard_rows(gf, 0, counts, rank, group)])
+        idx, d = ops.qe_lists(x, [(0, nq), (lo, lo + n_own)], qe_k)
+        mixed = ops.qe_mix(idx, d, x, alpha)
+        qf, gf = mixed[:nq], mixed[nq:]
+    return qf, gf
 
 
 def _shard_layout(n_local_rows, dev, world, group, gallery_counts):

@@ -460,6 +460,30 @@ AGRL_API int    agrl_rerank_shard_finish_dev(const int32_t *rank_all_dev, const 
                        int64_t g_off, int64_t n_own, int64_t k1, int64_t k2, double lambda_value,
                        float *out_dev, int64_t ld_out, void *workspace_dev, size_t workspace_bytes, void *stream);
 
+/* ---- alpha query expansion (FastReID fastreid/evaluation/query_expansion.py `aqe`, TEST.AQE) ---------------------
+ * One iteration over the joint set X (queries, then the gallery; N rows) replaces every row by the mean of its k nearest
+ * neighbours' rows, each weighted by its cosine similarity to the power alpha:
+ *   lists    idx, dist = the first k entries of each row of the cosine distance matrix d(X, X) in the order of section
+ *            (3) (each row includes itself; ties to the lower index): agrl_distance_topk_dev on cosine operands of X,
+ *            or agrl_rank_mars_partial_dev on distance blocks, then agrl_rank_lists_dev with parts == 1.
+ *   mix      out[r, :] = (sum_{j < k} powf(1 - dist[r, j], alpha) * feats[idx[r, j], :]) / k, with feats = X (the
+ *            un-normalised features).  The similarity 1 - dist and the weight are fp32 (C99 powf: a negative similarity
+ *            with a non-integer alpha gives NaN, as numpy.power does; alpha == 0 gives plain mean query expansion).
+ *            The sum runs over j in list order in fp32, so repeated calls are bit-identical.
+ * agrl_qe_mix_dev is the mix:
+ *   idx_dev     (rows, k) int64 rows of feats, row stride ld_list; an entry outside [0, num_feats) (e.g. the -1 padding
+ *               of a short list) contributes nothing
+ *   dist_dev    (rows, k) fp32 cosine distances of those entries, row stride ld_list
+ *   feats_dev   (num_feats, dim) fp32, row stride ld_feat;  out_dev (rows, dim) fp32, row stride ld_out, must not
+ *               overlap feats (AGRL_E_INVALID)
+ * Any dim and row strides; rows 16-byte aligned with dim, ld_feat and ld_out multiples of 4 take 16-byte loads.  No
+ * workspace, nothing allocated.  AGRL_E_INVALID for a negative size, k < 1, ld_list < k, ld_feat or ld_out < dim, or a
+ * non-finite alpha.  Repeat the two steps qe_times times (FastReID: QE_TIME = 1, QE_K = 5, ALPHA = 3.0) and split X' back
+ * into its query and gallery rows. */
+AGRL_API int agrl_qe_mix_dev(const int64_t *idx_dev, const float *dist_dev, int64_t ld_list, int64_t rows, int64_t k,
+                             const float *feats_dev, int64_t ld_feat, int64_t num_feats, int64_t dim, float alpha,
+                             float *out_dev, int64_t ld_out, void *stream);
+
 /* Clip pooling of the `dense` / `skipdense` test sampling (train_vidreid_xent_htri.py:461-476):
  * feats (tracklets * clips, dim) with the clips of a tracklet consecutive -> out (tracklets, dim),
  * torch.mean(features, 0) (AVG) or torch.max(features, 0) values (MAX) over the clip axis. */
