@@ -1,6 +1,6 @@
 """ctypes binding of libagrl_b200.so (the C ABI declared in include/agrl_b200.h).
 
-The library is the product; this module only loads it and declares argument types.  There is no
+The library is the product; this module only loads it, declares argument types and checks return codes.  There is no
 CPU fallback anywhere in agrl.pytorch_b200: if the shared library is missing, or no sm_100 device
 is present, every compute call raises.
 """
@@ -160,6 +160,13 @@ def check(code):
     if code == E_INVALID:
         raise ValueError(text)
     raise AgrlError(code, text)
+
+
+def call(device, fn, *args):
+    """``fn(*args, stream)`` with ``device`` current and ``stream`` its current CUDA stream, the return code checked."""
+    import torch
+    with torch.cuda.device(device):
+        check(fn(*args, torch.cuda.current_stream(device).cuda_stream))
 
 
 def require_device():

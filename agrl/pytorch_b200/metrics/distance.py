@@ -25,6 +25,16 @@ def _workspace(dev, nbytes):
     return ws
 
 
+def _check_metric(metric):
+    """The library's code of a metric name; ValueError as distance.py:50-54 for any other name."""
+    if metric not in _METRICS:
+        raise ValueError(
+            'Unknown distance metric: {}. '
+            'Please choose either "euclidean" or "cosine"'.format(metric)
+        )
+    return _METRICS[metric]
+
+
 def compute_distance_matrix(input1, input2, metric='euclidean', split=_lib.SPLIT_FP16X2):
     """A wrapper function for computing distance matrix (distance.py:11).
 
@@ -41,11 +51,7 @@ def compute_distance_matrix(input1, input2, metric='euclidean', split=_lib.SPLIT
     assert input1.dim() == 2, 'Expected 2-D tensor, but got {}-D'.format(input1.dim())
     assert input2.dim() == 2, 'Expected 2-D tensor, but got {}-D'.format(input2.dim())
     assert input1.size(1) == input2.size(1)
-    if metric not in _METRICS:
-        raise ValueError(
-            'Unknown distance metric: {}. '
-            'Please choose either "euclidean" or "cosine"'.format(metric)
-        )
+    code = _check_metric(metric)
     lib = _lib.require_device()
     m, n, d = input1.size(0), input2.size(0), input1.size(1)
     if input1.is_cuda != input2.is_cuda:
@@ -55,8 +61,7 @@ def compute_distance_matrix(input1, input2, metric='euclidean', split=_lib.SPLIT
         b = input2.detach().to(torch.float32).contiguous()
         out = torch.empty(m, n, dtype=torch.float32)
         if m and n:
-            _lib.check(lib.agrl_distance_host(a.data_ptr(), b.data_ptr(), out.data_ptr(), m, n, d,
-                                              _METRICS[metric], split))
+            _lib.check(lib.agrl_distance_host(a.data_ptr(), b.data_ptr(), out.data_ptr(), m, n, d, code, split))
         return out
     dev = input1.device
     a = input1.detach().to(torch.float32)
@@ -68,12 +73,10 @@ def compute_distance_matrix(input1, input2, metric='euclidean', split=_lib.SPLIT
     out = torch.empty(m, n, dtype=torch.float32, device=dev)
     if m == 0 or n == 0:
         return out
-    with torch.cuda.device(dev):
-        wsb = lib.agrl_distance_workspace_bytes(m, n, d, split)
-        ws = _workspace(dev, wsb)
-        _lib.check(lib.agrl_distance_dev(a.data_ptr(), a.stride(0), b.data_ptr(), b.stride(0),
-                                         out.data_ptr(), out.stride(0), m, n, d, _METRICS[metric], split,
-                                         ws.data_ptr(), wsb, torch.cuda.current_stream(dev).cuda_stream))
+    wsb = lib.agrl_distance_workspace_bytes(m, n, d, split)
+    ws = _workspace(dev, wsb)
+    _lib.call(dev, lib.agrl_distance_dev, a.data_ptr(), a.stride(0), b.data_ptr(), b.stride(0),
+              out.data_ptr(), out.stride(0), m, n, d, code, split, ws.data_ptr(), wsb)
     return out
 
 
@@ -85,9 +88,7 @@ class PreparedOperand(object):
 
     def __init__(self, x, metric='euclidean', split=_lib.SPLIT_FP16X2):
         assert isinstance(x, torch.Tensor) and x.dim() == 2 and x.is_cuda
-        if metric not in _METRICS:
-            raise ValueError('Unknown distance metric: {}. '
-                             'Please choose either "euclidean" or "cosine"'.format(metric))
+        code = _check_metric(metric)
         lib = _lib.require_device()
         x = x.detach().to(torch.float32)
         if x.stride(1) != 1:
@@ -95,10 +96,8 @@ class PreparedOperand(object):
         self.rows, self.dim, self.metric, self.split, self.device = x.size(0), x.size(1), metric, split, x.device
         nbytes = lib.agrl_distance_operand_bytes(self.rows, self.dim, split)
         self.buf = torch.empty(max(nbytes, 16), dtype=torch.uint8, device=x.device)
-        with torch.cuda.device(x.device):
-            _lib.check(lib.agrl_distance_prepare_operand_dev(
-                x.data_ptr(), x.stride(0), self.rows, self.dim, _METRICS[metric], split, self.buf.data_ptr(),
-                nbytes, torch.cuda.current_stream(x.device).cuda_stream))
+        _lib.call(x.device, lib.agrl_distance_prepare_operand_dev, x.data_ptr(), x.stride(0), self.rows, self.dim, code,
+                  split, self.buf.data_ptr(), nbytes)
 
 
     def rows_view(self, r0, r1):
@@ -134,8 +133,6 @@ def distance_prepared(q, g, out=None):
         out = torch.empty(q.rows, g.rows, dtype=torch.float32, device=q.device)
     assert out.shape == (q.rows, g.rows) and out.stride(1) == 1 and out.dtype == torch.float32
     if q.rows and g.rows:
-        with torch.cuda.device(q.device):
-            _lib.check(lib.agrl_distance_prepared_dev(
-                q.buf.data_ptr(), q.rows, g.buf.data_ptr(), g.rows, q.dim, _METRICS[q.metric], q.split,
-                out.data_ptr(), out.stride(0), torch.cuda.current_stream(q.device).cuda_stream))
+        _lib.call(q.device, lib.agrl_distance_prepared_dev, q.buf.data_ptr(), q.rows, g.buf.data_ptr(), g.rows, q.dim,
+                  _METRICS[q.metric], q.split, out.data_ptr(), out.stride(0))
     return out

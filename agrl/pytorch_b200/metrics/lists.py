@@ -17,23 +17,17 @@ import torch
 
 from .. import _lib
 from .distance import PreparedOperand
-
-_ops = None
-
-
-def _cuda_ops():
-    global _ops
-    if _ops is None:
-        from ..sharded import CudaOps
-        _ops = CudaOps()
-    return _ops
+from .rank import _dev_labels
 
 
-def _labels(q_pids, g_pids, q_camids, g_camids, dev):
-    if q_pids is None:
-        return None
-    from ..sharded import _as_dev_i64
-    return [_as_dev_i64(x, dev) for x in (q_pids, g_pids, q_camids, g_camids)]
+def _lists(ops, keys_of, nq, ng, dev, k, labels, exclude_junk):
+    """The (indices, distances) lists of k from the keys ``keys_of(depth)`` of a non-empty gallery of ng rows."""
+    from .. import sharded
+    labels = None if labels[0] is None else [_dev_labels(x, dev) for x in labels]
+    with torch.cuda.device(dev):
+        depth = sharded.list_depth(k, ops, labels, exclude_junk)
+        keys = keys_of(depth) if ng else torch.full((nq, depth), -1, dtype=torch.int64, device=dev)
+        return ops.lists(keys.unsqueeze(0), int(k), *(labels or [None] * 4), exclude_junk=exclude_junk)
 
 
 def rank_lists(distmat, k, q_pids=None, g_pids=None, q_camids=None, g_camids=None, exclude_junk=False):
@@ -41,23 +35,15 @@ def rank_lists(distmat, k, q_pids=None, g_pids=None, q_camids=None, g_camids=Non
 
     ``distmat`` is a (num_q, num_g) fp32 CUDA tensor (any row stride) or a numpy array, which is copied to the current
     device.  Raises ValueError when k plus the junk depth (the most items of one query's pid and camera) exceeds 8192."""
-    from .. import sharded
-    ops = _cuda_ops()
+    from ..sharded import CudaOps
+    ops = CudaOps()
     if not isinstance(distmat, torch.Tensor):
         distmat = torch.from_numpy(np.ascontiguousarray(distmat, dtype=np.float32)).cuda()
     assert distmat.dim() == 2 and distmat.dtype == torch.float32 and distmat.is_cuda
     if distmat.stride(1) != 1:
         distmat = distmat.contiguous()
-    dev = distmat.device
-    nq, ng = distmat.shape
-    labels = _labels(q_pids, g_pids, q_camids, g_camids, dev)
-    with torch.cuda.device(dev):
-        depth = sharded.list_depth(k, ops, labels, exclude_junk)
-        if ng == 0:
-            keys = torch.full((nq, depth), -1, dtype=torch.int64, device=dev)
-        else:
-            keys = ops.keys(distmat, depth, 0)
-        return ops.lists(keys.unsqueeze(0), int(k), *(labels or [None] * 4), exclude_junk=exclude_junk)
+    return _lists(ops, lambda depth: ops.keys(distmat, depth, 0), distmat.shape[0], distmat.shape[1], distmat.device, k,
+                  (q_pids, g_pids, q_camids, g_camids), exclude_junk)
 
 
 def retrieve(qf, gallery, k, metric='euclidean', q_pids=None, g_pids=None, q_camids=None, g_camids=None,
@@ -70,17 +56,11 @@ def retrieve(qf, gallery, k, metric='euclidean', q_pids=None, g_pids=None, q_cam
     queries whose candidate list overflows the fused route go through distance blocks.  The lists are the same either
     way."""
     from .. import sharded
-    ops = _cuda_ops()
+    ops = sharded.CudaOps()
     gop = gallery if isinstance(gallery, PreparedOperand) else PreparedOperand(gallery, metric, split)
-    dev = gop.device
-    qop = PreparedOperand(qf.to(dev), gop.metric, gop.split)
-    labels = _labels(q_pids, g_pids, q_camids, g_camids, dev)
-    with torch.cuda.device(dev):
-        depth = sharded.list_depth(k, ops, labels, exclude_junk)
-        if fused is None:
-            fused = gop.rows >= sharded.FUSED_MIN_GALLERY
-        if gop.rows == 0:
-            keys = torch.full((qop.rows, depth), -1, dtype=torch.int64, device=dev)
-        else:
-            keys = ops.topk_keys(qop, gop, depth, 0, fused=fused and depth <= sharded.FUSED_MAX_DEPTH)
-        return ops.lists(keys.unsqueeze(0), int(k), *(labels or [None] * 4), exclude_junk=exclude_junk)
+    qop = PreparedOperand(qf.to(gop.device), gop.metric, gop.split)
+
+    def keys_of(depth):
+        use = sharded.fused_default(gop.rows, depth) if fused is None else fused and depth <= sharded.FUSED_MAX_DEPTH
+        return ops.topk_keys(qop, gop, depth, 0, fused=use)
+    return _lists(ops, keys_of, qop.rows, gop.rows, gop.device, k, (q_pids, g_pids, q_camids, g_camids), exclude_junk)

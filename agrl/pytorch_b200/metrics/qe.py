@@ -15,8 +15,6 @@ import torch
 
 from .. import _lib
 
-_ops = {}
-
 
 def query_expansion(qf, gf, qe_k=5, qe_times=1, alpha=3.0, split=_lib.SPLIT_FP16X2, fused=None):
     """(qf', gf'): the query and gallery features after ``qe_times`` iterations of alpha query expansion over their
@@ -32,9 +30,7 @@ def query_expansion(qf, gf, qe_k=5, qe_times=1, alpha=3.0, split=_lib.SPLIT_FP16
     assert gf.dim() == 2, 'Expected 2-D tensor, but got {}-D'.format(gf.dim())
     assert qf.size(1) == gf.size(1)
     sharded.check_qe_args(qe_k, qe_times, alpha, qf.size(0) + gf.size(0))
-    lib_ops = _ops.get(split)
-    if lib_ops is None:
-        lib_ops = _ops[split] = sharded.CudaOps(split)
+    lib_ops = sharded.CudaOps(split)
     dev = qf.device if qf.is_cuda else torch.device('cuda', torch.cuda.current_device())
     x = torch.cat([qf.detach().to(device=dev, dtype=torch.float32), gf.detach().to(device=dev, dtype=torch.float32)])
     nq, n = qf.size(0), x.size(0)

@@ -82,21 +82,18 @@ def _market1501_device(distmat, q_pids, g_pids, q_camids, g_camids, max_rank, re
         print('Note: number of gallery samples is quite small, got {}'.format(num_g))
     if distmat.stride(1) != 1:
         distmat = distmat.contiguous()
-    with torch.cuda.device(dev):
-        qp, gp, qc, gc = (_dev_labels(x, dev) for x in (q_pids, g_pids, q_camids, g_camids))
-        rank_len = min(max_rank, num_g)
-        cmc = torch.empty(rank_len, dtype=torch.float32, device=dev)
-        scal = torch.zeros(4, dtype=torch.float32, device=dev)          # [mAP, status(u32), num_valid(i64)]
-        all_ap = torch.empty(max(num_q, 1), dtype=torch.float32, device=dev)
-        wsb = lib.agrl_rank_workspace_bytes(num_q, num_g, max_rank)
-        ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
-        rc = lib.agrl_rank_market1501_dev(
-            distmat.data_ptr(), distmat.stride(0), qp.data_ptr(), gp.data_ptr(), qc.data_ptr(), gc.data_ptr(),
-            num_q, num_g, max_rank, cmc.data_ptr(), scal.data_ptr(), all_ap.data_ptr(),
-            scal.data_ptr() + 8, scal.data_ptr() + 4, ws.data_ptr(), wsb,
-            torch.cuda.current_stream(dev).cuda_stream)
-        _lib.check(rc)
-        host = scal.cpu()                                                # synchronises the stream
+    qp, gp, qc, gc = (_dev_labels(x, dev) for x in (q_pids, g_pids, q_camids, g_camids))
+    rank_len = min(max_rank, num_g)
+    cmc = torch.empty(rank_len, dtype=torch.float32, device=dev)
+    scal = torch.zeros(4, dtype=torch.float32, device=dev)              # [mAP, status(u32), num_valid(i64)]
+    all_ap = torch.empty(max(num_q, 1), dtype=torch.float32, device=dev)
+    wsb = lib.agrl_rank_workspace_bytes(num_q, num_g, max_rank)
+    ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
+    _lib.call(dev, lib.agrl_rank_market1501_dev,
+              distmat.data_ptr(), distmat.stride(0), qp.data_ptr(), gp.data_ptr(), qc.data_ptr(), gc.data_ptr(),
+              num_q, num_g, max_rank, cmc.data_ptr(), scal.data_ptr(), all_ap.data_ptr(),
+              scal.data_ptr() + 8, scal.data_ptr() + 4, ws.data_ptr(), wsb)
+    host = scal.cpu()                                                    # synchronises the stream
     status = int(host.view(torch.int32)[1])
     _raise_status(status)
     out = (cmc.cpu().numpy(), float(host[0]))
@@ -116,19 +113,16 @@ def _mars_device(distmat, q_pids, g_pids, q_camids, g_camids, max_rank, return_a
         raise ValueError('could not broadcast input array from shape ({},) into shape ({},)'.format(num_g, max_rank))
     if distmat.stride(1) != 1:
         distmat = distmat.contiguous()
-    with torch.cuda.device(dev):
-        qp, gp, qc, gc = (_dev_labels(x, dev) for x in (q_pids, g_pids, q_camids, g_camids))
-        out = torch.zeros(max_rank + 2, dtype=torch.float64, device=dev)   # [cmc.., mAP, status]
-        all_ap = torch.empty(num_q, dtype=torch.float64, device=dev)
-        wsb = lib.agrl_rank_workspace_bytes(num_q, num_g, max_rank)
-        ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
-        rc = lib.agrl_rank_mars_dev(
-            distmat.data_ptr(), distmat.stride(0), qp.data_ptr(), gp.data_ptr(), qc.data_ptr(), gc.data_ptr(),
-            num_q, num_g, max_rank, out.data_ptr(), out.data_ptr() + 8 * max_rank, all_ap.data_ptr(),
-            out.data_ptr() + 8 * (max_rank + 1), ws.data_ptr(), wsb,
-            torch.cuda.current_stream(dev).cuda_stream)
-        _lib.check(rc)
-        host = out.cpu()
+    qp, gp, qc, gc = (_dev_labels(x, dev) for x in (q_pids, g_pids, q_camids, g_camids))
+    out = torch.zeros(max_rank + 2, dtype=torch.float64, device=dev)       # [cmc.., mAP, status]
+    all_ap = torch.empty(num_q, dtype=torch.float64, device=dev)
+    wsb = lib.agrl_rank_workspace_bytes(num_q, num_g, max_rank)
+    ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
+    _lib.call(dev, lib.agrl_rank_mars_dev,
+              distmat.data_ptr(), distmat.stride(0), qp.data_ptr(), gp.data_ptr(), qc.data_ptr(), gc.data_ptr(),
+              num_q, num_g, max_rank, out.data_ptr(), out.data_ptr() + 8 * max_rank, all_ap.data_ptr(),
+              out.data_ptr() + 8 * (max_rank + 1), ws.data_ptr(), wsb)
+    host = out.cpu()
     _raise_status(int(host.view(torch.int32)[2 * (max_rank + 1)]))
     res = (host[:max_rank].numpy().copy(), np.float64(host[max_rank]))
     return res + (all_ap.cpu().numpy(),) if return_all_ap else res

@@ -25,6 +25,8 @@ import torch
 import torch.distributed as dist
 
 from . import _lib
+from .metrics.distance import PreparedOperand, _check_metric, _workspace, _METRICS, distance_prepared
+from .metrics.rank import _dev_labels, _raise_status
 
 
 def shard_bounds(n, world):
@@ -39,13 +41,23 @@ def shard_bounds(n, world):
 
 
 def or_across_ranks(status, group=None):
-    """Bitwise OR of every rank's status word (bit flags: LABEL_RANGE, ZERO_DIVISION, TOPK_OVERFLOW, ...), in place.
-    NCCL has no BOR reduction: the word is expanded into one 0/1 lane per bit, all-reduced with MAX and re-packed."""
+    """Bitwise OR of every rank's status word (bit flags: LABEL_RANGE, ZERO_DIVISION, TOPK_OVERFLOW, ...), in place."""
+    return status.copy_(_max_and_or(None, status, group)[1])
+
+
+def _max_and_or(maxed, status, group):
+    """(MAX over the ranks of the int32 tensor ``maxed``, bitwise OR over the ranks of the status words) in one
+    all-reduce.  NCCL has no BOR reduction: each word is expanded into one 0/1 lane per bit, all-reduced with MAX and
+    re-packed."""
     shifts = torch.arange(16, device=status.device, dtype=torch.int32)
-    bits = (status.to(torch.int32).view(-1, 1) >> shifts) & 1
-    dist.all_reduce(bits, op=dist.ReduceOp.MAX, group=group)
-    status.copy_((bits << shifts).sum(dim=1).to(status.dtype).view_as(status))
-    return status
+    lanes = ((status.to(torch.int32).view(-1, 1) >> shifts) & 1).view(-1)
+    n = 0 if maxed is None else maxed.numel()
+    word = lanes if maxed is None else torch.cat([maxed.to(torch.int32).view(-1), lanes])
+    dist.all_reduce(word, op=dist.ReduceOp.MAX, group=group)
+    return word[:n], (word[n:].view(-1, 16) << shifts).sum(dim=1).to(status.dtype).view_as(status)
+
+
+TOPK_BLOCK_BYTES = 1 << 31       # largest distance block (num_q rows x num_g fp32) of the unfused top-k routes
 
 
 class CudaOps(object):
@@ -54,14 +66,6 @@ class CudaOps(object):
     def __init__(self, split=_lib.SPLIT_FP16X2):
         self.lib = _lib.require_device()
         self.split = split
-        self._ws = {}
-
-    def _workspace(self, dev, nbytes):
-        key = (dev, torch.cuda.current_stream(dev).cuda_stream)       # never shared between streams
-        ws = self._ws.get(key)
-        if ws is None or ws.numel() < nbytes:
-            ws = self._ws[key] = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-        return ws
 
     def distance(self, qf, gf, metric):
         from .metrics import compute_distance_matrix
@@ -75,54 +79,51 @@ class CudaOps(object):
         ngood = torch.empty(nq, dtype=torch.int32, device=dev)
         status = torch.zeros(1, dtype=torch.int32, device=dev)
         wsb = self.lib.agrl_rank_workspace_bytes(nq, ng, max_rank)
-        ws = self._workspace(dev, wsb)
-        with torch.cuda.device(dev):
-            _lib.check(self.lib.agrl_rank_mars_partial_dev(
-                d.data_ptr(), d.stride(0), q_pids.data_ptr(), g_pids.data_ptr(), q_camids.data_ptr(),
-                g_camids.data_ptr(), nq, ng, max_rank, offset, keys.data_ptr(), cls.data_ptr(), ngood.data_ptr(),
-                status.data_ptr(), ws.data_ptr(), wsb, torch.cuda.current_stream(dev).cuda_stream))
+        _lib.call(dev, self.lib.agrl_rank_mars_partial_dev,
+                  d.data_ptr(), d.stride(0), q_pids.data_ptr(), g_pids.data_ptr(), q_camids.data_ptr(),
+                  g_camids.data_ptr(), nq, ng, max_rank, offset, keys.data_ptr(), cls.data_ptr(), ngood.data_ptr(),
+                  status.data_ptr(), _workspace(dev, wsb).data_ptr(), wsb)
         return keys, cls, ngood, status
+
+    def _fused_keys(self, qop, gop, depth, offset):
+        """(keys (num_q, depth) int64, status) of two PreparedOperand from the distance -> top-k fused into the GEMM
+        epilogue (agrl_distance_topk_dev); the status has ST_TOPK_OVERFLOW when a query's candidate list overflowed."""
+        assert (qop.metric, qop.split, qop.dim, qop.device) == (gop.metric, gop.split, gop.dim, gop.device)
+        dev, nq = qop.device, qop.rows
+        keys = torch.empty(nq, depth, dtype=torch.int64, device=dev)
+        status = torch.zeros(1, dtype=torch.int32, device=dev)
+        wsb = self.lib.agrl_distance_topk_workspace_bytes(nq)
+        _lib.call(dev, self.lib.agrl_distance_topk_dev,
+                  qop.buf.data_ptr(), nq, gop.buf.data_ptr(), gop.rows, qop.dim, _METRICS[qop.metric], qop.split, depth,
+                  offset, keys.data_ptr(), status.data_ptr(), _workspace(dev, wsb).data_ptr(), wsb)
+        return keys, status
 
     def topk_fused(self, qop, gop, q_pids, g_pids, q_camids, g_camids, max_rank, offset, allow_fallback=True):
         """Same outputs as ``partial`` from two PreparedOperand, with the distance -> top-k fused into the GEMM epilogue
         (agrl_distance_topk_dev + agrl_rank_mars_classify_dev): no (num_q x num_g) matrix is allocated.  When a query's
         candidate list overflows (a gallery ordered by distance to the query) the call falls back to distance blocks +
         ``partial`` -- the results are the same either way."""
-        from .metrics.distance import _METRICS
-        assert (qop.metric, qop.split, qop.dim, qop.device) == (gop.metric, gop.split, gop.dim, gop.device)
+        keys, status = self._fused_keys(qop, gop, max_rank, offset)
         dev, nq, ng = qop.device, qop.rows, gop.rows
-        keys = torch.empty(nq, max_rank, dtype=torch.int64, device=dev)
         cls = torch.empty(nq, max_rank, dtype=torch.uint8, device=dev)
         ngood = torch.empty(nq, dtype=torch.int32, device=dev)
-        status = torch.zeros(1, dtype=torch.int32, device=dev)
-        lib = self.lib
-        wsb = max(lib.agrl_distance_topk_workspace_bytes(nq), lib.agrl_rank_mars_classify_workspace_bytes(nq, ng))
-        ws = self._workspace(dev, wsb)
-        with torch.cuda.device(dev):
-            stream = torch.cuda.current_stream(dev).cuda_stream
-            _lib.check(lib.agrl_distance_topk_dev(
-                qop.buf.data_ptr(), nq, gop.buf.data_ptr(), ng, qop.dim, _METRICS[qop.metric], qop.split, max_rank, offset,
-                keys.data_ptr(), status.data_ptr(), ws.data_ptr(), wsb, stream))
-            _lib.check(lib.agrl_rank_mars_classify_dev(
-                keys.data_ptr(), q_pids.data_ptr(), g_pids.data_ptr(), q_camids.data_ptr(), g_camids.data_ptr(),
-                nq, ng, max_rank, offset, cls.data_ptr(), ngood.data_ptr(), status.data_ptr(), ws.data_ptr(), wsb, stream))
+        wsb = self.lib.agrl_rank_mars_classify_workspace_bytes(nq, ng)
+        _lib.call(dev, self.lib.agrl_rank_mars_classify_dev,
+                  keys.data_ptr(), q_pids.data_ptr(), g_pids.data_ptr(), q_camids.data_ptr(), g_camids.data_ptr(),
+                  nq, ng, max_rank, offset, cls.data_ptr(), ngood.data_ptr(), status.data_ptr(),
+                  _workspace(dev, wsb).data_ptr(), wsb)
         if allow_fallback and int(status.cpu()) & _lib.ST_TOPK_OVERFLOW:
             return self.topk_unfused(qop, gop, q_pids, g_pids, q_camids, g_camids, max_rank, offset)
         return keys, cls, ngood, status
 
-    def topk_unfused(self, qop, gop, q_pids, g_pids, q_camids, g_camids, max_rank, offset, block_bytes=1 << 31):
+    def topk_unfused(self, qop, gop, q_pids, g_pids, q_camids, g_camids, max_rank, offset, block_bytes=TOPK_BLOCK_BYTES):
         """distance blocks (at most ``block_bytes`` each) written to HBM + the streaming top-k kernel"""
-        from .metrics.distance import distance_prepared
-        dev, nq, ng = qop.device, qop.rows, gop.rows
-        rows = max(1, min(nq, block_bytes // max(4 * ng, 1)))
+        dev, nq = qop.device, qop.rows
         keys = torch.empty(nq, max_rank, dtype=torch.int64, device=dev)
         cls = torch.empty(nq, max_rank, dtype=torch.uint8, device=dev)
         ngood = torch.empty(nq, dtype=torch.int32, device=dev)
         status = torch.zeros(1, dtype=torch.int32, device=dev)
-        dbuf = torch.empty(rows, ng, device=dev)
-        for q0 in range(0, nq, rows):
-            q1 = min(nq, q0 + rows)
-            dm = distance_prepared(qop.rows_view(q0, q1), gop, out=dbuf[:q1 - q0])
+        for q0, q1, dm in _distance_blocks(qop, gop, block_bytes):
             k, c, n, st = self.partial(dm, q_pids[q0:q1], g_pids, q_camids[q0:q1], g_camids, max_rank, offset)
             keys[q0:q1], cls[q0:q1], ngood[q0:q1] = k, c, n
             status |= st
@@ -133,17 +134,12 @@ class CudaOps(object):
         parts, nq = keys_all.shape[0], keys_all.shape[1]
         out = torch.zeros(max_rank + 2, dtype=torch.float64, device=dev)      # [cmc.., mAP, status]
         wsb = self.lib.agrl_rank_workspace_bytes(nq, 0, max_rank)
-        ws = self._workspace(dev, wsb)
-        with torch.cuda.device(dev):
-            _lib.check(self.lib.agrl_rank_mars_merge_dev(
-                keys_all.data_ptr(), cls_all.data_ptr(), ngood.data_ptr(), parts, nq, max_rank,
-                out.data_ptr(), out.data_ptr() + 8 * max_rank, None, out.data_ptr() + 8 * (max_rank + 1),
-                ws.data_ptr(), wsb, torch.cuda.current_stream(dev).cuda_stream))
-            host = out.cpu()
-            st_parts = int(status_parts.cpu())
-        status = int(host.view(torch.int32)[2 * (max_rank + 1)]) | st_parts
-        from .metrics.rank import _raise_status
-        _raise_status(status)
+        _lib.call(dev, self.lib.agrl_rank_mars_merge_dev,
+                  keys_all.data_ptr(), cls_all.data_ptr(), ngood.data_ptr(), parts, nq, max_rank,
+                  out.data_ptr(), out.data_ptr() + 8 * max_rank, None, out.data_ptr() + 8 * (max_rank + 1),
+                  _workspace(dev, wsb).data_ptr(), wsb)
+        host = out.cpu()
+        _raise_status(int(host.view(torch.int32)[2 * (max_rank + 1)]) | int(status_parts.cpu()))
         return host[:max_rank].numpy().copy(), np.float64(host[max_rank])
 
     # ---- ranked lists (agrl_rank_lists_dev) ---------------------------------------------------------------------------
@@ -155,26 +151,15 @@ class CudaOps(object):
     def topk_keys(self, qop, gop, depth, offset, fused=True):
         """``keys`` of the distance block of two PreparedOperand without materialising it: distance -> top-k fused into
         the GEMM epilogue (depth <= 256); when a query's candidate list overflows, or with ``fused=False``, distance blocks
-        of at most 2 GiB + ``keys``.  The keys are the same either way."""
-        from .metrics.distance import _METRICS, distance_prepared
-        assert (qop.metric, qop.split, qop.dim, qop.device) == (gop.metric, gop.split, gop.dim, gop.device)
-        dev, nq, ng = qop.device, qop.rows, gop.rows
-        keys = torch.empty(nq, depth, dtype=torch.int64, device=dev)
+        of at most TOPK_BLOCK_BYTES + ``keys``.  The keys are the same either way."""
         if fused:
-            status = torch.zeros(1, dtype=torch.int32, device=dev)
-            wsb = self.lib.agrl_distance_topk_workspace_bytes(nq)
-            ws = self._workspace(dev, wsb)
-            with torch.cuda.device(dev):
-                _lib.check(self.lib.agrl_distance_topk_dev(
-                    qop.buf.data_ptr(), nq, gop.buf.data_ptr(), ng, qop.dim, _METRICS[qop.metric], qop.split, depth, offset,
-                    keys.data_ptr(), status.data_ptr(), ws.data_ptr(), wsb, torch.cuda.current_stream(dev).cuda_stream))
+            keys, status = self._fused_keys(qop, gop, depth, offset)
             if not int(status.cpu()) & _lib.ST_TOPK_OVERFLOW:
                 return keys
-        rows = max(1, min(nq, (1 << 31) // max(4 * ng, 1)))
-        dbuf = torch.empty(rows, ng, device=dev)
-        for q0 in range(0, nq, rows):
-            q1 = min(nq, q0 + rows)
-            keys[q0:q1] = self.keys(distance_prepared(qop.rows_view(q0, q1), gop, out=dbuf[:q1 - q0]), depth, offset)
+        else:
+            keys = torch.empty(qop.rows, depth, dtype=torch.int64, device=qop.device)
+        for q0, q1, dm in _distance_blocks(qop, gop):
+            keys[q0:q1] = self.keys(dm, depth, offset)
         return keys
 
     def junk_depth(self, q_pids, g_pids, q_camids, g_camids):
@@ -184,11 +169,9 @@ class CudaOps(object):
         nq, ng = q_pids.numel(), g_pids.numel()
         out = torch.zeros(2, dtype=torch.int32, device=dev)                   # [J, status]
         wsb = self.lib.agrl_rank_mars_classify_workspace_bytes(nq, ng)
-        ws = self._workspace(dev, wsb)
-        with torch.cuda.device(dev):
-            _lib.check(self.lib.agrl_rank_junk_depth_dev(
-                q_pids.data_ptr(), g_pids.data_ptr(), q_camids.data_ptr(), g_camids.data_ptr(), nq, ng, out.data_ptr(),
-                out.data_ptr() + 4, ws.data_ptr(), wsb, torch.cuda.current_stream(dev).cuda_stream))
+        _lib.call(dev, self.lib.agrl_rank_junk_depth_dev,
+                  q_pids.data_ptr(), g_pids.data_ptr(), q_camids.data_ptr(), g_camids.data_ptr(), nq, ng, out.data_ptr(),
+                  out.data_ptr() + 4, _workspace(dev, wsb).data_ptr(), wsb)
         return out[0:1], out[1:2]
 
     def lists(self, keys_all, k, q_pids=None, g_pids=None, q_camids=None, g_camids=None, exclude_junk=False):
@@ -202,16 +185,12 @@ class CudaOps(object):
         status = torch.zeros(1, dtype=torch.int32, device=dev)
         ng = g_pids.numel() if exclude_junk else 0
         wsb = self.lib.agrl_rank_mars_classify_workspace_bytes(nq, ng) if exclude_junk else 0
-        ws = self._workspace(dev, max(wsb, 1))
+        ws = _workspace(dev, max(wsb, 1))
         lab = [x.data_ptr() if exclude_junk else None for x in (q_pids, g_pids, q_camids, g_camids)]
-        with torch.cuda.device(dev):
-            _lib.check(self.lib.agrl_rank_lists_dev(
-                keys_all.data_ptr(), parts, nq, depth, k, lab[0], lab[1], lab[2], lab[3], ng, int(bool(exclude_junk)),
-                index.data_ptr(), dist_.data_ptr(), k, status.data_ptr(), ws.data_ptr(), wsb,
-                torch.cuda.current_stream(dev).cuda_stream))
-            st = int(status.cpu())
-        from .metrics.rank import _raise_status
-        _raise_status(st)
+        _lib.call(dev, self.lib.agrl_rank_lists_dev,
+                  keys_all.data_ptr(), parts, nq, depth, k, lab[0], lab[1], lab[2], lab[3], ng, int(bool(exclude_junk)),
+                  index.data_ptr(), dist_.data_ptr(), k, status.data_ptr(), ws.data_ptr(), wsb)
+        _raise_status(int(status.cpu()))
         return index, dist_
 
     # ---- alpha query expansion (agrl_qe_mix_dev) ----------------------------------------------------------------------
@@ -219,12 +198,11 @@ class CudaOps(object):
         """(indices int64, cosine distances fp32), (rows, k) each: the ranked lists of the rows x[r0:r1] of every
         (r0, r1) in ``ranges``, in order, against all rows of x (each row's list includes itself).  x is split into
         cosine operand planes once; a range that is not the whole of x is a rows_view of those planes.  The distance ->
-        top-k is fused into the GEMM epilogue from FUSED_MIN_GALLERY rows of x on (``fused`` overrides); the lists are
-        the same either way."""
-        from .metrics.distance import PreparedOperand
+        top-k is fused into the GEMM epilogue as fused_default decides for the rows of x (``fused`` overrides); the
+        lists are the same either way."""
         n, dev = x.shape[0], x.device
         if fused is None:
-            fused = n >= FUSED_MIN_GALLERY
+            fused = fused_default(n, k)
         op = PreparedOperand(x, 'cosine', self.split)
         keys = [self.topk_keys(op if (r0, r1) == (0, n) else op.rows_view(r0, r1), op, k, 0,
                                fused=fused and k <= FUSED_MAX_DEPTH) for r0, r1 in ranges if r1 > r0]
@@ -239,10 +217,9 @@ class CudaOps(object):
         rows, k = idx.shape
         dim = x.shape[1]
         out = torch.empty(rows, dim, dtype=torch.float32, device=x.device)
-        with torch.cuda.device(x.device):
-            _lib.check(self.lib.agrl_qe_mix_dev(
-                idx.data_ptr(), d.data_ptr(), idx.stride(0), rows, k, x.data_ptr(), x.stride(0), x.shape[0], dim,
-                float(alpha), out.data_ptr(), dim, torch.cuda.current_stream(x.device).cuda_stream))
+        _lib.call(x.device, self.lib.agrl_qe_mix_dev,
+                  idx.data_ptr(), d.data_ptr(), idx.stride(0), rows, k, x.data_ptr(), x.stride(0), x.shape[0], dim,
+                  float(alpha), out.data_ptr(), dim)
         return out
 
 
@@ -252,11 +229,9 @@ class CudaOps(object):
         nq, ng = q_pids.numel(), g_pids.numel()
         out = torch.zeros(2, dtype=torch.int32, device=dev)                   # [max_count, status]
         wsb = self.lib.agrl_rank_workspace_bytes(nq, ng, 1)
-        ws = self._workspace(dev, wsb)
-        with torch.cuda.device(dev):
-            _lib.check(self.lib.agrl_rank_market1501_count_dev(
-                q_pids.data_ptr(), g_pids.data_ptr(), q_camids.data_ptr(), g_camids.data_ptr(), nq, ng,
-                out.data_ptr(), out.data_ptr() + 4, ws.data_ptr(), wsb, torch.cuda.current_stream(dev).cuda_stream))
+        _lib.call(dev, self.lib.agrl_rank_market1501_count_dev,
+                  q_pids.data_ptr(), g_pids.data_ptr(), q_camids.data_ptr(), g_camids.data_ptr(), nq, ng,
+                  out.data_ptr(), out.data_ptr() + 4, _workspace(dev, wsb).data_ptr(), wsb)
         return out[0:1], out[1:2]
 
     def market_gather(self, d, q_pids, g_pids, q_camids, g_camids, offset, cap):
@@ -266,12 +241,10 @@ class CudaOps(object):
         counts = torch.empty(2, nq, dtype=torch.int32, device=dev)            # [npos, njunk]
         status = torch.zeros(1, dtype=torch.int32, device=dev)
         wsb = self.lib.agrl_rank_workspace_bytes(nq, ng, 1)
-        ws = self._workspace(dev, wsb)
-        with torch.cuda.device(dev):
-            _lib.check(self.lib.agrl_rank_market1501_gather_dev(
-                d.data_ptr(), d.stride(0), q_pids.data_ptr(), g_pids.data_ptr(), q_camids.data_ptr(), g_camids.data_ptr(),
-                nq, ng, offset, cap, keys.data_ptr(), counts[0].data_ptr(), counts[1].data_ptr(), status.data_ptr(),
-                ws.data_ptr(), wsb, torch.cuda.current_stream(dev).cuda_stream))
+        _lib.call(dev, self.lib.agrl_rank_market1501_gather_dev,
+                  d.data_ptr(), d.stride(0), q_pids.data_ptr(), g_pids.data_ptr(), q_camids.data_ptr(), g_camids.data_ptr(),
+                  nq, ng, offset, cap, keys.data_ptr(), counts[0].data_ptr(), counts[1].data_ptr(), status.data_ptr(),
+                  _workspace(dev, wsb).data_ptr(), wsb)
         return keys, counts, status
 
     def market_bin(self, d, offset, keys_all):
@@ -283,10 +256,8 @@ class CudaOps(object):
             _lib.check(_lib.E_UNSUPPORTED)
         cnt = torch.empty(nq, n2, dtype=torch.int32, device=dev)
         srt = torch.empty(nq, n2, dtype=torch.int64, device=dev)
-        with torch.cuda.device(dev):
-            _lib.check(self.lib.agrl_rank_market1501_bin_dev(
-                d.data_ptr(), d.stride(0), nq, ng, offset, keys_all.data_ptr(), parts, cap, cnt.data_ptr(), srt.data_ptr(),
-                torch.cuda.current_stream(dev).cuda_stream))
+        _lib.call(dev, self.lib.agrl_rank_market1501_bin_dev,
+                  d.data_ptr(), d.stride(0), nq, ng, offset, keys_all.data_ptr(), parts, cap, cnt.data_ptr(), srt.data_ptr())
         return cnt, srt
 
     def market_finalize(self, cnt, srt, counts, ng_total, parts, cap, max_rank, status_parts):
@@ -296,16 +267,12 @@ class CudaOps(object):
         cmc = torch.empty(rank_len, dtype=torch.float32, device=dev)
         scal = torch.zeros(4, dtype=torch.float32, device=dev)               # [mAP, status(u32), num_valid(i64)]
         wsb = self.lib.agrl_rank_market1501_finalize_workspace_bytes(nq, parts, cap, max_rank)
-        ws = self._workspace(dev, wsb)
-        with torch.cuda.device(dev):
-            _lib.check(self.lib.agrl_rank_market1501_finalize_dev(
-                cnt.data_ptr(), srt.data_ptr(), counts[0].data_ptr(), counts[1].data_ptr(), nq, ng_total, parts, cap, max_rank,
-                cmc.data_ptr(), scal.data_ptr(), None, scal.data_ptr() + 8, scal.data_ptr() + 4, ws.data_ptr(), wsb,
-                torch.cuda.current_stream(dev).cuda_stream))
-            host = scal.cpu()
-            st_parts = int(status_parts.cpu())
-        from .metrics.rank import _raise_status
-        _raise_status(int(host.view(torch.int32)[1]) | st_parts)
+        _lib.call(dev, self.lib.agrl_rank_market1501_finalize_dev,
+                  cnt.data_ptr(), srt.data_ptr(), counts[0].data_ptr(), counts[1].data_ptr(), nq, ng_total, parts, cap,
+                  max_rank, cmc.data_ptr(), scal.data_ptr(), None, scal.data_ptr() + 8, scal.data_ptr() + 4,
+                  _workspace(dev, wsb).data_ptr(), wsb)
+        host = scal.cpu()
+        _raise_status(int(host.view(torch.int32)[1]) | int(status_parts.cpu()))
         return cmc.cpu().numpy(), float(host[0])
 
     # ---- gallery-sharded k-reciprocal re-ranking (agrl_rerank_shard_*) ----------------------------------------------
@@ -321,17 +288,15 @@ class CudaOps(object):
         st = SimpleNamespace(ws=torch.empty(wsb, dtype=torch.uint8, device=dev), wsb=wsb, nq=nq, ng=ng, offset=offset,
                              n_own=n_own, k1=k1, k2=k2)
         rank_rows = torch.empty(nq + n_own, K, dtype=torch.int32, device=dev)
-        with torch.cuda.device(dev):
-            stream = torch.cuda.current_stream(dev).cuda_stream
 
-            def rows(slab, r0, r1):
-                _lib.check(lib.agrl_rerank_shard_rows_dev(
-                    qg.data_ptr(), qg.stride(0), qq.data_ptr(), qq.stride(0), slab.data_ptr() if slab is not None else None,
-                    slab.stride(0) if slab is not None else 0, nq, ng, offset, n_own, r0, r1, k1, k2, rank_rows.data_ptr(),
-                    st.ws.data_ptr(), wsb, stream))
-            rows(None, 0, nq)
-            for s0, slab in gg_slabs:
-                rows(slab.contiguous(), nq + s0, nq + s0 + slab.shape[1])
+        def rows(slab, r0, r1):
+            _lib.call(dev, lib.agrl_rerank_shard_rows_dev,
+                      qg.data_ptr(), qg.stride(0), qq.data_ptr(), qq.stride(0), slab.data_ptr() if slab is not None else None,
+                      slab.stride(0) if slab is not None else 0, nq, ng, offset, n_own, r0, r1, k1, k2, rank_rows.data_ptr(),
+                      st.ws.data_ptr(), wsb)
+        rows(None, 0, nq)
+        for s0, slab in gg_slabs:
+            rows(slab.contiguous(), nq + s0, nq + s0 + slab.shape[1])
         return st, rank_rows
 
     def rerank_expand(self, st, rank_all):
@@ -342,22 +307,32 @@ class CudaOps(object):
         idx = torch.empty(rows, cap, dtype=torch.int32, device=dev)
         val = torch.empty(rows, cap, dtype=torch.float32, device=dev)
         cnt = torch.empty(rows, dtype=torch.int32, device=dev)
-        with torch.cuda.device(dev):
-            _lib.check(self.lib.agrl_rerank_shard_expand_dev(
-                rank_all.data_ptr(), st.nq, st.ng, st.offset, st.n_own, st.k1, st.k2, idx.data_ptr(), val.data_ptr(),
-                cnt.data_ptr(), st.ws.data_ptr(), st.wsb, torch.cuda.current_stream(dev).cuda_stream))
+        _lib.call(dev, self.lib.agrl_rerank_shard_expand_dev,
+                  rank_all.data_ptr(), st.nq, st.ng, st.offset, st.n_own, st.k1, st.k2, idx.data_ptr(), val.data_ptr(),
+                  cnt.data_ptr(), st.ws.data_ptr(), st.wsb)
         return idx, val, cnt
 
     def rerank_finish(self, st, rank_all, idx_all, val_all, cnt_all, lambda_value):
         """Phase C: this rank's (num_q, n_own) block of the re-ranked distance matrix."""
         dev = rank_all.device
         out = torch.empty(st.nq, st.n_own, dtype=torch.float32, device=dev)
-        with torch.cuda.device(dev):
-            _lib.check(self.lib.agrl_rerank_shard_finish_dev(
-                rank_all.data_ptr(), idx_all.data_ptr(), val_all.data_ptr(), cnt_all.data_ptr(), st.nq, st.ng, st.offset,
-                st.n_own, st.k1, st.k2, float(lambda_value), out.data_ptr() if st.n_own else None, max(st.n_own, 1),
-                st.ws.data_ptr(), st.wsb, torch.cuda.current_stream(dev).cuda_stream))
+        _lib.call(dev, self.lib.agrl_rerank_shard_finish_dev,
+                  rank_all.data_ptr(), idx_all.data_ptr(), val_all.data_ptr(), cnt_all.data_ptr(), st.nq, st.ng, st.offset,
+                  st.n_own, st.k1, st.k2, float(lambda_value), out.data_ptr() if st.n_own else None, max(st.n_own, 1),
+                  st.ws.data_ptr(), st.wsb)
         return out
+
+
+def _distance_blocks(qop, gop, block_bytes=TOPK_BLOCK_BYTES):
+    """(q0, q1, distance rows q0:q1 of two PreparedOperand) over the queries, in blocks of at most ``block_bytes`` that
+    reuse one buffer: consume each block before taking the next."""
+    assert (qop.metric, qop.split, qop.dim, qop.device) == (gop.metric, gop.split, gop.dim, gop.device)
+    nq, ng = qop.rows, gop.rows
+    rows = max(1, min(nq, block_bytes // max(4 * ng, 1)))
+    dbuf = torch.empty(rows, ng, device=qop.device)
+    for q0 in range(0, nq, rows):
+        q1 = min(nq, q0 + rows)
+        yield q0, q1, distance_prepared(qop.rows_view(q0, q1), gop, out=dbuf[:q1 - q0])
 
 
 def rerank_row_dims(k1, k2):
@@ -370,12 +345,6 @@ def rerank_row_dims(k1, k2):
     return max(k1 + 1, k2), cap
 
 
-def _as_dev_i64(x, dev):
-    if isinstance(x, torch.Tensor):
-        return x.to(device=dev, dtype=torch.int64).contiguous()
-    return torch.as_tensor(np.ascontiguousarray(np.asarray(x), dtype=np.int64)).to(dev)
-
-
 def _unlabelled(nq, ng, dev):
     """query / gallery labels for a ranking that needs none: no gallery item shares a query's pid"""
     return torch.zeros(nq, dtype=torch.int64, device=dev), torch.ones(ng, dtype=torch.int64, device=dev)
@@ -383,6 +352,13 @@ def _unlabelled(nq, ng, dev):
 
 MAX_LIST_DEPTH = 8192            # k + J per query and shard (agrl_rank_mars_partial_dev / agrl_rank_lists_dev)
 FUSED_MAX_DEPTH = 256            # deepest list the fused distance -> top-k keeps (agrl_distance_topk_dev)
+FUSED_MIN_GALLERY = 32768        # gallery rows per shard from which the fused distance -> top-k is the default
+
+
+def fused_default(gallery_rows, depth):
+    """Whether lists of ``depth`` keys against ``gallery_rows`` rows come from the distance -> top-k fused into the
+    GEMM epilogue unless the caller says otherwise: from FUSED_MIN_GALLERY rows on, up to FUSED_MAX_DEPTH keys."""
+    return gallery_rows >= FUSED_MIN_GALLERY and depth <= FUSED_MAX_DEPTH
 
 
 def list_depth(k, ops, labels, exclude_junk, group=None, world=1):
@@ -397,12 +373,8 @@ def list_depth(k, ops, labels, exclude_junk, group=None, world=1):
         if labels is None:
             raise ValueError('exclude_junk needs q_pids, g_pids, q_camids and g_camids')
         j, status = ops.junk_depth(*labels)
-        if world > 1:                     # J and the status bits in one MAX reduction
-            shifts = torch.arange(16, device=status.device, dtype=torch.int32)
-            word = torch.cat([j.to(torch.int32), (status.to(torch.int32) >> shifts) & 1])
-            dist.all_reduce(word, op=dist.ReduceOp.MAX, group=group)
-            j, status = word[0:1], (word[1:] << shifts).sum().view(1)
-        from .metrics.rank import _raise_status
+        if world > 1:
+            j, status = _max_and_or(j, status, group)
         host = torch.cat([j, status.to(j.dtype)]).cpu()
         _raise_status(int(host[1]))
         J = int(host[0])
@@ -423,22 +395,19 @@ def rank_lists_sharded(qf, gf_local, k, q_pids=None, g_pids_local=None, q_camids
     Exchanges: the query broadcast and shard layout of evaluate_mars_sharded, one all-reduce(max) of the junk depth J with
     ``exclude_junk`` (plus one all-gather of the gallery labels), and one all-gather of num_q x (k + J) keys.
     Raises ValueError when k + J exceeds MAX_LIST_DEPTH."""
-    if metric not in ('euclidean', 'cosine'):
-        raise ValueError('Unknown distance metric: {}. Please choose either "euclidean" or "cosine"'.format(metric))
-    world = dist.get_world_size(group) if dist.is_initialized() else 1
+    _check_metric(metric)
     dev = qf.device
     ops = ops or CudaOps()
     qf = qf.contiguous()
     labels = None
     if q_pids is not None:
-        labels = [_as_dev_i64(x, dev) for x in (q_pids, g_pids_local, q_camids, g_camids_local)]
-    if world > 1 and broadcast_queries:
-        _broadcast_queries(qf, labels[0] if labels else None, labels[2] if labels else None, group)
-    counts, rank = _shard_layout(gf_local.shape[0], dev, world, group, gallery_counts)
-    offset, n_own, nq = sum(counts[:rank]), counts[rank], qf.shape[0]
+        labels = [_dev_labels(x, dev) for x in (q_pids, g_pids_local, q_camids, g_camids_local)]
+    world, rank, counts, offset, n_own = _shard_prologue(qf, gf_local, group, broadcast_queries, gallery_counts,
+                                                         *(labels[0::2] if labels else ()))      # q_pids, q_camids
+    nq = qf.shape[0]
     depth = list_depth(k, ops, labels, exclude_junk, group, world)
     if fused is None:
-        fused = n_own >= FUSED_MIN_GALLERY and hasattr(ops, 'topk_keys') and depth <= FUSED_MAX_DEPTH
+        fused = hasattr(ops, 'topk_keys') and fused_default(n_own, depth)
     if re_rank:
         d = re_ranking_sharded(qf, gf_local, metric, k1, k2, lambda_value, group=group, broadcast_queries=False, ops=ops,
                                gallery_counts=counts)
@@ -447,24 +416,15 @@ def rank_lists_sharded(qf, gf_local, k, q_pids=None, g_pids_local=None, q_camids
     elif re_rank:
         keys = ops.keys(d, depth, offset)
     elif fused:
-        from .metrics.distance import PreparedOperand
         keys = ops.topk_keys(PreparedOperand(qf, metric, ops.split), PreparedOperand(gf_local, metric, ops.split), depth,
                              offset, fused=depth <= FUSED_MAX_DEPTH)
     else:
         keys = ops.keys(ops.distance(qf, gf_local, metric), depth, offset)
-    if world > 1:
-        keys_all = torch.empty((world * nq, depth), dtype=keys.dtype, device=dev)
-        dist.all_gather_into_tensor(keys_all, keys.contiguous(), group=group)
-        keys_all = keys_all.view(world, nq, depth)
-        if exclude_junk:                  # the junk test needs the labels of every listed item
-            labels[1] = _gather_shard_rows(labels[1], 0, counts, rank, group)
-            labels[3] = _gather_shard_rows(labels[3], 0, counts, rank, group)
-    else:
-        keys_all = keys.unsqueeze(0)
+    keys_all = _gather_lists(keys, world, group)
+    if world > 1 and exclude_junk:        # the junk test needs the labels of every listed item
+        labels[1] = _gather_shard_rows(labels[1], 0, counts, rank, group)
+        labels[3] = _gather_shard_rows(labels[3], 0, counts, rank, group)
     return ops.lists(keys_all, k, *(labels or [None] * 4), exclude_junk=exclude_junk)
-
-
-FUSED_MIN_GALLERY = 32768        # gallery rows per shard from which the fused distance -> top-k is the default
 
 
 def check_qe_args(qe_k, qe_times, alpha, n):
@@ -487,17 +447,15 @@ def query_expansion_sharded(qf, gf_local, qe_k=5, qe_times=1, alpha=3.0, group=N
     bit-identical to the matching rows of metrics.query_expansion on the whole sets.  Arguments as in
     evaluate_mars_sharded; shards may be empty.  Each iteration all-gathers the gallery rows; each rank then ranks its
     query and gallery rows against the whole joint set and mixes them.  Raises ValueError as check_qe_args."""
-    world = dist.get_world_size(group) if dist.is_initialized() else 1
     ops = ops or CudaOps()
     assert qf.dim() == 2 and gf_local.dim() == 2 and qf.size(1) == gf_local.size(1)
     dev = qf.device
     qf = qf.detach().to(torch.float32).contiguous()
     gf = gf_local.detach().to(device=dev, dtype=torch.float32).contiguous()
-    if world > 1 and broadcast_queries:
+    if broadcast_queries and _world_size(group) > 1:
         qf = qf.clone()                   # the broadcast writes into it
-        _broadcast_queries(qf, None, None, group)
-    counts, rank = _shard_layout(gf.shape[0], dev, world, group, gallery_counts)
-    nq, offset, n_own = qf.shape[0], sum(counts[:rank]), counts[rank]
+    _, rank, counts, offset, n_own = _shard_prologue(qf, gf, group, broadcast_queries, gallery_counts)
+    nq = qf.shape[0]
     check_qe_args(qe_k, qe_times, alpha, nq + sum(counts))
     lo = nq + offset
     for _ in range(qe_times):
@@ -506,6 +464,21 @@ def query_expansion_sharded(qf, gf_local, qe_k=5, qe_times=1, alpha=3.0, group=N
         mixed = ops.qe_mix(idx, d, x, alpha)
         qf, gf = mixed[:nq], mixed[nq:]
     return qf, gf
+
+
+def _world_size(group):
+    return dist.get_world_size(group) if dist.is_initialized() else 1
+
+
+def _shard_prologue(qf, gf_local, group, broadcast_queries, gallery_counts, qp=None, qc=None):
+    """(world, rank, counts, offset, n_own) of a sharded entry: rank 0's queries (and their labels qp, qc) broadcast
+    into qf (qp, qc) with ``broadcast_queries``, then the rows of every rank's gallery shard (_shard_layout), the global
+    index of this rank's first gallery row and its number of rows."""
+    world = _world_size(group)
+    if world > 1 and broadcast_queries:
+        _broadcast_queries(qf, qp, qc, group)
+    counts, rank = _shard_layout(gf_local.shape[0], qf.device, world, group, gallery_counts)
+    return world, rank, counts, sum(counts[:rank]), counts[rank]
 
 
 def _shard_layout(n_local_rows, dev, world, group, gallery_counts):
@@ -548,6 +521,15 @@ def _gather_shard_rows(t, head, counts, rank, group):
     return torch.cat([t[:head]] + [buf[r * most:r * most + c] for r, c in enumerate(counts)])
 
 
+def _gather_lists(t, world, group):
+    """(world, num_q, depth) view of every rank's per-query lists t (num_q, depth), in rank order (one all-gather)."""
+    if world == 1:
+        return t.unsqueeze(0)
+    out = t.new_empty((world * t.shape[0],) + tuple(t.shape[1:]))
+    dist.all_gather_into_tensor(out, t.contiguous(), group=group)
+    return out.view((world,) + tuple(t.shape))
+
+
 RERANK_SLAB_BYTES = 1 << 31      # largest g_g column slab (num_g x columns fp32) alive at a time
 
 
@@ -562,15 +544,11 @@ def re_ranking_sharded(qf, gf_local, metric='euclidean', k1=20, k2=6, lambda_val
     (num_g x K int32) and of the k-reciprocal rows (num_g x cap x 8 B + counts).  Per-rank limits: k1 <= 30, k2 <= 8,
     num_g_r <= 50000 (agrl_rerank_shard_workspace_bytes); the D rows take 4 (num_q + num_g_r)(num_q + num_g) bytes.
     """
-    if metric not in ('euclidean', 'cosine'):
-        raise ValueError('Unknown distance metric: {}. Please choose either "euclidean" or "cosine"'.format(metric))
-    world = dist.get_world_size(group) if dist.is_initialized() else 1
+    _check_metric(metric)
     ops = ops or CudaOps()
     qf, gf_own = qf.contiguous(), gf_local.contiguous()
-    if world > 1 and broadcast_queries:
-        _broadcast_queries(qf, None, None, group)
-    counts, rank = _shard_layout(gf_own.shape[0], qf.device, world, group, gallery_counts)
-    nq, ng, n_own, offset = qf.shape[0], sum(counts), counts[rank], sum(counts[:rank])
+    _, rank, counts, offset, n_own = _shard_prologue(qf, gf_own, group, broadcast_queries, gallery_counts)
+    nq, ng = qf.shape[0], sum(counts)
     gf_all = _gather_shard_rows(gf_own, 0, counts, rank, group)
     # the operand roles of the single-device path: qq = d(q, q), qg = d(q, g), gg[:, own] = d(g, g_own)
     qq = ops.distance(qf, qf, metric)
@@ -600,45 +578,32 @@ def evaluate_mars_sharded(qf, gf_local, q_pids, g_pids_local, q_camids, g_camids
     evaluate_rank(use_metric_mars=True) on one device.
     Returns (numpy.float64[max_rank], numpy.float64) on every rank.
     """
-    world = dist.get_world_size(group) if dist.is_initialized() else 1
     dev = qf.device
     ops = ops or CudaOps()
-    qp, qc = _as_dev_i64(q_pids, dev), _as_dev_i64(q_camids, dev)
-    gp, gc = _as_dev_i64(g_pids_local, dev), _as_dev_i64(g_camids_local, dev)
+    qp, qc = _dev_labels(q_pids, dev), _dev_labels(q_camids, dev)
+    gp, gc = _dev_labels(g_pids_local, dev), _dev_labels(g_camids_local, dev)
     qf = qf.contiguous()
-    if world > 1 and broadcast_queries:
-        _broadcast_queries(qf, qp, qc, group)
-    # global index of this shard's first row
-    counts, rank = _shard_layout(gf_local.shape[0], dev, world, group, gallery_counts)
+    world, _, counts, offset, n_own = _shard_prologue(qf, gf_local, group, broadcast_queries, gallery_counts, qp, qc)
     total = sum(counts)
     if total < max_rank:
         raise ValueError('could not broadcast input array from shape ({},) into shape ({},)'.format(total, max_rank))
-    offset = sum(counts[:rank])
 
     if fused is None:
-        fused = gf_local.shape[0] >= FUSED_MIN_GALLERY and hasattr(ops, 'topk_fused') and max_rank <= 256
+        fused = hasattr(ops, 'topk_fused') and fused_default(n_own, max_rank)
     if re_rank:
         d = re_ranking_sharded(qf, gf_local, metric, k1, k2, lambda_value, group=group, broadcast_queries=False, ops=ops,
                                gallery_counts=counts)
         keys, cls, ngood, status = ops.partial(d, qp, gp, qc, gc, max_rank, offset)
     elif fused:
-        from .metrics.distance import PreparedOperand
         keys, cls, ngood, status = ops.topk_fused(PreparedOperand(qf, metric, ops.split), PreparedOperand(gf_local, metric, ops.split),
                                                   qp, gp, qc, gc, max_rank, offset)
     else:
         d = ops.distance(qf, gf_local, metric)
         keys, cls, ngood, status = ops.partial(d, qp, gp, qc, gc, max_rank, offset)
+    keys_all, cls_all = _gather_lists(keys, world, group), _gather_lists(cls, world, group)
     if world > 1:
-        nq = keys.shape[0]
-        keys_all = torch.empty((world * nq, max_rank), dtype=keys.dtype, device=dev)   # rank-major concatenation
-        cls_all = torch.empty((world * nq, max_rank), dtype=cls.dtype, device=dev)
-        dist.all_gather_into_tensor(keys_all, keys, group=group)
-        dist.all_gather_into_tensor(cls_all, cls, group=group)
-        keys_all, cls_all = keys_all.view(world, nq, max_rank), cls_all.view(world, nq, max_rank)
         dist.all_reduce(ngood, op=dist.ReduceOp.SUM, group=group)
         or_across_ranks(status, group)
-    else:
-        keys_all, cls_all = keys.unsqueeze(0), cls.unsqueeze(0)
     return ops.merge(keys_all, cls_all, ngood, max_rank, status)
 
 
@@ -650,16 +615,13 @@ def evaluate_market1501_sharded(qf, gf_local, q_pids, g_pids_local, q_camids, g_
 
     Exchanges: all-reduce(max) of one int, all-gather of the per-query same-pid key lists, all-reduce(sum)
     of their positive / junk counts, all-reduce(sum) of the per-list-item rank counts."""
-    world = dist.get_world_size(group) if dist.is_initialized() else 1
     dev = qf.device
     ops = ops or CudaOps()
-    qp, qc = _as_dev_i64(q_pids, dev), _as_dev_i64(q_camids, dev)
-    gp, gc = _as_dev_i64(g_pids_local, dev), _as_dev_i64(g_camids_local, dev)
+    qp, qc = _dev_labels(q_pids, dev), _dev_labels(q_camids, dev)
+    gp, gc = _dev_labels(g_pids_local, dev), _dev_labels(g_camids_local, dev)
     qf = qf.contiguous()
-    if world > 1 and broadcast_queries:
-        _broadcast_queries(qf, qp, qc, group)
-    counts_g, rank = _shard_layout(gf_local.shape[0], dev, world, group, gallery_counts)
-    ng_total, offset = sum(counts_g), sum(counts_g[:rank])
+    world, _, counts_g, offset, _ = _shard_prologue(qf, gf_local, group, broadcast_queries, gallery_counts, qp, qc)
+    ng_total = sum(counts_g)
     if ng_total < max_rank:
         print('Note: number of gallery samples is quite small, got {}'.format(ng_total))     # rank_cy.pyx:160-162
 
@@ -671,15 +633,10 @@ def evaluate_market1501_sharded(qf, gf_local, q_pids, g_pids_local, q_camids, g_
     d = ops.distance(qf, gf_local, metric)
     keys, counts, st2 = ops.market_gather(d, qp, gp, qc, gc, offset, cap)
     status = torch.bitwise_or(status, st2)
-    nq = keys.shape[0]
+    keys_all = _gather_lists(keys, world, group)
     if world > 1:
-        keys_all = torch.empty((world * nq, cap), dtype=keys.dtype, device=dev)
-        dist.all_gather_into_tensor(keys_all, keys, group=group)
-        keys_all = keys_all.view(world, nq, cap)
         dist.all_reduce(counts, op=dist.ReduceOp.SUM, group=group)
         or_across_ranks(status, group)
-    else:
-        keys_all = keys.unsqueeze(0)
     cnt, srt = ops.market_bin(d, offset, keys_all)
     if world > 1:
         dist.all_reduce(cnt, op=dist.ReduceOp.SUM, group=group)

@@ -31,11 +31,9 @@ def re_ranking_dev(q_g_dist, q_q_dist, g_g_dist, k1=20, k2=6, lambda_value=0.3):
     if wsb == 0:
         _lib.check(_lib.E_UNSUPPORTED)
     out = torch.empty(nq, ng, dtype=torch.float32, device=dev)
-    with torch.cuda.device(dev):
-        ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
-        _lib.check(lib.agrl_rerank_dev(qg.data_ptr(), qg.stride(0), qq.data_ptr(), qq.stride(0), gg.data_ptr(), gg.stride(0),
-                                       nq, ng, int(k1), int(k2), float(lambda_value), out.data_ptr(), out.stride(0),
-                                       ws.data_ptr(), wsb, torch.cuda.current_stream(dev).cuda_stream))
+    ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
+    _lib.call(dev, lib.agrl_rerank_dev, qg.data_ptr(), qg.stride(0), qq.data_ptr(), qq.stride(0), gg.data_ptr(), gg.stride(0),
+              nq, ng, int(k1), int(k2), float(lambda_value), out.data_ptr(), out.stride(0), ws.data_ptr(), wsb)
     return out
 
 

@@ -70,7 +70,7 @@ def run_case(name, nq, ng, dim, args, flush):
     g = torch.Generator(device=DEV).manual_seed(nq)
     qf, gf = torch.randn(nq, dim, generator=g, device=DEV), torch.randn(ng, dim, generator=g, device=DEV)
     n = nq + ng
-    ops = metrics.qe._ops.get(_lib.SPLIT_FP16X2) or sharded.CudaOps()
+    ops = sharded.CudaOps()
     x = torch.cat([qf, gf])
     idx, d = ops.qe_lists(x, [(0, n)], k)
     q, gq = metrics.query_expansion(qf, gf, k, 1, alpha)

@@ -108,7 +108,7 @@ def main():
     nq, ng, dim = 10000, 1000000, 2048
     gop = PreparedOperand(torch.randn(ng, dim, generator=g, device=DEV))      # the fp32 gallery is freed afterwards
     qf = torch.randn(nq, dim, generator=g, device=DEV)
-    ops = metrics.lists._cuda_ops()
+    ops = sharded.CudaOps()
     qop = PreparedOperand(qf)
     keys = ops.topk_keys(qop, gop, k, 0)
     emit(args.out, 'retrieve_10kx1mx2048', {
